@@ -71,6 +71,19 @@ def main():
         sched[f"{name}.args"] = np.array([ns, nmin, nmax, steps], dtype=np.float64)
     np.savez(os.path.join(OUT, "schedule.npz"), **sched)
 
+    # ---------------------------------------------------------------- the reference's conf/*.toml, parsed (f4)
+    import json
+    import tomllib
+    conf_dir = os.path.join(ref_shim.REFERENCE_ROOT, "conf")
+    confs = {}
+    for f in sorted(os.listdir(conf_dir)):
+        if f.endswith(".toml"):
+            with open(os.path.join(conf_dir, f), "rb") as fh:
+                confs[f] = tomllib.load(fh)
+    with open(os.path.join(OUT, "reference_conf.json"), "w") as fh:
+        json.dump(confs, fh, indent=1, sort_keys=True)
+        fh.write("\n")
+
     # ---------------------------------------------------------------- common small problem
     cfg = ref_shim.make_config(ref, "tiktok", **{
         "base.denoise_dim": f"[{H}]", "hyper.noise_scale": 0.5, "hyper.sim_weight": 0.01,

@@ -141,12 +141,12 @@ def test_load_config_accepts_every_shipped_toml(name):
 
 @pytest.mark.parametrize("name", sorted(_EXPECT))
 def test_shipped_tomls_carry_the_reference_values(name):
-    ref = os.path.join("/root/reference/conf", name)
-    if not os.path.isfile(ref):
-        pytest.skip("reference tree not present on this machine")
+    """tests/golden/reference_conf.json holds the reference's conf/*.toml, parsed (oracle/gen_golden.py)."""
+    import json
     import tomllib
-    with open(ref, "rb") as f, open(os.path.join(_CONF, name), "rb") as g:
-        assert tomllib.load(f) == tomllib.load(g)
+    from conftest import GOLDEN
+    with open(os.path.join(GOLDEN, "reference_conf.json")) as f, open(os.path.join(_CONF, name), "rb") as g:
+        assert tomllib.load(g) == json.load(f)[name]
 
 
 def test_load_config_rejects_a_sampling_step_beyond_the_schedule(tmp_path):
@@ -157,36 +157,71 @@ def test_load_config_rejects_a_sampling_step_beyond_the_schedule(tmp_path):
 
 
 def test_reference_arm_and_gpu_arm_draw_identical_denoise_weights(monkeypatch):
-    """bench.py's two arms must time the same model: the reference's Denoise (oracle/_ref) and ours are constructed in
-    the same order from the same seed, so their parameters are bit-identical."""
-    import sys
-    root = os.path.dirname(_CONF)
-    if not os.path.isfile(os.path.join(root, "oracle", "_ref", "Model.py")):
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py)")
-    sys.path.insert(0, root)
+    """bench.py's two arms must time the same model: the GPU arm's Denoise models and GaussianDiffusion
+    (bench.build_workload) draw the reference's weights and noise schedule from the same seed.  The reference's side is
+    golden data of oracle/gen_golden.py: its Denoise (I = 120, H = 32) drawn right after torch.manual_seed(1818), then
+    moved by 0.05 * randn_like of every parameter, and its schedules for the noise of conf/tiktok.toml and of
+    conf/sports.toml (which conf/baby.toml shares).  Replaying those moves on the first modality gives the same tensors
+    bit for bit only if its construction drew exactly the reference's numbers, in the reference's order and count; the
+    second modality must then be the same construction from where the first one left the generator, as in the
+    reference arm (bench.load_reference_arm)."""
     import bench
-    monkeypatch.setitem(bench.WORKLOADS, "baby", dict(users=50, items=70, modalities=["image", "text"], hidden=32,
-                                                      conf="baby.toml"))
+    from conftest import load_golden, params_of
+    from diffmm_b200.Model import Denoise
+    g, sched = load_golden("denoise_forward"), load_golden("schedule")
+    for name, golden_noise in (("tiktok", "tiktok"), ("baby", "sports")):
+        hyper = bench.workload_hyper(name)
+        assert hyper["noise"] + (hyper["steps"],) == tuple(sched[f"{golden_noise}.args"]), name
+        monkeypatch.setitem(bench.WORKLOADS, name, dict(users=40, items=120, modalities=["image", "text"], hidden=32,
+                                                        conf=f"{name}.toml"))
+        _, _, diff, _ = bench.build_workload(name, "cpu", 1818, "bf16", 1, hyper)
+        np.testing.assert_array_equal(diff.posterior_mean_coef1.cpu().numpy(),
+                                      sched[f"{golden_noise}.posterior_mean_coef1"], err_msg=name)
     hyper = bench.workload_hyper("baby")
-    assert hyper["sampling_step"] == 5
-    saved = {k: sys.modules.get(k) for k in ("Conf", "Model", "DataHandler", "Main", "Utils", "Utils.Utils", "Utils.Log")}
-    is_avail, t_cuda, m_cuda = torch.cuda.is_available, torch.Tensor.cuda, torch.nn.Module.cuda
-    try:
-        _, _, diff_o, dens_o = bench.build_workload("baby", "cpu", 3, "bf16", 1, hyper)
-        _, diff_r, dens_r = bench.load_reference_arm(bench.WORKLOADS["baby"], 3, hyper)
-    finally:
-        torch.cuda.is_available, torch.Tensor.cuda, torch.nn.Module.cuda = is_avail, t_cuda, m_cuda
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-    for m in dens_o:
-        so, sr = dens_o[m].state_dict(), dens_r[m].state_dict()
+    cfg, _, _, dens = bench.build_workload("baby", "cpu", 1818, "bf16", 1, hyper)
+    # the first modality: the reference's draws (golden replay)
+    monkeypatch.setitem(bench.WORKLOADS, "baby", dict(users=40, items=120, modalities=["image"], hidden=32,
+                                                      conf="baby.toml"))
+    _, _, _, first = bench.build_workload("baby", "cpu", 1818, "bf16", 1, hyper)
+    after_first = torch.get_rng_state()
+    moved = {k: v.clone() for k, v in first["image"].state_dict().items()}
+    for k in moved:                                   # parameters() order == state_dict() order for Denoise
+        moved[k].add_(0.05 * torch.randn_like(moved[k]))
+    want = params_of(g)
+    names = dict(emb_w="emb_layer.weight", emb_b="emb_layer.bias", w1="in_layers.0.weight", b1="in_layers.0.bias",
+                 w2="out_layers.0.weight", b2="out_layers.0.bias", gate_w="gate_layer.weight", gate_b="gate_layer.bias")
+    assert sorted(names.values()) == sorted(moved)
+    for k, sd in names.items():
+        np.testing.assert_array_equal(moved[sd].numpy(), want[k], err_msg=k)
+    # both modalities of the two-modality workload: the first as above, the second drawn where the first left off
+    torch.set_rng_state(after_first)
+    second = Denoise([120, 32], [32, 120], cfg)
+    for m, ref in (("image", first["image"]), ("text", second)):
+        so, sr = dens[m].state_dict(), ref.state_dict()
         assert list(so) == list(sr)
         for k in so:
             assert torch.equal(so[k], sr[k]), (m, k)
-    assert torch.equal(diff_o.posterior_mean_coef1.cpu(), diff_r.posterior_mean_coef1.cpu())
+
+
+def test_bench_dump_outputs_writes_float_arrays_within_the_budget(tmp_path):
+    """bench.py --dump-outputs: integer outputs become exact float64, fp32 stays fp32; over the byte budget every array
+    keeps the same seeded sample of its elements, the same from run to run."""
+    import bench
+    ids = np.arange(5000, dtype=np.int32) * 7
+    vals = torch.linspace(0, 1, 3000)
+    bench.dump_outputs(str(tmp_path / "all"), {"ids": ids, "vals": vals})
+    a, v = np.load(tmp_path / "all" / "ids.npy"), np.load(tmp_path / "all" / "vals.npy")
+    assert a.dtype == np.float64 and np.array_equal(a, ids) and v.dtype == np.float32 and np.array_equal(v, vals.numpy())
+    budget = 3 * bench.NPY_HEADER_BYTES + 20000
+    for run in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / run), {"ids": ids, "vals": vals, "one": np.ones(10, np.float64)}, budget=budget)
+    files = sorted((tmp_path / "s1").iterdir())
+    assert sum(f.stat().st_size for f in files) <= budget
+    for f in files:
+        s1, s2 = np.load(f), np.load(tmp_path / "s2" / f.name)
+        assert 0 < s1.size and np.array_equal(s1, s2)
+    s = np.load(tmp_path / "s1" / "ids.npy")
+    assert np.all(np.diff(s) > 0) and np.all(np.isin(s, ids))
 
 
 def test_fused_step_adam_falls_back_to_torch_on_unsupported_configurations():
@@ -208,3 +243,15 @@ def test_fused_step_adam_falls_back_to_torch_on_unsupported_configurations():
     for x, y in zip(a, b):
         assert torch.equal(x, y)
     assert oa.state_dict()["param_groups"][0]["lr"] == ob.state_dict()["param_groups"][0]["lr"]
+
+
+def test_bench_rejects_dump_outputs_for_the_reference_arm(tmp_path):
+    """--dump-outputs writes what our timed path computed; the reference arm has nothing to write, so the combination is
+    an argument error instead of an empty directory."""
+    import subprocess
+    import sys
+    root = os.path.dirname(_CONF)
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--dump-outputs",
+                        str(tmp_path / "out")], capture_output=True, text=True, timeout=120, cwd=root)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr, r.stderr[-1000:]
+    assert not (tmp_path / "out").exists()
