@@ -10,6 +10,7 @@ Differences, all on purpose (SURVEY.md §0):
 """
 from __future__ import annotations
 
+import ast
 import dataclasses
 from dataclasses import dataclass, field
 
@@ -131,3 +132,12 @@ def validate(cfg: Config) -> None:
         raise ValueError(f"hyper.steps must be >= 1, got {cfg.hyper.steps}")
     if cfg.base.precision not in ("bf16", "bf16x3"):
         raise ValueError(f"base.precision must be 'bf16' or 'bf16x3', got {cfg.base.precision!r}")
+    # Main.py:155-156 literal_eval's the hidden widths of the Denoise; an empty list builds a Denoise without layers
+    # (the loss shapes fail in the reference too)
+    try:
+        dims = ast.literal_eval(cfg.base.denoise_dim) if isinstance(cfg.base.denoise_dim, str) else None
+    except (ValueError, SyntaxError, TypeError, MemoryError, RecursionError):
+        dims = None
+    if not (isinstance(dims, list) and dims and all(type(w) is int and w > 0 for w in dims)):
+        raise ValueError(f"base.denoise_dim must be a non-empty list of positive ints such as \"[1024]\", "
+                         f"got {cfg.base.denoise_dim!r}")

@@ -334,11 +334,11 @@ class GaussianDiffusion(nn.Module):
         if noise is None:
             noise = rng.randn_like(x_start)
         from . import train_step
-        if (train_step.enabled() and x_start.is_cuda and len(model.in_layers) == 1 and len(model.out_layers) == 1
+        if (train_step.enabled() and x_start.is_cuda
                 and modal_feat is not None and modal_feat.shape[1] == 64 and not modal_feat.requires_grad
                 and not i_embs.requires_grad and not x_start.requires_grad):
             # the hot configuration (Main.py:153-170 with the dead item-embedding gradient dropped): forward and backward
-            # of the whole loss scheduled by hand on the kernels (train_step.py)
+            # of the whole loss scheduled by hand on the kernels (train_step.py), for any denoise_dim depth
             core = train_step.denoise_loss(self, model, x_start, timesteps, noise, modal_feat, i_embs)
             reg_loss = l2_reg_loss(self.config.train.reg, [i_embs], self.device)
             return core + reg_loss * self.config.train.reg

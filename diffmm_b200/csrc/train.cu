@@ -229,7 +229,7 @@ __global__ void __launch_bounds__(256) diff_loss_bwd_kernel(const double* __rest
 // ---------------------------------------------------------------------------------------------- hidden layer backward
 // 32 x 32 tiles: dz[b, h] = cm[b] dh[b, h] (1 - hv^2), hv = h_hi (+ h_lo).  Writes dz fp32 (bias gradient source), dz as
 // the operand of the input-gradient contraction, and through a shared-memory transpose dz^T and (cm h)^T, the operands
-// of the two weight-gradient contractions (K = batch).
+// of the two weight-gradient contractions (K = batch).  cm == NULL: no row scale (cm = 1, so (cm h)^T is h^T).
 __global__ void __launch_bounds__(256) hidden_bwd_kernel(const float* __restrict__ dh, int64_t ld_dh,
                                                          const float* __restrict__ h_f32, int64_t ld_hf,
                                                          const uint16_t* __restrict__ h_hi, const uint16_t* __restrict__ h_lo,
@@ -257,7 +257,7 @@ __global__ void __launch_bounds__(256) hidden_bwd_kernel(const float* __restrict
         hv = dmm_bf16_to_f32(h_hi[b * ld_h + c]);
         if (h_lo) hv += dmm_bf16_to_f32(h_lo[b * ld_h + c]);
       }
-      const float s = cm[b];
+      const float s = cm ? cm[b] : 1.f;
       dz = s * dh[b * ld_dh + c] * (1.f - hv * hv);
       hc = s * hv;
       dz_f32[b * ld_dz + c] = dz;
@@ -418,7 +418,7 @@ extern "C" int dmm_hidden_bwd(dmm_ctx* ctx, const float* dh, int64_t ld_dh, cons
                               int64_t ld_h, const float* cm, int64_t n_rows, int64_t H, float* dz_f32, int64_t ld_dz,
                               uint16_t* dz_hi, uint16_t* dz_lo, int64_t ld_dz16, uint16_t* dzt_hi, uint16_t* dzt_lo,
                               uint16_t* hct_hi, uint16_t* hct_lo, int64_t ld_t, void* stream) {
-  DMM_CHECK_ARG(ctx && dh && (h_hi || h_f32) && cm && dz_f32 && dz_hi && dzt_hi && hct_hi, "dmm_hidden_bwd: null argument");
+  DMM_CHECK_ARG(ctx && dh && (h_hi || h_f32) && dz_f32 && dz_hi && dzt_hi && hct_hi, "dmm_hidden_bwd: null argument");
   DMM_CHECK_ARG(H > 0 && ld_dh >= H && (!h_hi || ld_h >= H) && (!h_f32 || ld_hf >= H) && ld_dz >= H && ld_dz16 >= H && ld_t >= n_rows,
                 "dmm_hidden_bwd: bad shape");
   DMM_CHECK_ARG(!!dz_lo == !!dzt_lo && !!dz_lo == !!hct_lo, "dmm_hidden_bwd: lo parts must be given together");

@@ -572,6 +572,7 @@ def diff_loss_bwd(g_loss, um, ui, stats, t, w_tab, sim_weight, n_cols, cm, dumc_
 
 
 def hidden_bwd(dh, h_f32, h_hi, h_lo, cm, H, dz, dz_hi, dz_lo, dzt_hi, dzt_lo, hct_hi, hct_lo):
+    """dz = cm dh (1 - h^2) (fp32 and operand), dz^T and (cm h)^T; cm None: no row scale (dz = dh (1 - h^2), h^T)."""
     B = dh.shape[0]
     _lib.call("dmm_hidden_bwd", _ctx(dh), _p(dh), _row_major(dh, "dh"), _p(h_f32),
               _row_major(h_f32, "h_f32") if h_f32 is not None else 0, _p(h_hi), _p(h_lo),

@@ -13,6 +13,7 @@ Per user block the data flow is
                      (first step, binary CSR rows: gather-sum of W1^T  dmm_csr_gather_act)
                    x_t = c1[i] (h W2^T + b2) + c2[i] x_t  (bf16 operand in place; fp32 scores at i = 0)
                      (first step: c2 x0 added at the CSR positions     dmm_csr_axpy_bf16)
+                   (deeper denoise_dim: h = tanh(h W_k^T + b_k) for each hidden-to-hidden layer in between, dmm_gemm_bf16_tn)
   top-k_u (k_u = deg(u)) -> item ids at the train-CSR offsets          dmm_topk_edges
 and once per modality
   edges -> normalised CSR adjacency                                    dmm_build_norm_adj_csr
@@ -33,19 +34,24 @@ from .autograd import check_precision, packed_weight, packed_weight_pair
 
 
 class ChainWorkspace:
-    """Device buffers of one user block, reused across steps, modalities and blocks."""
+    """Device buffers of one user block, reused across steps, modalities and blocks.  ``hidden`` is the width of a
+    one-hidden-layer Denoise or the tuple of hidden widths of a deeper one (hidden_widths): the two hidden operand
+    buffers are sized by the widest layer, the fp32 state and the time bias by the first (= last) hidden width."""
 
-    def __init__(self, rows: int, n_items: int, hidden: int, d_emb: int, split: bool, device):
-        self.rows, self.n_items, self.hidden, self.d_emb, self.split = rows, n_items, hidden, d_emb, split
+    def __init__(self, rows: int, n_items: int, hidden, d_emb: int, split: bool, device):
+        widths = _widths(hidden)
+        self.rows, self.n_items, self.widths, self.d_emb, self.split = rows, n_items, widths, d_emb, split
+        self.hidden = widths[0]
         self.ld_a = ops.pad_to(n_items, 64)
         self.ld_x = ops.pad_to(n_items, 32)
-        self.ld_h = ops.pad_to(hidden, 64)
+        self.ld_h = ops.pad_to(max(widths), 64)
         bf = dict(dtype=torch.bfloat16, device=device)
         self.device = device
         self._a = None            # bf16 operand copy of x_t [rows, ld_a] (+ lo): only the dense-input / full-chain paths
         self.h_hi = torch.empty((rows, self.ld_h), **bf)
         self.h_lo = torch.empty((rows, self.ld_h), **bf) if split else None
-        self._h2 = None           # second hidden operand (the hidden-space chain ping-pongs: a step reads h_t, writes h_{t-1})
+        self._h2 = None           # second hidden operand (the hidden-space chain ping-pongs: a step reads h_t, writes h_{t-1};
+                                  # so do the hidden-to-hidden layers of a deeper Denoise)
         self.x = torch.empty((rows, self.ld_x), dtype=torch.float32, device=device)
         self.z = None             # fp32 hidden pre-activation state [rows, pad4(hidden)] of the hidden-space chain
         self.bias_eff = None      # [S, hidden] fp32, sized on first use
@@ -77,14 +83,40 @@ class ChainWorkspace:
         return self._cmax
 
     def fits(self, rows, n_items, hidden, d_emb, split):
-        return (rows <= self.rows and n_items == self.n_items and hidden == self.hidden and d_emb == self.d_emb
+        return (rows <= self.rows and n_items == self.n_items and _widths(hidden) == self.widths and d_emb == self.d_emb
                 and split == self.split)
 
 
-def _single_layer(den):
-    if len(den.in_layers) != 1 or len(den.out_layers) != 1:
-        raise NotImplementedError("the fused chain supports denoise_dim with one hidden layer (all shipped configs)")
-    return den.in_layers[0], den.out_layers[0]
+def _widths(hidden) -> Tuple[int, ...]:
+    return (int(hidden),) if isinstance(hidden, (int, np.integer)) else tuple(int(w) for w in hidden)
+
+
+def hidden_widths(den) -> Tuple[int, ...]:
+    """Widths of the 2L - 1 hidden activations of a Denoise with denoise_dim = [d_1, ..., d_L], in forward order:
+    d_L, d_{L-1}, ..., d_1, ..., d_{L-1}, d_L (Model.py:160-162).  (d_L,) for the shipped one-entry configs."""
+    return tuple(int(layer.weight.shape[0]) for layer in list(den.in_layers) + list(den.out_layers)[:-1])
+
+
+def _layers(den):
+    """(first, inner, last) Linear layers of a Denoise: in_layers[0] ([x_t, temb] -> d_L), the 2L - 2 hidden-to-hidden
+    layers in forward order (tanh after each, like after the first) and out_layers[-1] (d_L -> items, no activation)."""
+    layers = list(den.in_layers) + list(den.out_layers)
+    return layers[0], layers[1:-1], layers[-1]
+
+
+def _inner_operands(inner, split):
+    """(W_k hi, lo), b_k, out width, in width of every hidden-to-hidden layer (packed operands are cached per version)."""
+    return [(packed_weight(layer.weight, False, split), layer.bias.detach(), layer.weight.shape[0], layer.weight.shape[1])
+            for layer in inner]
+
+
+def _inner_layers(inner_ops, M, h_hi, h_lo, g_hi, g_lo):
+    """h <- tanh(h W_k^T + b_k) through the hidden-to-hidden layers (one contraction with a bias + tanh epilogue each),
+    ping-ponging between the two operand buffers.  Returns (current, other) with the last activation current."""
+    for (w_hi, w_lo), b, n_out, k in inner_ops:
+        ops.gemm_bf16_tn(h_hi, h_lo, w_hi, w_lo, M, n_out, k, bias=b, act=1, out_hi=g_hi, out_lo=g_lo)
+        h_hi, h_lo, g_hi, g_lo = g_hi, g_lo, h_hi, h_lo
+    return h_hi, h_lo, g_hi, g_lo
 
 
 def chain_mode() -> str:
@@ -148,13 +180,19 @@ def denoise_chain(diff, den, *, x_dense: Optional[torch.Tensor] = None,
     Same function of the inputs, S - 1 item-space contraction pairs fewer.  P and q are rebuilt (inside the
     timed region of bench.py) whenever the weights change.  z_S comes from the CSR gather (x_S = x0) or from one
     dense first-layer contraction (dense x_start or sampling_step > 0).
-    mode 'full' (DIFFMM_CHAIN=full) runs the literal chain: 2 item-space contractions per step."""
-    lin1, lin2 = _single_layer(den)
-    W1, b1, W2, b2 = lin1.weight, lin1.bias, lin2.weight, lin2.bias
+    mode 'full' (DIFFMM_CHAIN=full) runs the literal chain: 2 item-space contractions per step.
+
+    A deeper Denoise (denoise_dim = [d_1, ..., d_L]) has the 2L - 2 hidden-to-hidden layers between its first layer
+    in_layers[0] (W1 above) and its last layer out_layers[-1] (W2 above).  Both chains run them as one contraction with
+    a bias + tanh epilogue each, between producing h (the first activation) and reading it (the last one); the hidden
+    space of the algebra above is the d_L wide one at both ends, so P = W1x W2 stays d_L x d_L."""
+    first, inner, last = _layers(den)
+    W1, b1, W2, b2 = first.weight, first.bias, last.weight, last.bias
     H, K1 = W1.shape
     I = W2.shape[0]
     d = den.time_emb_dim
     assert K1 == I + d
+    widths = hidden_widths(den)
     precision = check_precision(precision or den.precision)
     split = precision == "bf16x3"
     dev = W1.device
@@ -162,8 +200,8 @@ def denoise_chain(diff, den, *, x_dense: Optional[torch.Tensor] = None,
         n_rows = x_dense.shape[0]
         assert x_dense.shape[1] == I
     assert n_rows is not None and n_rows > 0
-    if ws is None or not ws.fits(n_rows, I, H, d, split):
-        ws = ChainWorkspace(n_rows, I, H, d, split, dev)
+    if ws is None or not ws.fits(n_rows, I, widths, d, split):
+        ws = ChainWorkspace(n_rows, I, widths, d, split, dev)
     M = n_rows
     S = diff.steps
     mode = mode or chain_mode()
@@ -204,9 +242,11 @@ def denoise_chain(diff, den, *, x_dense: Optional[torch.Tensor] = None,
         ops.bias_act_pack(z, ws.bias_eff[S - 1], 1, h_hi, h_lo)
     g_hi, g_lo = ws.hidden2()
     g_hi, g_lo = g_hi[:M], (g_lo[:M] if split else None)
+    inner_ops = _inner_operands(inner, split)
     for i in range(S - 1, 0, -1):
         c1 = float(np.float32(diff._h_coef1[i]))          # fp64 table -> .float() (Model.py:352)
         c2 = float(np.float32(diff._h_coef2[i]))
+        h_hi, h_lo, g_hi, g_lo = _inner_layers(inner_ops, M, h_hi, h_lo, g_hi, g_lo)
         # z_i = c1 (h_i P^T + q) + c2 z_{i+1} (fp32 state, in place) and, in the same epilogue,
         # h_{i-1} = tanh(z_i + b1'(i-1)) into the OTHER operand buffer (other CTAs still read h_i)
         # (the last intermediate step only needs h_0: its z is never read again, so it is not written: 80 MB less at baby)
@@ -214,6 +254,7 @@ def denoise_chain(diff, den, *, x_dense: Optional[torch.Tensor] = None,
                          out_hi=g_hi, out_lo=g_lo, post_bias=ws.bias_eff[i - 1], post_act=1)
         h_hi, h_lo, g_hi, g_lo = g_hi, g_lo, h_hi, h_lo
     c1 = float(np.float32(diff._h_coef1[0]))
+    h_hi, h_lo, g_hi, g_lo = _inner_layers(inner_ops, M, h_hi, h_lo, g_hi, g_lo)
     ops.gemm_bf16_tn(h_hi, h_lo, w2_hi, w2_lo, M, I, H, bias=b2d, alpha=c1, out_f32=xv,
                      cmax=ws.chunk_max()[:M] if want_cmax else None)
     return xv
@@ -288,9 +329,10 @@ def _fill_operand(diff, ws, M, I, a_hi, a_lo, x_dense, csr, row_ids, row0, sampl
 
 def _denoise_chain_full(diff, den, ws, M, *, x_dense, csr, row_ids, row0, sampling_step, split, noise, order=None,
                         want_cmax=False):
-    """The literal chain: S x (first layer + tanh, second layer + posterior mean) in item space."""
-    lin1, lin2 = _single_layer(den)
-    W1, b1, W2, b2 = lin1.weight, lin1.bias, lin2.weight, lin2.bias
+    """The literal chain: S x (first layer + tanh, [hidden-to-hidden layers + tanh,] last layer + posterior mean) in item
+    space."""
+    first, inner, last = _layers(den)
+    W1, b1, W2, b2 = first.weight, first.bias, last.weight, last.bias
     H = W1.shape[0]
     I = W2.shape[0]
     dev = W1.device
@@ -299,6 +341,10 @@ def _denoise_chain_full(diff, den, ws, M, *, x_dense, csr, row_ids, row0, sampli
     a_lo = a_lo[:M] if split else None
     h_lo = ws.h_lo[:M] if split else None
     xv = x[:, :I]
+    inner_ops = _inner_operands(inner, split)
+    if inner_ops:
+        g_hi, g_lo = ws.hidden2()
+        g_hi, g_lo = g_hi[:M], (g_lo[:M] if split else None)
 
     S = diff.steps
     # Binary CSR rows at the head of the chain (sampling_step == 0): the first layer of the first reverse step
@@ -328,6 +374,8 @@ def _denoise_chain_full(diff, den, ws, M, *, x_dense, csr, row_ids, row0, sampli
                                row_ids=row_ids, row0=row0, order=order)
         else:
             _gemm1(ws, a_hi, a_lo, w1_hi, w1_lo, M, H, I, bias1, h_hi, h_lo)
+        if inner_ops:
+            h_hi, h_lo, g_hi, g_lo = _inner_layers(inner_ops, M, h_hi, h_lo, g_hi, g_lo)
         c1 = float(np.float32(diff._h_coef1[i]))          # fp64 table -> .float() (Model.py:352)
         c2 = float(np.float32(diff._h_coef2[i]))
         # x_t lives only as the bf16 operand (hi, and lo in bf16x3 mode: hi + lo carries 16 mantissa bits):
@@ -382,10 +430,11 @@ def _gemm1(ws, a_hi, a_lo, w1_hi, w1_lo, M, H, K, bias, h_hi, h_lo):
         k0 += kc
 
 
-def default_block_rows(n_users: int, n_items: int, hidden: int, split: bool, budget_bytes: int = 12 << 30) -> int:
-    """Largest user block whose workspace stays under ``budget_bytes`` (multiple of 128 rows)."""
+def default_block_rows(n_users: int, n_items: int, hidden, split: bool, budget_bytes: int = 12 << 30) -> int:
+    """Largest user block whose workspace stays under ``budget_bytes`` (multiple of 128 rows).  ``hidden``: a width or
+    the tuple of hidden widths (the hidden operands are sized by the widest)."""
     per_row = ops.pad_to(n_items + 16, 64) * 2 * (2 if split else 1) + ops.pad_to(n_items, 32) * 4 \
-        + ops.pad_to(hidden, 64) * 2 * (2 if split else 1)
+        + ops.pad_to(max(_widths(hidden)), 64) * 2 * (2 if split else 1)
     rows = max(128, (budget_bytes // per_row) // 128 * 128)
     return int(min(n_users, rows))
 
@@ -443,9 +492,8 @@ def rebuild_edges(diff, denoise_models: Dict[str, torch.nn.Module], indptr: torc
     any_den = next(iter(denoise_models.values()))
     precision = check_precision(precision or any_den.precision)
     split = precision == "bf16x3"
-    H = any_den.in_layers[0].weight.shape[0]
     if block_rows is None:
-        block_rows = default_block_rows(r1 - r0, n_items, H, split)
+        block_rows = default_block_rows(r1 - r0, n_items, max(max(hidden_widths(d)) for d in denoise_models.values()), split)
         env = os.environ.get("DIFFMM_BLOCK_ROWS")
         if env:
             block_rows = max(128, min(block_rows, int(env)))
@@ -471,10 +519,11 @@ def rebuild_edges(diff, denoise_models: Dict[str, torch.nn.Module], indptr: torc
             st = streams[mi % len(streams)] if streams else None
             with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
                 ws = None
+                widths = hidden_widths(den)
                 for b0 in range(r0, r1, block_rows):
                     b1 = min(b0 + block_rows, r1)
-                    if ws is None or not ws.fits(b1 - b0, n_items, H, den.time_emb_dim, split):
-                        ws = ChainWorkspace(b1 - b0, n_items, H, den.time_emb_dim, split, dev)
+                    if ws is None or not ws.fits(b1 - b0, n_items, widths, den.time_emb_dim, split):
+                        ws = ChainWorkspace(b1 - b0, n_items, widths, den.time_emb_dim, split, dev)
                     scores = denoise_chain(diff, den, csr=(indptr, indices), row0=b0, n_rows=b1 - b0,
                                            sampling_step=sampling_step, precision=precision, ws=ws, order=orders.get(b0),
                                            want_cmax=prune)

@@ -20,6 +20,9 @@ products, cosine similarity) becomes twelve tensor-pipe contractions (dmm_gemm_b
             G8  dW2 = d_out'^T (cm h) ;  dmm_transpose_bf16 -> a^T ;  G10 dW1 = dz^T [x_t', temb]
             G11 dxa = dz W1 ;  G12 dG = dxa F ;  dmm_gate_bwd_pre, dmm_atb_small, dmm_colsum -> gate / emb_layer grads
 
+A deeper denoise_dim adds, per hidden-to-hidden layer, one forward contraction (bias + tanh epilogue) and in the
+backward dh = dz W_k, dmm_hidden_bwd without a row scale, dW_k = dz^T h and dmm_colsum (DenoiseLossFn).
+
 The gradient w.r.t. the item embeddings (through ui and the reg term) is NOT produced here: the reference zeroes it
 before any optimiser step uses it (Main.py:375; SURVEY App. D.6).  Callers that need it keep the per-op path
 (GaussianDiffusion.training_losses falls back when i_embs requires grad)."""
@@ -80,13 +83,23 @@ def feature_operands(feat: torch.Tensor, i_embs: torch.Tensor, split: bool):
 
 class DenoiseLossFn(torch.autograd.Function):
     """loss_core[b] = w_t mse_b + sim_weight (1 - cos(um_b, ui_b)) (float64 [B]) for one modality and batch; gradients for
-    the eight Denoise parameters."""
+    every Denoise parameter.  ``layers`` is the flat list w_0, b_0, ..., w_{2L-1}, b_{2L-1} of the Denoise's Linear
+    layers in forward order (in_layers then out_layers; every one a Parameter autograd sees): the first maps
+    [x_t', temb] to the hidden space, the 2L - 2 inner ones map hidden to hidden (tanh after each), the last maps back
+    to the items.
+
+    Where the per-row scale cm (dL/dout = cm d_out') enters: exactly once, at the top.  The last layer's gradients take
+    it through (cm h)^T and the scaled column sum; dz of the top hidden activation is cm dh' (1 - h^2).  Every layer
+    below works on that true gradient, so its hidden_bwd runs without a row scale (cm NULL: dz = dh (1 - h^2), h^T)."""
 
     @staticmethod
-    def forward(ctx, x0, t, noise, feat, i_embs, emb_w, emb_b, w1, b1, w2, b2, gate_w, gate_b, tabs, sim_weight, precision):
+    def forward(ctx, x0, t, noise, feat, i_embs, emb_w, emb_b, gate_w, gate_b, tabs, sim_weight, precision, *layers):
         split = precision == "bf16x3"
         dev = x0.device
         B, I = x0.shape
+        weights, biases = layers[0::2], layers[1::2]
+        assert len(weights) >= 2 and len(biases) == len(weights)
+        w1, b1, w2, b2 = weights[0], biases[0], weights[-1], biases[-1]
         H, K1 = w1.shape
         d = emb_w.shape[0]
         assert K1 == I + d and w2.shape == (I, H) and feat.shape == (I, 64)
@@ -120,21 +133,30 @@ class DenoiseLossFn(torch.autograd.Function):
         ops.gate_fwd(P, gate_w.detach(), gate_b.detach(), sig, g_hi, g_lo)
         ops.gemm_bf16_tn(g_hi, g_lo, f_hi, f_lo, B, I, 64, alpha=1.0, beta=1.0, res_hi=a_hi[:, :I], res_lo=a_lo[:, :I],
                          out_hi=a_hi[:, :I], out_lo=a_lo[:, :I] if split else None)
-        # h = tanh([x_t', temb] W1^T + b1)
-        (w1_hi, w1_lo), _ = packed_weight_pair(w1, split)
-        Hp = ops.pad_to(H, 64)
-        h_hi = torch.empty((B, Hp), **bf)
-        h_lo = torch.empty((B, Hp), **bf) if split else None
-        h_f32 = torch.empty((B, ops.pad_to(H, 4)), **f32)[:, :H]      # tanh' of saturated units needs h beyond bf16 (4 MB)
-        ops.gemm_bf16_tn(a_hi, a_lo_op, w1_hi, w1_lo, B, H, I + d, bias=b1.detach(), act=1, out_f32=h_f32, out_hi=h_hi[:, :H],
-                         out_lo=h_lo[:, :H] if split else None)
+        # h = tanh([x_t', temb] W1^T + b1), then h <- tanh(h W_k^T + b_k) through the inner layers: every activation is
+        # kept as the bf16 operand (next contraction, h^T of the weight gradient) and in fp32 (tanh' of saturated units
+        # needs h beyond bf16; 4 MB each at B = 1024, width 1024)
+        acts = []
+        h_prev, h_prev_lo, k = a_hi, a_lo_op, I + d
+        for w, b in zip(weights[:-1], biases[:-1]):
+            n = w.shape[0]
+            assert w.shape[1] == k
+            (w_hi, w_lo), _ = packed_weight_pair(w, split)
+            Hp = ops.pad_to(n, 64)
+            h_hi = torch.empty((B, Hp), **bf)
+            h_lo = torch.empty((B, Hp), **bf) if split else None
+            h_f32 = torch.empty((B, ops.pad_to(n, 4)), **f32)[:, :n]
+            ops.gemm_bf16_tn(h_prev, h_prev_lo, w_hi, w_lo, B, n, k, bias=b.detach(), act=1, out_f32=h_f32,
+                             out_hi=h_hi[:, :n], out_lo=h_lo[:, :n] if split else None)
+            acts.append((h_f32, h_hi, h_lo))
+            h_prev, h_prev_lo, k = h_hi, h_lo, n
         # diff = h W2^T + b2 - x0
         (w2_hi, w2_lo), _ = packed_weight_pair(w2, split)
         diff = torch.empty((B, ops.pad_to(I, 4)), **f32)[:, :I]
         d_hi = torch.empty((B, ops.pad_to(I, 64)), **bf)
         d_lo = torch.empty((B, ops.pad_to(I, 64)), **bf) if split else None
-        ops.gemm_bf16_tn(h_hi, h_lo, w2_hi, w2_lo, B, I, H, bias=b2.detach(), alpha=1.0, beta=-1.0, residual=x0, out_f32=diff,
-                         out_hi=d_hi[:, :I], out_lo=d_lo[:, :I] if split else None)
+        ops.gemm_bf16_tn(h_prev, h_prev_lo, w2_hi, w2_lo, B, I, H, bias=b2.detach(), alpha=1.0, beta=-1.0, residual=x0,
+                         out_f32=diff, out_hi=d_hi[:, :I], out_lo=d_lo[:, :I] if split else None)
         umd = torch.empty((B, 64), **f32)
         ops.gemm_bf16_tn(d_hi, d_lo, fte_hi[:64], fte_lo[:64] if split else None, B, 64, I, out_f32=umd)
         loss = torch.empty(B, dtype=torch.float64, device=dev)
@@ -145,22 +167,34 @@ class DenoiseLossFn(torch.autograd.Function):
         ctx.split, ctx.sim_weight, ctx.dims = split, float(sim_weight), (B, I, H, d)
         ctx.tabs = tabs
         ctx.feat_ops = (f_hi, f_lo, fte_hi, fte_lo)
-        ctx.bufs = (a_hi, a_lo_op, h_f32, d_hi, d_lo, diff)
-        ctx.save_for_backward(t, P, sig, um, ui, stats, te_raw, w1, w2)
+        ctx.bufs = (a_hi, a_lo_op, acts, d_hi, d_lo, diff)
+        ctx.save_for_backward(t, P, sig, um, ui, stats, te_raw, *weights)
         ctx.mse = mse
         return loss
 
     @staticmethod
     def backward(ctx, g_loss):
-        t, P, sig, um, ui, stats, te_raw, w1, w2 = ctx.saved_tensors
+        t, P, sig, um, ui, stats, te_raw, *weights = ctx.saved_tensors
+        w1, w2 = weights[0], weights[-1]
         split = ctx.split
         B, I, H, d = ctx.dims
         f_hi, f_lo, fte_hi, fte_lo = ctx.feat_ops
-        a_hi, a_lo, h_f32, d_hi, d_lo, diff = ctx.bufs
+        a_hi, a_lo, acts, d_hi, d_lo, diff = ctx.bufs
         _, _, w_tab = ctx.tabs
         dev = t.device
         bf = dict(dtype=torch.bfloat16, device=dev)
         f32 = dict(dtype=torch.float32, device=dev)
+        Bp = ops.pad_to(B, 64)
+
+        def hidden_grad_bufs(n):
+            """dz (fp32, operand), dz^T and the transposed activation of a hidden activation of width n."""
+            Np = ops.pad_to(n, 64)
+            dz = torch.empty((B, ops.pad_to(n, 4)), **f32)[:, :n]
+            hi = (torch.empty((B, Np), **bf), torch.empty((n, Bp), **bf), torch.empty((n, Bp), **bf))
+            lo = (torch.empty((B, Np), **bf), torch.empty((n, Bp), **bf), torch.empty((n, Bp), **bf)) if split \
+                else (None, None, None)
+            return dz, hi, lo
+
         g_loss = g_loss.to(torch.float64).contiguous()
         cm = torch.empty(B, **f32)
         dumc_hi = torch.empty((B, 64), **bf)
@@ -174,22 +208,32 @@ class DenoiseLossFn(torch.autograd.Function):
         w2t_hi, w2t_lo = packed_weight(w2, True, split)                                   # W2^T [H, pad64(I)]
         dh = torch.empty((B, ops.pad_to(H, 4)), **f32)[:, :H]
         ops.gemm_bf16_tn(d_hi, d_lo, w2t_hi, w2t_lo, B, H, I, out_f32=dh)
-        Bp, Hp = ops.pad_to(B, 64), ops.pad_to(H, 64)
-        dz = torch.empty((B, ops.pad_to(H, 4)), **f32)[:, :H]
-        dz_hi = torch.empty((B, Hp), **bf)
-        dzt_hi = torch.empty((H, Bp), **bf)
-        hct_hi = torch.empty((H, Bp), **bf)
-        dz_lo, dzt_lo, hct_lo = (torch.empty((B, Hp), **bf), torch.empty((H, Bp), **bf), torch.empty((H, Bp), **bf)) if split \
-            else (None, None, None)
-        ops.hidden_bwd(dh, h_f32, None, None, cm, H, dz, dz_hi, dz_lo, dzt_hi, dzt_lo, hct_hi, hct_lo)
+        # top hidden activation: the row scale cm enters here, once
+        dz, (dz_hi, dzt_hi, hct_hi), (dz_lo, dzt_lo, hct_lo) = hidden_grad_bufs(H)
+        ops.hidden_bwd(dh, acts[-1][0], None, None, cm, H, dz, dz_hi, dz_lo, dzt_hi, dzt_lo, hct_hi, hct_lo)
         dW2 = torch.empty((I, ops.pad_to(H, 4)), **f32)[:, :H]
         ops.gemm_bf16_tn(dT_hi, dT_lo, hct_hi, hct_lo, I, H, B, out_f32=dW2)
+        grads = [(dW2.contiguous() if dW2.stride(0) != H else dW2, db2)]
+        # inner layers, top down: layer j maps activation j - 1 (width k) to activation j (width n, whose dz is at hand)
+        for j in range(len(weights) - 2, 0, -1):
+            w = weights[j]
+            n, k = w.shape
+            wt_hi, wt_lo = packed_weight(w, True, split)                                  # W_j^T [k, pad64(n)]
+            dh = torch.empty((B, ops.pad_to(k, 4)), **f32)[:, :k]
+            ops.gemm_bf16_tn(dz_hi, dz_lo, wt_hi, wt_lo, B, k, n, out_f32=dh)
+            dzp, (dzp_hi, dzpt_hi, ht_hi), (dzp_lo, dzpt_lo, ht_lo) = hidden_grad_bufs(k)
+            ops.hidden_bwd(dh, acts[j - 1][0], None, None, None, k, dzp, dzp_hi, dzp_lo, dzpt_hi, dzpt_lo, ht_hi, ht_lo)
+            dW = torch.empty((n, ops.pad_to(k, 4)), **f32)[:, :k]
+            ops.gemm_bf16_tn(dzt_hi, dzt_lo, ht_hi, ht_lo, n, k, B, out_f32=dW)
+            grads.append((dW.contiguous() if dW.stride(0) != k else dW, ops.colsum(dz, None)))
+            dz, dz_hi, dz_lo, dzt_hi, dzt_lo = dzp, dzp_hi, dzp_lo, dzpt_hi, dzpt_lo
         db1 = ops.colsum(dz, None)
         aT_hi = torch.empty((I + d, Bp), **bf)
         aT_lo = torch.empty((I + d, Bp), **bf) if split else None
         ops.transpose_bf16(a_hi, a_lo, B, I + d, aT_hi, aT_lo)
         dW1 = torch.empty((H, ops.pad_to(I + d, 4)), **f32)[:, :I + d]
         ops.gemm_bf16_tn(dzt_hi, dzt_lo, aT_hi, aT_lo, H, I + d, B, out_f32=dW1)
+        grads.append((dW1.contiguous() if dW1.stride(0) != I + d else dW1, db1))
         w1t_hi, w1t_lo = packed_weight(w1, True, split)                                   # W1^T [I + d, pad64(H)]
         dxa = torch.empty((B, ops.pad_to(I + d, 4)), **f32)[:, :I + d]
         dxa_hi = torch.empty((B, ops.pad_to(I + d, 64)), **bf)
@@ -206,16 +250,16 @@ class DenoiseLossFn(torch.autograd.Function):
         dWe = ops.atb_small(dtemb, te_raw)
         dbe = ops.colsum(dtemb, None)
         ctx.bufs = None
-        # x0, t, noise, feat, i_embs, emb_w, emb_b, w1, b1, w2, b2, gate_w, gate_b, tabs, sim_weight, precision
-        return (None, None, None, None, None, dWe, dbe, dW1.contiguous() if dW1.stride(0) != I + d else dW1, db1,
-                dW2.contiguous() if dW2.stride(0) != H else dW2, db2, dWg, dbg, None, None, None)
+        layer_grads = [g for pair in reversed(grads) for g in pair]
+        # x0, t, noise, feat, i_embs, emb_w, emb_b, gate_w, gate_b, tabs, sim_weight, precision, *layers
+        return (None, None, None, None, None, dWe, dbe, dWg, dbg, None, None, None, *layer_grads)
 
 
 def denoise_loss(diff, den, x_start, timesteps, noise, modal_feat, i_embs):
     """Fused training_losses core for one modality: (B,) float64 = w_t mse + sim_weight sim (the reg term is added by
     the caller)."""
-    lin1, lin2 = den.in_layers[0], den.out_layers[0]
     tabs = diff._train_tables(x_start.device)
+    layers = [p for layer in list(den.in_layers) + list(den.out_layers) for p in (layer.weight, layer.bias)]
     return DenoiseLossFn.apply(x_start, timesteps, noise, modal_feat, i_embs, den.emb_layer.weight, den.emb_layer.bias,
-                               lin1.weight, lin1.bias, lin2.weight, lin2.bias, den.gate_layer.weight, den.gate_layer.bias, tabs,
-                               diff.config.hyper.sim_weight, den.precision)
+                               den.gate_layer.weight, den.gate_layer.bias, tabs, diff.config.hyper.sim_weight, den.precision,
+                               *layers)

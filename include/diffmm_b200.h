@@ -423,7 +423,9 @@ int dmm_diff_loss_bwd(dmm_ctx* ctx, const double* g_loss, const float* um, const
                       uint16_t* dumc_hi, uint16_t* dumc_lo, int64_t ld_dumc, float* d_ui, void* stream);
 /* Hidden layer backward: dz = cm[r] dh (1 - h^2) as fp32, as bf16 operand [n_rows, ld_dz16], and transposed [H, ld_t]
  * together with (cm h)^T [H, ld_t]: the K = batch operands of the weight-gradient contractions.  h comes from h_f32
- * (fp32 [n_rows, ld_hf]) when given, else from h_hi (+ h_lo): tanh' of a saturated unit needs more than bf16's 8 bits. */
+ * (fp32 [n_rows, ld_hf]) when given, else from h_hi (+ h_lo): tanh' of a saturated unit needs more than bf16's 8 bits.
+ * cm NULL means no row scale: dz = dh (1 - h^2) and the transposed activation is h^T itself (the inner layers of a
+ * deeper Denoise, whose dh already carries the scale).                                                               */
 int dmm_hidden_bwd(dmm_ctx* ctx, const float* dh, int64_t ld_dh, const float* h_f32, int64_t ld_hf, const uint16_t* h_hi,
                    const uint16_t* h_lo, int64_t ld_h,
                    const float* cm, int64_t n_rows, int64_t H, float* dz_f32, int64_t ld_dz, uint16_t* dz_hi, uint16_t* dz_lo,
