@@ -141,3 +141,8 @@ def validate(cfg: Config) -> None:
     if not (isinstance(dims, list) and dims and all(type(w) is int and w > 0 for w in dims)):
         raise ValueError(f"base.denoise_dim must be a non-empty list of positive ints such as \"[1024]\", "
                          f"got {cfg.base.denoise_dim!r}")
+    # the time-embedding kernels (dmm_train_prep, dmm_time_embedding, dmm_time_bias) take widths 2 ... 64 and would
+    # reject any other one only at their first launch
+    d = cfg.base.d_emb_size
+    if not (type(d) is int and 2 <= d <= 64):
+        raise ValueError(f"base.d_emb_size must be an int in [2, 64], got {d!r}")

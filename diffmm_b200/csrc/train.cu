@@ -443,7 +443,8 @@ extern "C" int dmm_transpose_bf16(dmm_ctx* ctx, const uint16_t* src_hi, const ui
 
 extern "C" int dmm_colsum(dmm_ctx* ctx, const float* src, int64_t ld, int64_t rows, int64_t cols, const float* row_scale,
                           float* out, void* stream) {
-  DMM_CHECK_ARG(ctx && src && out, "dmm_colsum: null argument");
+  // rows == 0 (an empty batch) is a valid call that writes zeros; an empty tensor has no storage, so src may be NULL then
+  DMM_CHECK_ARG(ctx && (src || rows == 0) && out, "dmm_colsum: null argument");
   DMM_CHECK_ARG(rows >= 0 && cols > 0 && ld >= cols, "dmm_colsum: bad shape");
   colsum_kernel<<<(unsigned)dmm_ceil_div(cols, 128), 128, 0, (cudaStream_t)stream>>>(src, ld, rows, cols, row_scale, out);
   DMM_LAUNCH_CHECK();
@@ -454,7 +455,7 @@ extern "C" int64_t dmm_atb_small_workspace_floats(int64_t m, int64_t n) { return
 
 extern "C" int dmm_atb_small(dmm_ctx* ctx, const float* x, int64_t ld_x, int64_t m, const float* y, int64_t ld_y, int64_t n,
                              int64_t rows, float* workspace, float* out, void* stream) {
-  DMM_CHECK_ARG(ctx && x && y && workspace && out, "dmm_atb_small: null argument");
+  DMM_CHECK_ARG(ctx && ((x && y) || rows == 0) && workspace && out, "dmm_atb_small: null argument");   // as dmm_colsum
   DMM_CHECK_ARG(m >= 1 && m <= 64 && n >= 1 && n <= 64 && ld_x >= m && ld_y >= n && rows >= 0, "dmm_atb_small: m, n must be in [1, 64]");
   cudaStream_t st = (cudaStream_t)stream;
   atb_partial_kernel<<<dim3((unsigned)m, ATB_SPLIT), 256, 0, st>>>(x, ld_x, y, ld_y, rows, (int)m, (int)n, workspace);

@@ -434,10 +434,12 @@ int dmm_hidden_bwd(dmm_ctx* ctx, const float* dh, int64_t ld_dh, const float* h_
 /* dst[c, r] = src[r, c] for bf16 operands (hi and optionally lo); dst columns up to ld_dst are written (zero padded). */
 int dmm_transpose_bf16(dmm_ctx* ctx, const uint16_t* src_hi, const uint16_t* src_lo, int64_t ld_src, int64_t rows,
                        int64_t cols, uint16_t* dst_hi, uint16_t* dst_lo, int64_t ld_dst, void* stream);
-/* out[c] = sum_r row_scale[r] * src[r, c] (row_scale NULL = 1): bias gradients, rows added in order (deterministic). */
+/* out[c] = sum_r row_scale[r] * src[r, c] (row_scale NULL = 1): bias gradients, rows added in order (deterministic).
+   rows = 0 writes zeros; src may then be NULL. */
 int dmm_colsum(dmm_ctx* ctx, const float* src, int64_t ld, int64_t rows, int64_t cols, const float* row_scale, float* out,
                void* stream);
-/* out[m, n] = x^T y for skinny fp32 x [rows, m], y [rows, n] (m, n <= 64): gate / time-embedding weight gradients. */
+/* out[m, n] = x^T y for skinny fp32 x [rows, m], y [rows, n] (m, n <= 64): gate / time-embedding weight gradients.
+   rows = 0 writes zeros; x and y may then be NULL. */
 int64_t dmm_atb_small_workspace_floats(int64_t m, int64_t n);
 int dmm_atb_small(dmm_ctx* ctx, const float* x, int64_t ld_x, int64_t m, const float* y, int64_t ld_y, int64_t n, int64_t rows,
                   float* workspace, float* out, void* stream);

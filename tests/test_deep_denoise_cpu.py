@@ -45,6 +45,30 @@ def test_conf_rejects_bad_denoise_dim(bad):
         validate(_cfg(bad))
 
 
+@pytest.mark.parametrize("bad", [0, 1, 65, 1000, -10, 10.0, "10", True, None])
+def test_conf_rejects_bad_d_emb_size(bad):
+    """The time-embedding kernels take widths 2 ... 64; load_config must say so instead of the first kernel call."""
+    from diffmm_b200.Conf import validate
+    cfg = _cfg("[1024]")
+    cfg.base.d_emb_size = bad
+    with pytest.raises(ValueError, match="d_emb_size"):
+        validate(cfg)
+
+
+def test_conf_accepts_d_emb_size_range(tmp_path):
+    from diffmm_b200.Conf import load_config, validate
+    for ok in (2, 9, 10, 64):
+        cfg = _cfg("[1024]")
+        cfg.base.d_emb_size = ok
+        validate(cfg)
+    p = tmp_path / "x.toml"
+    p.write_text('[base]\nd_emb_size = 65\n')
+    with pytest.raises(ValueError, match="d_emb_size"):
+        load_config(str(p))
+    p.write_text('[base]\nd_emb_size = 64\n')
+    assert load_config(str(p)).base.d_emb_size == 64
+
+
 def test_load_config_rejects_bad_denoise_dim(tmp_path):
     from diffmm_b200.Conf import load_config
     p = tmp_path / "x.toml"

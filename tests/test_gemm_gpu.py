@@ -39,7 +39,9 @@ def _ref(a, b, bias, act, alpha, beta, res):
 SHAPES = [(128, 256, 64), (128, 64, 64), (128, 128, 128), (200, 300, 210), (1024, 1024, 1000), (300, 7050, 1024),
           (2048, 1024, 7060), (1024, 64, 6710), (77, 40, 50),
           # CTA-pair (cta_group::2) kernel: >= 74 tiles of 256 x 256; tail wave cut into 64-column slices; ragged M and N
-          (2048, 2560, 136), (2000, 2500, 136), (5000, 2310, 200)]
+          (2048, 2560, 136), (2000, 2500, 136), (5000, 2310, 200),
+          # K = batch < 64: the weight-gradient contractions of the fused training step on a small last batch
+          (1003, 136, 1), (136, 1003, 17), (1024, 1024, 63)]
 
 
 @pytest.mark.parametrize("M,N,K", SHAPES)
@@ -239,6 +241,55 @@ def test_tcgen05_splitk(ops, M, N, K):
     hi2 = torch.zeros_like(hi)
     ops.gemm_bf16_tn_splitk(a_d[:, :K], b_d[:, :K], M, N, K, out_hi=hi2[:, :N])
     assert torch.equal(hi2[:, :N], hi[:, :N])
+
+
+@pytest.mark.parametrize("B,I", [(1, 1003), (1, 7050), (300, 1003), (300, 7050), (1024, 1003), (1024, 7050)])
+@pytest.mark.parametrize("mode", ["bf16", "bf16x3"])
+def test_tcgen05_bf16_residual_in_place(ops, B, I, mode):
+    """The gate add of the fused training step, x_t' = x_t + G F^T, written over its own bf16 residual: out_hi / out_lo
+    alias res_hi / res_lo.  The residual is hi + lo in both modes; single-pass mode writes only hi (lo stays the
+    residual's).  The columns past N of the same rows (the time-embedding columns of the step's operand) stay as
+    they were."""
+    rng = np.random.default_rng(B + I + (mode == "bf16x3"))
+    split = mode == "bf16x3"
+    d = 10
+    ld = ops.pad_to(I + d, 64)
+    g = (rng.standard_normal((B, 64)) * 0.5).astype(np.float32)
+    f = (rng.standard_normal((I, 64)) * 0.1).astype(np.float32)
+    x = np.zeros((B, ld), dtype=np.float32)
+    x[:, :I] = rng.standard_normal((B, I))
+    x[:, I:] = rng.standard_normal((B, ld - I)) * 3.0
+    g_hi, g_lo = ops.pack_bf16(T(g))
+    f_hi, f_lo = ops.pack_bf16(T(f))
+    x_hi, x_lo = ops.pack_bf16(T(x), ld_dst=ld)
+    res = (x_hi.double() + x_lo.double())[:, :I].cpu().numpy()
+    before_hi, before_lo = x_hi.clone(), x_lo.clone()
+    # the same contraction with an fp32 output, out of place: the value the bf16 outputs must split
+    want_f32 = torch.empty((B, ops.pad_to(I, 4)), device=DEV)
+    ops.gemm_bf16_tn(g_hi, g_lo if split else None, f_hi, f_lo if split else None, B, I, 64, alpha=1.0, beta=1.0,
+                     res_hi=before_hi[:, :I], res_lo=before_lo[:, :I], out_f32=want_f32[:, :I])
+    ops.gemm_bf16_tn(g_hi, g_lo if split else None, f_hi, f_lo if split else None, B, I, 64, alpha=1.0, beta=1.0,
+                     res_hi=x_hi[:, :I], res_lo=x_lo[:, :I], out_hi=x_hi[:, :I], out_lo=x_lo[:, :I] if split else None)
+    torch.cuda.synchronize()
+    if split:
+        a = (g_hi.double() + g_lo.double())[:, :64].cpu().numpy()
+        b = (f_hi.double() + f_lo.double())[:, :64].cpu().numpy()
+    else:
+        a, b = g_hi[:, :64].double().cpu().numpy(), f_hi[:, :64].double().cpu().numpy()
+    want = a @ b.T + res
+    v = want_f32[:, :I].cpu().numpy()
+    got_hi = x_hi[:, :I].double().cpu().numpy()
+    if split:
+        np.testing.assert_allclose(v, want, rtol=1e-5, atol=5e-5)
+        rec = got_hi + x_lo[:, :I].double().cpu().numpy()
+        np.testing.assert_allclose(rec, v, rtol=2 ** -15, atol=1e-30)
+        np.testing.assert_allclose(rec, want, rtol=1e-5, atol=5e-5)
+    else:
+        np.testing.assert_allclose(v, want, rtol=1e-5, atol=2e-5)
+        np.testing.assert_allclose(got_hi, v, rtol=2 ** -8, atol=1e-30)
+        assert torch.equal(x_lo.view(torch.int16), before_lo.view(torch.int16))      # no lo output: untouched
+    assert torch.equal(x_hi[:, I:].view(torch.int16), before_hi[:, I:].view(torch.int16))
+    assert torch.equal(x_lo[:, I:].view(torch.int16), before_lo[:, I:].view(torch.int16))
 
 
 def test_tcgen05_no_epilogue_extras(ops):
