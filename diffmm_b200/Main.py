@@ -24,7 +24,7 @@ from torch import Tensor
 from torch.optim.adam import Adam
 from torch.optim.lr_scheduler import CosineAnnealingLR
 
-from . import ops, rng
+from . import ops, recommend, rng
 from .autograd import joint_losses, linear_tn, spmm, spmm_cat
 from .Conf import Config, load_config
 from .DataHandler import DataHandler
@@ -646,6 +646,72 @@ class Coach:
         n = len(testData)
         self._tick("eval", t0)
         return {"Recall": epRecall / n, "NDCG": epNdcg / n, "Precision": epPrecision / n}
+
+    def _final_embs(self):
+        """(user, item) final embeddings of gcn_MM, as testEpoch computes them for its scores."""
+        with torch.no_grad():
+            if self.has_audio:
+                out = self.model.gcn_MM(self.handler.torchBiAdj, self.image_adj, self.text_adj, self.audio_adj)
+            else:
+                out = self.model.gcn_MM(self.handler.torchBiAdj, self.image_adj, self.text_adj)
+        return out.u_final_embs, out.i_final_embs
+
+    def recommend(self, users, n, exclude_train=True):
+        """The n best items of each user in ``users`` (host ints), in rank order: (items int64 [len(users), n], scores fp32
+        [len(users), n]) on the device, score descending then item id ascending, the evaluation's bf16x3 scores.  With
+        exclude_train the user's train items are never recommended (a list with fewer than n items left ends in item -1,
+        score -inf).  Draws no random numbers and changes no parameter."""
+        U, I = self.config.data.user_num, self.config.data.item_num
+        n = recommend.check_n(n, I)
+        rid = np.asarray(users.numpy() if isinstance(users, Tensor) else users)
+        if rid.ndim != 1 or (rid.size and (rid.dtype.kind not in "iu" or rid.min() < 0 or rid.max() >= U)):
+            raise ValueError(f"users must be a 1-D sequence of user ids in 0..{U - 1}")
+        rid = rid.astype(np.int64)
+        h = self.handler
+        user_embs, item_embs = self._final_embs()
+        with torch.no_grad():
+            u = user_embs[recommend.to_device(rid, self.device)]
+            return recommend.score_topn(u, item_embs, n, exclude=(h.train_indptr, h.train_indices, rid) if exclude_train
+                                        else None, precision="bf16x3")
+
+    def evaluate(self, cutoffs=(10, 20, 50)):
+        """Recall / NDCG / Precision at every cutoff over testEpoch's test users from ONE ranked list per user: the train
+        items are masked with the reference's -1e8 (Main.py:410), the lists are ranked on the device and scored at every
+        cutoff in float64 with calcRes' arithmetic (Main.py:422-448), and the per-user values are summed on the host in the
+        reference's association (per test_batch, then across batches).  evaluate((K,)) returns exactly testEpoch()'s
+        floats under the keys "Recall@K", "NDCG@K", "Precision@K".  Unlike testEpoch it does not touch the test DataLoader:
+        it draws no random numbers and changes no parameter, so it can run between epochs of a seeded run."""
+        I = self.config.data.item_num
+        cuts = recommend.check_cutoffs(cutoffs, I)
+        N = cuts[-1]
+        testData = self.handler.testData
+        users = np.asarray(testData.test_users, dtype=np.int64)
+        n = len(users)
+        dev = self.device
+        tptr, titems = recommend.heldout_csr(users, testData.test_user_its, self.config.data.user_num)
+        inv, max_dcg = recommend.metric_tables(N)
+        h = self.handler
+        user_embs, item_embs = self._final_embs()
+        with torch.no_grad():
+            usr = recommend.to_device(users, dev)
+            ranked, _ = recommend._topn(user_embs[usr], item_embs, N, (h.train_indptr, h.train_indices, usr), -1e8, "bf16x3")
+            out = torch.empty((n, len(cuts), 3), dtype=torch.float64, device=dev)
+            ops.eval_metrics_cutoffs(ranked, N, cuts, usr, recommend.to_device(tptr, dev), recommend.to_device(titems, dev),
+                                     recommend.to_device(inv, dev), recommend.to_device(max_dcg, dev), out)
+        vals = out.cpu().numpy()             # the one host sync of the evaluation
+        tb = int(self.config.train.test_batch)
+        res = {}
+        for j, c in enumerate(cuts):
+            tot = [0, 0, 0]
+            for s in range(0, n, tb):        # the reference's association: per-batch sums, then the sum of those
+                part = [0, 0, 0]
+                for row in vals[s:s + tb, j].tolist():
+                    for m in range(3):
+                        part[m] += row[m]
+                for m in range(3):
+                    tot[m] += part[m]
+            res[f"Recall@{c}"], res[f"NDCG@{c}"], res[f"Precision@{c}"] = (t / n for t in tot)
+        return res
 
     _MAX_DCG = None
 

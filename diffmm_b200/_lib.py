@@ -120,6 +120,10 @@ PROTOTYPES = {
     "dmm_atb_small": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "dmm_eval_mask_scores": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_f32, c_vp]),
     "dmm_eval_metrics": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "dmm_eval_mask_scores_cmax": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_f32, c_vp, c_i64, c_vp]),
+    "dmm_topn_rank": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp]),
+    "dmm_eval_metrics_cutoffs": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, C.POINTER(c_i32), c_i64, c_vp, c_vp, c_vp, c_vp,
+                                           c_vp, c_vp, c_vp]),
     "dmm_bpr_infonce_workspace_floats": (c_i64, [c_i64, C.c_int, C.c_int]),
     "dmm_bpr_infonce_fwd": (C.c_int, [c_vp, C.POINTER(NceProblem), C.c_int, C.POINTER(BprProblem), c_i64, c_vp, c_vp, c_vp, c_vp,
                                       c_vp]),

@@ -604,7 +604,7 @@ void launch_reg(const float* scores, int64_t ld, int64_t n_rows, int n_cols, con
 // PRUNE_KMAX or more than n_chunks / PRUNE_RATIO, a NaN maximum, crowded ties) are appended to a device list that
 // the whole-row / segmented kernels process afterwards: every row is emitted by exactly one path, bit-identically.
 constexpr int PRUNE_KMAX = 64;
-constexpr int PRUNE_RATIO = 4;
+constexpr int PRUNE_RATIO = 4;   // diffmm_b200/recommend.py PRUNE_RATIO selects this path by the same ratio
 constexpr int PRUNE_CAND = 512;
 
 struct PruneArgs {

@@ -536,6 +536,37 @@ def eval_metrics(scores, top_items, K, row_ids, test_ptr, test_items, inv_log2, 
     return out
 
 
+def eval_mask_scores_cmax(indptr, indices, row_ids, scores, n_cols, cmax, fill=-1e8):
+    """eval_mask_scores, then the chunk maxima cmax (gemm_bf16_tn(cmax=...)) of every chunk it wrote are recomputed, so
+    topk_edges_pruned stays exact on the masked scores."""
+    assert row_ids.dtype == torch.int64 and scores.dtype == torch.float32 and cmax.dtype == torch.float32
+    _lib.call("dmm_eval_mask_scores_cmax", _ctx(scores), _p(indptr), _p(indices), _p(row_ids), int(row_ids.numel()),
+              int(n_cols), _p(scores), _row_major(scores, "scores"), float(fill), _p(cmax), _row_major(cmax, "cmax"), _stream())
+
+
+def topn_rank(scores, sel, N, items, out_scores):
+    """Row r's N selected columns sel[r, :N] (topk_edges with k = N) in rank order (score desc, column asc):
+    items int32 [rows, >= N] (-1 where the score is -inf), out_scores fp32 [rows, >= N]."""
+    assert scores.dtype == torch.float32 and sel.dtype == torch.int32 and items.dtype == torch.int32
+    assert out_scores.dtype == torch.float32
+    n_rows = sel.shape[0]
+    assert scores.shape[0] >= n_rows and items.shape[0] >= n_rows and out_scores.shape[0] >= n_rows
+    _lib.call("dmm_topn_rank", _ctx(scores), _p(scores), _row_major(scores, "scores"), n_rows, _p(sel), _row_major(sel, "sel"),
+              int(N), _p(items), _row_major(items, "items"), _p(out_scores), _row_major(out_scores, "out_scores"), _stream())
+
+
+def eval_metrics_cutoffs(ranked, N, cutoffs, row_ids, test_ptr, test_items, inv_log2, max_dcg, out):
+    """out[r, j] = (recall, ndcg, precision) at cutoffs[j] (host ints, strictly increasing, <= N) of user row_ids[r]'s
+    ranked list ranked[r, :N] in float64 (Main.py:422-448 per prefix)."""
+    assert out.dtype == torch.float64 and inv_log2.dtype == torch.float64 and max_dcg.dtype == torch.float64
+    assert ranked.dtype == torch.int32 and test_items.dtype == torch.int32 and test_ptr.dtype == torch.int64
+    assert row_ids.dtype == torch.int64 and out.is_contiguous() and out.numel() >= row_ids.numel() * len(cutoffs) * 3
+    cut = (C.c_int32 * len(cutoffs))(*[int(c) for c in cutoffs])
+    _lib.call("dmm_eval_metrics_cutoffs", _ctx(ranked), _p(ranked), _row_major(ranked, "ranked"), int(row_ids.numel()), int(N),
+              cut, len(cutoffs), _p(row_ids), _p(test_ptr), _p(test_items), _p(inv_log2), _p(max_dcg), _p(out), _stream())
+    return out
+
+
 # ----------------------------------------------------------------------------------------- fused training step
 def train_prep(x0, noise, t, tab_a, tab_b, emb_w, emb_b, a_hi, a_lo, x0_hi, te_raw):
     """x_t = tab_a[t] x0 + tab_b[t] noise and the time-embedding columns as the bf16 operand a_hi (+ a_lo); x0 as a bf16

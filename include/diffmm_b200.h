@@ -458,6 +458,33 @@ int dmm_eval_metrics(dmm_ctx* ctx, const float* scores, int64_t ld, int64_t n_ro
                      const int64_t* row_ids, const int64_t* test_ptr, const int32_t* test_items,
                      const double* inv_log2, const double* max_dcg, double* out, void* stream);
 
+/* ---- ranked recommendation lists and metrics at several cutoffs (Main.py:410-411, Main.py:422-448) -----------------
+ * dmm_eval_mask_scores_cmax: dmm_eval_mask_scores (Main.py:410), then, for every 32-column chunk of row r that holds a
+ * filled column, cmax[r * ld_cmax + c] is recomputed from the row as it now stands, exactly as dmm_gemm_epilogue.cmax
+ * builds it (max over the columns < n_cols, NaN-propagating); other chunks are left unchanged.  The chunk maxima written by
+ * the contraction stay valid upper bounds for dmm_topk_edges_pruned after the mask.  ld_cmax >= ceil(n_cols / 32).    */
+int dmm_eval_mask_scores_cmax(dmm_ctx* ctx, const int64_t* indptr, const int32_t* indices, const int64_t* row_ids,
+                              int64_t n_rows, int64_t n_cols, float* scores, int64_t ld, float fill, float* cmax,
+                              int64_t ld_cmax, void* stream);
+/* dmm_topn_rank: the torch.topk(predict, N) ranking of Main.py:411.  Row r's N columns sel[r * ld_sel + 0 .. N) (as
+ * dmm_topk_edges[_pruned] emits them, ascending) are put into rank order: score descending, then column ascending, in the
+ * top-k kernels' total order (-0.0 ties with +0.0, +NaN above +inf, -NaN below -inf), so the first k ranked entries are
+ * dmm_topk_edges' k-set for every k <= N.  items[r * ld_items + i] = the i-th column, or -1 where its score is -inf;
+ * out_scores[r * ld_out + i] = its score.  1 <= N <= 1024.                                                          */
+int dmm_topn_rank(dmm_ctx* ctx, const float* scores, int64_t ld, int64_t n_rows, const int32_t* sel, int64_t ld_sel, int64_t N,
+                  int32_t* items, int64_t ld_items, float* out_scores, int64_t ld_out, void* stream);
+/* dmm_eval_metrics_cutoffs: calcRes (Main.py:422-448) at every cutoff of the HOST array cutoffs[0 .. n_cutoffs)
+ * (strictly increasing, in 1..N) from one ranked list ranked[r * ld_ranked + 0 .. N) of user row_ids[r] (dmm_topn_rank's
+ * items).  The user's test items test_items[test_ptr[u] .. test_ptr[u+1]) are walked once in stored order; one at position
+ * p < c of the list is a hit at cutoff c and adds inv_log2[p].  out[(r * n_cutoffs + j) * 3 + 0/1/2] = recall = hits / tst,
+ * ndcg = dcg / max_dcg[min(tst, c)], precision = hits / c in float64 (recall = ndcg = 0 for a user without test items).
+ * inv_log2[p] = 1 / log2(p + 2) (p < N) and max_dcg[t] (t <= N) are host-computed float64 tables on the device.  N <= 1024.
+ * For all three, n_rows = 0 is a no-op (the device pointers may then be NULL).                                             */
+int dmm_eval_metrics_cutoffs(dmm_ctx* ctx, const int32_t* ranked, int64_t ld_ranked, int64_t n_rows, int64_t N,
+                             const int32_t* cutoffs, int64_t n_cutoffs, const int64_t* row_ids, const int64_t* test_ptr,
+                             const int32_t* test_items, const double* inv_log2, const double* max_dcg, double* out,
+                             void* stream);
+
 /* ---- host helper (no device work) --------------------------------------------------------------
  * Replays the reference's rejection-sampling loop (TrainData.negSampling, DataHandler.py:159-169)
  * over `n_draws` values pre-drawn by the caller from the same numpy generator: interaction i
