@@ -713,6 +713,69 @@ class Coach:
             res[f"Recall@{c}"], res[f"NDCG@{c}"], res[f"Precision@{c}"] = (t / n for t in tot)
         return res
 
+    def score(self, users, items):
+        """The bf16x3 scores of the pairs (users[p], items[p]) (fp32 [P] on the device; users / items: equal-length 1-D
+        integer arrays, host data or CUDA tensors).  Same terms as ``evaluate``'s scores, summed in another order
+        (recommend.score_pairs).  Draws no random numbers and changes no parameter."""
+        user_embs, item_embs = self._final_embs()
+        with torch.no_grad():
+            return recommend.score_pairs(user_embs, item_embs, users, items, precision="bf16x3")
+
+    def rank_candidates(self, users, candidates, n):
+        """Row b of ``candidates`` (int [len(users), C], -1 = empty slot) ranked for user users[b] (host ints): (items
+        int64, scores fp32) [len(users), n] on the device, score descending then item id ascending, bf16x3 scores as
+        ``score`` gives them.  Train items are not excluded: the caller chose the candidates."""
+        U = self.config.data.user_num
+        rid = np.asarray(users.numpy() if isinstance(users, Tensor) else users)
+        if rid.ndim != 1 or (rid.size and (rid.dtype.kind not in "iu" or rid.min() < 0 or rid.max() >= U)):
+            raise ValueError(f"users must be a 1-D sequence of user ids in 0..{U - 1}")
+        user_embs, item_embs = self._final_embs()
+        with torch.no_grad():
+            u = user_embs[recommend.to_device(rid.astype(np.int64), self.device)]
+            return recommend.rank_candidates(u, item_embs, candidates, n, precision="bf16x3")
+
+    def evaluate_sampled(self, n_neg=100, cutoffs=(1, 5, 10), seed=0):
+        """HR@K and NDCG@K of the sampled-negative protocol over testEpoch's test users: every (user, held-out item)
+        instance ranks its item against n_neg negatives drawn uniformly without replacement from the items in neither
+        the user's train nor its test items (recommend.sampled_candidates with np.random.default_rng(seed)).  The rows are
+        ranked on the device with bf16x3 scores (recommend.rank_candidates); a tie between the held-out item and a
+        negative goes to the smaller item id (the library's total order).  With one test item per row,
+        dmm_eval_metrics_cutoffs' Recall@K is HR@K and its NDCG@K is 1 / log2(p + 2) at position p < K.  Returns
+        {"HR@K": ..., "NDCG@K": ...} per cutoff (1 <= K <= min(1024, 1 + n_neg)), each the mean over instances summed on
+        the host in float64 in instance order.  Draws no random numbers from a global generator, does not touch the test
+        DataLoader and changes no parameter."""
+        cuts = recommend.check_cutoffs(cutoffs, 1 + recommend.check_n_neg(n_neg))
+        N = cuts[-1]
+        h = self.handler
+        testData = h.testData
+        users = np.asarray(testData.test_users, dtype=np.int64)
+        train_csr = (h.train_indptr.cpu().numpy(), h.train_indices.cpu().numpy())
+        inst_users, cand = recommend.sampled_candidates(users, testData.test_user_its, train_csr,
+                                                        self.config.data.item_num, n_neg, seed)
+        T = inst_users.size
+        if T == 0:
+            raise ValueError("the test set holds no held-out items")
+        dev = self.device
+        inv, max_dcg = recommend.metric_tables(N)
+        user_embs, item_embs = self._final_embs()
+        with torch.no_grad(), torch.cuda.device(dev):
+            u = user_embs[recommend.to_device(inst_users, dev)]
+            ranked, _ = recommend._rank_candidates(u, item_embs, recommend.to_device(cand, dev), N, "bf16x3")
+            rows = torch.arange(T, dtype=torch.int64, device=dev)
+            out = torch.empty((T, len(cuts), 3), dtype=torch.float64, device=dev)
+            ops.eval_metrics_cutoffs(ranked, N, cuts, rows, torch.arange(T + 1, dtype=torch.int64, device=dev),
+                                     recommend.to_device(np.ascontiguousarray(cand[:, 0]), dev),
+                                     recommend.to_device(inv, dev), recommend.to_device(max_dcg, dev), out)
+        vals = out.cpu().numpy()             # the one host sync of the evaluation
+        res = {}
+        for j, c in enumerate(cuts):
+            hr = ndcg = 0.0
+            for r_, g_ in vals[:, j, :2].tolist():
+                hr += r_
+                ndcg += g_
+            res[f"HR@{c}"], res[f"NDCG@{c}"] = hr / T, ndcg / T
+        return res
+
     _MAX_DCG = None
 
     def calcRes(self, top_idxs: np.ndarray, test_u_its: list, users: Tensor):

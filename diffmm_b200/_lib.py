@@ -124,7 +124,10 @@ PROTOTYPES = {
     "dmm_topn_rank": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp]),
     "dmm_eval_metrics_cutoffs": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, C.POINTER(c_i32), c_i64, c_vp, c_vp, c_vp, c_vp,
                                            c_vp, c_vp, c_vp]),
-    "dmm_bpr_infonce_workspace_floats": (c_i64, [c_i64, C.c_int, C.c_int]),
+    "dmm_score_pairs": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64, C.c_int, c_vp, c_vp]),
+    "dmm_rank_candidates": (C.c_int, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, C.c_int,
+                                      c_vp, c_i64, c_vp, c_i64, c_vp]),
+    "dmm_bpr_infonce_workspace_floats":(c_i64, [c_i64, C.c_int, C.c_int]),
     "dmm_bpr_infonce_fwd": (C.c_int, [c_vp, C.POINTER(NceProblem), C.c_int, C.POINTER(BprProblem), c_i64, c_vp, c_vp, c_vp, c_vp,
                                       c_vp]),
     "dmm_bpr_infonce_bwd": (C.c_int, [c_vp, C.POINTER(NceProblem), C.c_int, C.POINTER(BprProblem), c_i64, c_vp, c_vp, c_vp, c_vp,

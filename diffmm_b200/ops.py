@@ -555,6 +555,30 @@ def topn_rank(scores, sel, N, items, out_scores):
               int(N), _p(items), _row_major(items, "items"), _p(out_scores), _row_major(out_scores, "out_scores"), _stream())
 
 
+def score_pairs(user, item, u_idx, i_idx, x3, out):
+    """out[p] = score(user[u_idx[p]], item[i_idx[p]]) (fp32 rows; split-bf16 terms, bf16x3 when x3, else bf16); NaN for
+    an index out of range."""
+    assert user.dtype == torch.float32 and item.dtype == torch.float32 and out.dtype == torch.float32
+    assert u_idx.dtype == torch.int64 and i_idx.dtype == torch.int32 and u_idx.numel() == i_idx.numel() <= out.numel()
+    assert u_idx.is_contiguous() and i_idx.is_contiguous() and out.is_contiguous()
+    _lib.call("dmm_score_pairs", _ctx(user), _p(user), _row_major(user, "user"), user.shape[0], _p(item),
+              _row_major(item, "item"), item.shape[0], user.shape[1], _p(u_idx), _p(i_idx), u_idx.numel(), int(bool(x3)),
+              _p(out), _stream())
+    return out
+
+
+def rank_candidates(user, item, cand, N, x3, items, out_scores):
+    """Row r's candidates cand[r] (int32, -1 = empty) scored for user[r], deduplicated and ranked (score desc, item asc):
+    the first N into items int32 [rows, >= N] / out_scores fp32 [rows, >= N], (-1, -inf) past the distinct candidates."""
+    assert user.dtype == torch.float32 and item.dtype == torch.float32 and cand.dtype == torch.int32
+    assert items.dtype == torch.int32 and out_scores.dtype == torch.float32
+    n_rows = cand.shape[0]
+    assert user.shape[0] >= n_rows and items.shape[0] >= n_rows and out_scores.shape[0] >= n_rows
+    _lib.call("dmm_rank_candidates", _ctx(user), _p(user), _row_major(user, "user"), _p(item), _row_major(item, "item"),
+              item.shape[0], user.shape[1], _p(cand), _row_major(cand, "cand"), n_rows, cand.shape[1], int(N), int(bool(x3)),
+              _p(items), _row_major(items, "items"), _p(out_scores), _row_major(out_scores, "out_scores"), _stream())
+
+
 def eval_metrics_cutoffs(ranked, N, cutoffs, row_ids, test_ptr, test_items, inv_log2, max_dcg, out):
     """out[r, j] = (recall, ndcg, precision) at cutoffs[j] (host ints, strictly increasing, <= N) of user row_ids[r]'s
     ranked list ranked[r, :N] in float64 (Main.py:422-448 per prefix)."""

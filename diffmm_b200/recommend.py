@@ -8,6 +8,12 @@ rows take the whole-row top-k without chunk maxima), and dmm_topn_rank puts them
 then item id ascending (the tie order of the library's top-k).  Users are processed in chunks whose score block stays
 under 1 GB, like ``Coach.testEpoch``.  Host data enters through pinned buffers with asynchronous copies, so the call
 does not wait for work already queued on the stream.
+
+``score_pairs`` scores given (user, item) pairs and ``rank_candidates`` ranks a given candidate list per user, both
+without the full contraction (dmm_score_pairs / dmm_rank_candidates): the same split-bf16 terms, summed in fp32 in a
+fixed order, so a pair gets the same bits from both, though not score_topn's bits (the contraction sums in another
+order).  ``sampled_candidates`` builds the rows of the sampled-negative evaluation protocol (one held-out item against
+n_neg sampled negatives) on the host.
 """
 from __future__ import annotations
 
@@ -20,6 +26,7 @@ import torch
 from . import ops
 
 MAX_N = 1024          # longest ranked list (dmm_topn_rank / dmm_eval_metrics_cutoffs)
+MAX_CANDIDATES = 4096  # longest candidate row of rank_candidates (dmm_rank_candidates: one row's keys in 32 KB of shared memory)
 # score_topn takes the pruned top-k when a row has at least PRUNE_RATIO * n chunks of 32 columns, the whole-row top-k
 # otherwise.  Chosen from tools/bench_recommend.py on a B200 at 1000 W (DESIGN §7, profiles/r03_recommend.json): the
 # pruned path lost at 0.22, 0.57 and 2.2 chunks per listed item, won at 5.7, 29 and 156, and was within the run-to-run
@@ -163,6 +170,208 @@ def _topn(user_embs, item_embs, n, exclude, fill, precision):
             ops.topk_edges(sc, I, kptr, 0, None, sel[:b * n])
         ops.topn_rank(sc, sel[:b * n].view(b, n), n, items[s:s + b], scores[s:s + b])
     return items, scores
+
+
+def _check_precision(precision):
+    if precision not in ("bf16", "bf16x3"):
+        raise ValueError(f"precision must be 'bf16' or 'bf16x3', got {precision!r}")
+
+
+def _check_on_device(user_embs, item_embs):
+    if not (user_embs.is_cuda and item_embs.is_cuda) or user_embs.device != item_embs.device:
+        raise ValueError(f"user_embs and item_embs must be CUDA tensors on one device, got {user_embs.device} and "
+                         f"{item_embs.device}")
+
+
+def _ids(a, name: str, ndim: int):
+    """Integer ids as a host numpy array or a CUDA tensor (left where they are), checked for rank and dtype."""
+    if isinstance(a, torch.Tensor):
+        if a.dim() != ndim or a.dtype.is_floating_point or a.dtype.is_complex or a.dtype == torch.bool:
+            raise ValueError(f"{name} must be a {ndim}-D integer array, got {a.dtype} {tuple(a.shape)}")
+        return a if a.is_cuda else a.numpy()
+    arr = np.asarray(a)
+    if arr.ndim != ndim or (arr.size and arr.dtype.kind not in "iu"):
+        raise ValueError(f"{name} must be a {ndim}-D integer array, got {arr.dtype} {arr.shape}")
+    return arr
+
+
+def _check_ranges(checks):
+    """checks: [(ids, lo, hi, name)]: every id in [lo, hi].  Host arrays are checked on the host; the CUDA tensors are
+    reduced on the device and read back together (one synchronisation)."""
+    dev = [(a, lo, hi, name) for a, lo, hi, name in checks if isinstance(a, torch.Tensor) and a.numel()]
+    host = [(a, lo, hi, name) for a, lo, hi, name in checks if not isinstance(a, torch.Tensor) and a.size]
+    bounds = [(int(a.min()), int(a.max())) for a, *_ in host]
+    if dev:
+        mm = torch.stack([torch.stack([a.min(), a.max()]).long() for a, *_ in dev]).cpu().tolist()
+        bounds += mm
+    for (mn, mx), (_, lo, hi, name) in zip(bounds, host + dev):
+        if mn < lo or mx > hi:
+            raise ValueError(f"{name} out of range {lo}..{hi} (found {mn}..{mx})")
+
+
+def _to(a, device, dtype) -> torch.Tensor:
+    """Checked ids -> contiguous device tensor of `dtype` (host data through to_device)."""
+    if isinstance(a, torch.Tensor):
+        return a.to(device=device, dtype=dtype).contiguous()
+    return to_device(a.astype({torch.int32: np.int32, torch.int64: np.int64}[dtype]), device)
+
+
+def score_pairs(user_embs: torch.Tensor, item_embs: torch.Tensor, users, items, precision: str = "bf16x3") -> torch.Tensor:
+    """Scores of given pairs: out[p] = user_embs[users[p]] . item_embs[items[p]] (fp32 [P] on the device).
+
+    users, items: 1-D integer arrays of equal length, host data (list / numpy / CPU tensor) or CUDA tensors on the
+    embeddings' device.  Every id is checked before any launch; for CUDA ids that costs one device synchronisation.
+    precision: "bf16x3" = sum over d of hi_u hi_i + hi_u lo_i + lo_u hi_i with hi = bf16(x), lo = bf16(x - hi) (the
+    evaluation's fp32-faithful split), "bf16" = sum of hi_u hi_i; fp32 sums in a fixed order, the same bits as
+    ``rank_candidates`` gives the pair, but not bit-identical to ``score_topn`` (its contraction sums in another order)."""
+    _check_precision(precision)
+    _check_embs(user_embs, item_embs)
+    u = _ids(users, "users", 1)
+    i = _ids(items, "items", 1)
+    if u.shape[0] != i.shape[0]:
+        raise ValueError(f"users and items differ in length ({u.shape[0]} vs {i.shape[0]})")
+    check = [(u, 0, user_embs.shape[0] - 1, "users"), (i, 0, item_embs.shape[0] - 1, "items")]
+    on_dev = any(isinstance(a, torch.Tensor) for a in (u, i))
+    if not on_dev:
+        _check_ranges(check)
+    _check_on_device(user_embs, item_embs)
+    for name, a in (("users", u), ("items", i)):
+        if isinstance(a, torch.Tensor) and a.device != user_embs.device:
+            raise ValueError(f"{name} is on {a.device}, the embeddings on {user_embs.device}")
+    with torch.cuda.device(user_embs.device):
+        if on_dev:
+            _check_ranges(check)
+        dev = user_embs.device
+        out = torch.empty(u.shape[0], dtype=torch.float32, device=dev)
+        if u.shape[0]:
+            ops.score_pairs(user_embs, item_embs, _to(u, dev, torch.int64), _to(i, dev, torch.int32),
+                            precision == "bf16x3", out)
+        return out
+
+
+def rank_candidates(user_embs: torch.Tensor, item_embs: torch.Tensor, candidates, n: int,
+                    precision: str = "bf16x3") -> Tuple[torch.Tensor, torch.Tensor]:
+    """Row b's candidate items ranked for user row b: (items int64 [B, n], scores fp32 [B, n]) on the device.
+
+    candidates: int [B, C] (host data or a CUDA tensor on the embeddings' device), 1 <= C <= MAX_CANDIDATES; every entry
+    is -1 (an empty slot) or an item id, checked before any launch (one device synchronisation for CUDA input).  Rank
+    order is score descending, then item id ascending; an item listed twice in a row is ranked once, and a candidate is
+    listed with its score even if that is -inf.  Slots past the row's distinct candidates hold item -1, score -inf.
+    1 <= n <= min(MAX_N, C).  Scores as ``score_pairs`` computes them, bit for bit (``precision`` likewise)."""
+    _check_precision(precision)
+    _check_embs(user_embs, item_embs)
+    cand = _ids(candidates, "candidates", 2)
+    B, C = cand.shape
+    if B != user_embs.shape[0]:
+        raise ValueError(f"candidates has {B} rows, user_embs {user_embs.shape[0]}")
+    if C < 1 or C > MAX_CANDIDATES:
+        raise ValueError(f"candidates must have 1..{MAX_CANDIDATES} columns, got {C}")
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral):
+        raise ValueError(f"n must be an int, got {n!r}")
+    n = int(n)
+    if n < 1 or n > min(MAX_N, C):
+        raise ValueError(f"n must be in 1..{min(MAX_N, C)} (at most {MAX_N} and the {C} candidates), got {n}")
+    check = [(cand, -1, item_embs.shape[0] - 1, "candidates")]
+    on_dev = isinstance(cand, torch.Tensor)
+    if not on_dev:
+        _check_ranges(check)
+    _check_on_device(user_embs, item_embs)
+    if on_dev and cand.device != user_embs.device:
+        raise ValueError(f"candidates is on {cand.device}, the embeddings on {user_embs.device}")
+    with torch.cuda.device(user_embs.device):
+        if on_dev:
+            _check_ranges(check)
+        items, scores = _rank_candidates(user_embs, item_embs, _to(cand, user_embs.device, torch.int32), n, precision)
+        return items.long(), scores
+
+
+def _rank_candidates(user_embs, item_embs, cand, n, precision):
+    """rank_candidates without the argument checks: cand int32 on the device, int32 items."""
+    B = cand.shape[0]
+    items = torch.empty((B, n), dtype=torch.int32, device=user_embs.device)
+    scores = torch.empty((B, n), dtype=torch.float32, device=user_embs.device)
+    if B:
+        ops.rank_candidates(user_embs, item_embs, cand, n, precision == "bf16x3", items, scores)
+    return items, scores
+
+
+def check_n_neg(n_neg) -> int:
+    """Negatives per held-out item: an int in 0..MAX_CANDIDATES - 1 (a row holds the held-out item and its negatives)."""
+    if isinstance(n_neg, bool) or not isinstance(n_neg, numbers.Integral) or not 0 <= n_neg < MAX_CANDIDATES:
+        raise ValueError(f"n_neg must be an int in 0..{MAX_CANDIDATES - 1}, got {n_neg!r}")
+    return int(n_neg)
+
+
+def sampled_candidates(users, test_user_its, train_csr, n_items: int, n_neg: int, seed):
+    """Candidate rows of the sampled-negative evaluation: one row per (user, held-out item) instance, instances in the
+    order of ``users`` and then of each user's stored test items.  Column 0 is the held-out item; columns 1 .. n_neg are
+    negatives drawn uniformly without replacement (ascending) from the items in neither the user's train items
+    (train_csr = (indptr, indices), host arrays) nor its test items.  Draws come from np.random.default_rng(seed) only:
+    no global RNG state (torch, numpy, random) is read or moved.  Returns (instance users int64 [T], candidates int32
+    [T, 1 + n_neg]).  A user with fewer than n_neg eligible items raises ValueError."""
+    if isinstance(n_items, bool) or not isinstance(n_items, numbers.Integral) or n_items < 1:
+        raise ValueError(f"n_items must be a positive int, got {n_items!r}")
+    n_items, n_neg = int(n_items), check_n_neg(n_neg)
+    try:
+        indptr, indices = (np.asarray(a.cpu() if isinstance(a, torch.Tensor) else a) for a in train_csr)
+    except (TypeError, ValueError):
+        raise ValueError("train_csr must be an (indptr, indices) pair") from None
+    if indptr.ndim != 1 or indptr.size < 1 or indices.ndim != 1 or (indices.size and indices.dtype.kind not in "iu") \
+            or indptr.dtype.kind not in "iu":
+        raise ValueError("train_csr must be 1-D integer (indptr, indices) arrays")
+    usr = _ids(users.cpu() if isinstance(users, torch.Tensor) else users, "users", 1).astype(np.int64)
+    n_rows = indptr.size - 1
+    if usr.size and (usr.min() < 0 or usr.max() >= n_rows):
+        raise ValueError(f"users out of range 0..{n_rows - 1}")
+    if indices.size and (indices.min() < 0 or indices.max() >= n_items):
+        raise ValueError(f"train items out of range 0..{n_items - 1}")
+    tests = [np.asarray(test_user_its[u] if test_user_its[u] is not None else [], dtype=np.int64) for u in usr]
+    for u, t in zip(usr, tests):
+        if t.size and (t.min() < 0 or t.max() >= n_items):
+            raise ValueError(f"test items of user {u} out of range 0..{n_items - 1}")
+    counts = np.array([t.size for t in tests], dtype=np.int64)
+    inst_users = np.repeat(usr, counts)
+    pos = np.concatenate(tests) if tests else np.zeros(0, dtype=np.int64)
+    T = inst_users.size
+    cand = np.empty((T, 1 + n_neg), dtype=np.int32)
+    cand[:, 0] = pos
+    if T == 0 or n_neg == 0:
+        return inst_users, cand
+    # per user: its excluded items (train + test, sorted, distinct) and the number of eligible ones
+    excl = [np.unique(np.concatenate([indices[indptr[u]:indptr[u + 1]].astype(np.int64), t]))
+            for u, t in zip(usr, tests)]
+    n_ok = np.array([n_items - e.size for e in excl], dtype=np.int64)
+    short = np.flatnonzero((n_ok < n_neg) & (counts > 0))
+    if short.size:
+        u = int(usr[short[0]])
+        raise ValueError(f"user {u} has {int(n_ok[short[0]])} items outside its train and test items, fewer than "
+                         f"n_neg = {n_neg}")
+    # ranks among the eligible items, uniform without replacement: draw with replacement, then redraw the surplus copies
+    # of any repeated value until a row is distinct (every step treats all values alike, so the resulting set is uniform
+    # over the n_neg-subsets)
+    rng = np.random.default_rng(seed)
+    m = np.repeat(n_ok, counts)
+    ranks = np.sort(rng.integers(0, m[:, None], size=(T, n_neg)), axis=1)
+    rows = np.flatnonzero((ranks[:, 1:] == ranks[:, :-1]).any(axis=1))
+    while rows.size:
+        sub = ranks[rows]
+        dup = np.zeros(sub.shape, dtype=bool)
+        dup[:, 1:] = sub[:, 1:] == sub[:, :-1]
+        r_idx, c_idx = np.nonzero(dup)
+        sub[r_idx, c_idx] = rng.integers(0, m[rows][r_idx])
+        sub.sort(axis=1)
+        ranks[rows] = sub
+        rows = rows[(sub[:, 1:] == sub[:, :-1]).any(axis=1)]
+    # rank k of a user -> its k-th eligible item: k + #{excluded <= item}, by one search over all users' excluded lists
+    # (user j's list shifted by j * (n_items + 1) so the lists stay apart)
+    lens = np.array([e.size for e in excl], dtype=np.int64)
+    base = np.arange(usr.size, dtype=np.int64) * (n_items + 1)
+    gaps = np.concatenate([e - np.arange(e.size) for e in excl]) + np.repeat(base, lens)
+    off = np.concatenate([[0], np.cumsum(lens)[:-1]])
+    j = np.repeat(np.arange(usr.size), counts)[:, None]
+    shifted = ranks + base[j]
+    cand[:, 1:] = ranks + np.searchsorted(gaps, shifted, side="right") - off[j]
+    return inst_users, cand
 
 
 def metric_tables(n: int):

@@ -485,6 +485,28 @@ int dmm_eval_metrics_cutoffs(dmm_ctx* ctx, const int32_t* ranked, int64_t ld_ran
                              const int32_t* test_items, const double* inv_log2, const double* max_dcg, double* out,
                              void* stream);
 
+/* ---- scores of given pairs, rankings of given candidates (the user . item score of Main.py:410) --------------------
+ * Both score a (user row, item row) pair of fp32 rows (D = 1..1024, leading dimensions ld_u, ld_i >= D) the same way:
+ * each value is split in registers into hi = bf16_rn(x) and lo = bf16_rn(x - hi) (the operands of dmm_pack_bf16), and
+ * score = sum over d of hi_u hi_i + hi_u lo_i + lo_u hi_i (x3 = 1, bf16x3) or of hi_u hi_i (x3 = 0, bf16), accumulated
+ * in fp32 in a fixed order, so a pair gets the same bits from either function; a zero score is +0.0.  These are the
+ * terms of the tensor-pipe contraction (dmm_gemm_bf16_tn), but not its bits: the summation order differs.
+ * dmm_score_pairs: out[p] = score(user[u_idx[p]], item[i_idx[p]]) for p < P; a pair with u_idx outside [0, n_users) or
+ * i_idx outside [0, n_items) gets NaN and reads no row.
+ * dmm_rank_candidates: row r (< n_rows) ranks the candidates cand[r * ld_c + 0 .. C) for user row r in one launch, in
+ * the top-k kernels' total order (score descending, then item ascending; -0.0 ties with +0.0, +NaN above +inf, -NaN
+ * below -inf).  -1 or any id outside [0, n_items) is an empty slot; an item listed several times is ranked once.  The
+ * first N ranked items go to out_items[r * ld_oi + i] with their scores in out_scores[r * ld_os + i], a score of -inf
+ * included; only the slots past the row's distinct valid candidates hold (-1, -inf).  1 <= C <= 4096,
+ * 1 <= N <= min(1024, C).  No score but the N emitted reaches global memory.
+ * For both, zero pairs / rows is a no-op (the device pointers may then be NULL).                                      */
+int dmm_score_pairs(dmm_ctx* ctx, const float* user, int64_t ld_u, int64_t n_users, const float* item, int64_t ld_i,
+                    int64_t n_items, int64_t D, const int64_t* u_idx, const int32_t* i_idx, int64_t P, int x3, float* out,
+                    void* stream);
+int dmm_rank_candidates(dmm_ctx* ctx, const float* user, int64_t ld_u, const float* item, int64_t ld_i, int64_t n_items,
+                        int64_t D, const int32_t* cand, int64_t ld_c, int64_t n_rows, int64_t C, int64_t N, int x3,
+                        int32_t* out_items, int64_t ld_oi, float* out_scores, int64_t ld_os, void* stream);
+
 /* ---- host helper (no device work) --------------------------------------------------------------
  * Replays the reference's rejection-sampling loop (TrainData.negSampling, DataHandler.py:159-169)
  * over `n_draws` values pre-drawn by the caller from the same numpy generator: interaction i
