@@ -55,6 +55,33 @@ def _row_major(t: torch.Tensor, name: str) -> int:
     return t.stride(0) if t.shape[0] > 1 else max(t.stride(0), t.shape[1])
 
 
+def _f32_vector(t, n: int, name: str):
+    """Checks that t is a contiguous 1-D fp32 tensor of exactly n elements: the kernels read it through a raw pointer."""
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or t.dim() != 1 or not t.is_contiguous():
+        raise ValueError(f"{name}: expected a contiguous 1-D float32 tensor, got "
+                         f"{getattr(t, 'dtype', type(t).__name__)} {tuple(getattr(t, 'shape', ()))}")
+    if t.numel() != n:
+        raise ValueError(f"{name}: expected {n} elements, got {t.numel()}")
+
+
+def _f32_matrix(t, name: str):
+    """Checks that t is a 2-D fp32 tensor with unit inner stride and returns its leading dimension."""
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+        raise ValueError(f"{name}: expected a float32 tensor, got {getattr(t, 'dtype', type(t).__name__)}")
+    return _row_major(t, name)
+
+
+def _time_emb_weights(emb_w, emb_b) -> int:
+    """The d x d time-embedding Linear (weight row-major and dense, as the kernels index it): returns d."""
+    if not isinstance(emb_w, torch.Tensor) or emb_w.dtype != torch.float32 or emb_w.dim() != 2 \
+            or emb_w.shape[0] != emb_w.shape[1] or not emb_w.is_contiguous():
+        raise ValueError(f"emb_w: expected a contiguous square float32 matrix, got "
+                         f"{getattr(emb_w, 'dtype', type(emb_w).__name__)} {tuple(getattr(emb_w, 'shape', ()))}")
+    d = emb_w.shape[0]
+    _f32_vector(emb_b, d, "emb_b")
+    return d
+
+
 # ----------------------------------------------------------------------------------------- packing
 def pack_bf16(src: torch.Tensor, ld_dst: Optional[int] = None, transpose: bool = False, split: bool = True):
     """fp32 [R, C] -> (hi, lo) bf16 [R, ld] (or [C, ld] transposed); lo is None when split=False."""
@@ -100,7 +127,7 @@ def csr_rows_to_dense(indptr, indices, n_rows, n_cols, *, row_ids=None, row0=0, 
 
 
 def time_embedding(emb_w, emb_b, n_rows, *, t=None, t_all=0, a_hi=None, a_lo=None, col0=0, temb_f32=None):
-    d = emb_w.shape[0]
+    d = _time_emb_weights(emb_w, emb_b)
     ld_a = _row_major(a_hi, "a_hi") if a_hi is not None else 0
     _lib.call("dmm_time_embedding", _ctx(emb_w), _p(t), int(t_all), int(n_rows), int(d), _p(emb_w), _p(emb_b),
               _p(a_hi), _p(a_lo), ld_a, int(col0), _p(temb_f32), _stream())
@@ -109,13 +136,18 @@ def time_embedding(emb_w, emb_b, n_rows, *, t=None, t_all=0, a_hi=None, a_lo=Non
 def time_bias(emb_w, emb_b, weight, col0, bias, t0, n_t=1, out=None):
     """bias_eff[i] = bias + weight[:, col0:col0+d] @ temb(t0 + i), i < n_t (fp32 [n_t, H]); weight is the fp32
     [H, K] Linear weight."""
-    d = emb_w.shape[0]
+    d = _time_emb_weights(emb_w, emb_b)
+    ld_w = _f32_matrix(weight, "weight")
     H = weight.shape[0]
+    if not 0 <= col0 <= weight.shape[1] - d:
+        raise ValueError(f"weight: columns col0 .. col0 + d = {col0} .. {col0 + d} outside its {weight.shape[1]} columns")
+    if bias is not None:
+        _f32_vector(bias, H, "bias")
     if out is None:
         out = torch.empty((n_t, H), dtype=torch.float32, device=weight.device)
     assert out.is_contiguous() and out.numel() >= n_t * H
     _lib.call("dmm_time_bias", _ctx(weight), int(t0), int(n_t), int(d), _p(emb_w), _p(emb_b), _p(weight),
-              _row_major(weight, "weight"), int(col0), _p(bias), H, _p(out), _stream())
+              ld_w, int(col0), _p(bias), H, _p(out), _stream())
     return out
 
 
@@ -179,17 +211,25 @@ def rows_long_first(indptr, row0, n_rows, threshold=32):
 
 def gemv_f32(w, K, x, out=None):
     """y = w[:, :K] @ x (fp32)."""
+    ld_w = _f32_matrix(w, "w")
     n_rows = w.shape[0]
+    if not 0 < K <= w.shape[1]:
+        raise ValueError(f"K = {K} outside 1..{w.shape[1]} (the columns of w)")
+    _f32_vector(x, K, "x")
     if out is None:
         out = torch.empty(n_rows, dtype=torch.float32, device=w.device)
-    _lib.call("dmm_gemv_f32", _ctx(w), _p(w), _row_major(w, "w"), int(n_rows), int(K), _p(x), _p(out), _stream())
+    _f32_vector(out, n_rows, "out")
+    _lib.call("dmm_gemv_f32", _ctx(w), _p(w), ld_w, int(n_rows), int(K), _p(x), _p(out), _stream())
     return out
 
 
 def bias_act_pack(z, bias, act, h_hi, h_lo=None):
     """h = act(z + bias) -> bf16 hi (+ lo)."""
+    ld_z = _f32_matrix(z, "z")
     n_rows, n_cols = z.shape
-    _lib.call("dmm_bias_act_pack", _ctx(z), _p(z), _row_major(z, "z"), _p(bias), int(n_rows), int(n_cols), int(act), _p(h_hi),
+    if bias is not None:
+        _f32_vector(bias, n_cols, "bias")
+    _lib.call("dmm_bias_act_pack", _ctx(z), _p(z), ld_z, _p(bias), int(n_rows), int(n_cols), int(act), _p(h_hi),
               _p(h_lo), _row_major(h_hi, "h_hi"), _stream())
 
 
