@@ -480,6 +480,10 @@ __global__ void __launch_bounds__(256) scatter_add_rows_kernel(const float* __re
   for (int c = lane; c < D; c += 32) atomicAdd(dst + r * ld_d + c, __ldg(src + b * ld_s + c));
 }
 
+// the widths nce_rows_kernel is instantiated for (D / 32 picks the instance, so any other D must be refused up front:
+// D = 48 would otherwise run the D = 32 kernel on rows of stride 48)
+inline bool nce_supported_d(int64_t D) { return D == 32 || D == 64 || D == 128 || D == 256; }
+
 template <int MODE>
 int launch_nce(int64_t B, int64_t D, const float* na, const float* nb, float inv_temp, const float* lse_in,
                const float* inv_norm, float coef, float* out_lse, float* out_row_loss, float* out_grad,
@@ -522,6 +526,7 @@ extern "C" int dmm_infonce_fwd(dmm_ctx* ctx, const float* v1, int64_t ld1, const
   DMM_CHECK_ARG(ctx && v1 && v2 && idx && workspace && row_loss && loss && lse && inv1 && inv2,
                 "dmm_infonce_fwd: null argument");
   DMM_CHECK_ARG(B > 0 && temperature > 0.f, "dmm_infonce_fwd: bad B or temperature");
+  DMM_CHECK_ARG(nce_supported_d(D), "InfoNCE: D must be 32, 64, 128 or 256 (got %lld)", (long long)D);
   DMM_CHECK_ARG(ld1 >= D && ld2 >= D, "dmm_infonce_fwd: leading dimension < D");
   cudaStream_t st = (cudaStream_t)stream;
   float* n1 = workspace;
@@ -557,6 +562,8 @@ extern "C" int dmm_infonce_bwd(dmm_ctx* ctx, const float* v1, int64_t ld1, const
                                float* g2, void* stream) {
   DMM_CHECK_ARG(ctx && v1 && v2 && idx && lse && inv1 && inv2 && workspace && g1 && g2, "dmm_infonce_bwd: null argument");
   DMM_CHECK_ARG(B > 0 && temperature > 0.f, "dmm_infonce_bwd: bad B or temperature");
+  DMM_CHECK_ARG(nce_supported_d(D), "InfoNCE: D must be 32, 64, 128 or 256 (got %lld)", (long long)D);
+  DMM_CHECK_ARG(ld1 >= D && ld2 >= D, "dmm_infonce_bwd: leading dimension < D");
   cudaStream_t st = (cudaStream_t)stream;
   float* n1 = workspace;
   float* n2 = workspace + B * D;

@@ -470,7 +470,8 @@ __global__ void __launch_bounds__(256, B16 ? 4 : 3) spmm64_units_kernel(const in
             q[t] = __ldg(reinterpret_cast<const float4*>(tl + (size_t)c * row_bytes));
           }
 #pragma unroll
-          for (int t = 0; t < 8; ++t) a4 = fma4(v[t], q[t], a4);      // v = 0 beyond this unit's entries
+          for (int t = 0; t < 8; ++t)
+            if (t < n) a4 = fma4(v[t], q[t], a4);      // beyond this unit's entries: column 0 with value 0 (0 * inf = NaN)
         } else {
 #pragma unroll
           for (int t = 0; t < 7; ++t)
@@ -481,7 +482,7 @@ __global__ void __launch_bounds__(256, B16 ? 4 : 3) spmm64_units_kernel(const in
             }
 #pragma unroll
           for (int t = 0; t < 7; ++t)
-            if (t < nw) a4 = fma4(v[t], q[t], a4);
+            if (t < nw && t < n) a4 = fma4(v[t], q[t], a4);
         }
         acc[0] = a4.x, acc[1] = a4.y, acc[2] = a4.z, acc[3] = a4.w;
       }

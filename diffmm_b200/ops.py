@@ -71,6 +71,24 @@ def _f32_matrix(t, name: str):
     return _row_major(t, name)
 
 
+def _f32_rows(t, n_cols: int, name: str):
+    """_f32_matrix with exactly n_cols columns (the kernels read that many per row); returns the leading dimension."""
+    ld = _f32_matrix(t, name)
+    if t.shape[1] != n_cols:
+        raise ValueError(f"{name}: expected {n_cols} columns, got shape {tuple(t.shape)}")
+    return ld
+
+
+def _i64_index(t, n: Optional[int], name: str):
+    """Checks that t is a contiguous 1-D int64 tensor (of n elements unless n is None): the kernels read int64 row ids
+    through a raw pointer, so an int32 tensor would be read as half as many ids of garbage."""
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.int64 or t.dim() != 1 or not t.is_contiguous():
+        raise ValueError(f"{name}: expected a contiguous 1-D int64 tensor, got "
+                         f"{getattr(t, 'dtype', type(t).__name__)} {tuple(getattr(t, 'shape', ()))}")
+    if n is not None and t.numel() != n:
+        raise ValueError(f"{name}: expected {n} elements, got {t.numel()}")
+
+
 def _time_emb_weights(emb_w, emb_b) -> int:
     """The d x d time-embedding Linear (weight row-major and dense, as the kernels index it): returns d."""
     if not isinstance(emb_w, torch.Tensor) or emb_w.dtype != torch.float32 or emb_w.dim() != 2 \
@@ -458,6 +476,10 @@ def spmm_replan(adj: CsrAdj):
 
 def sign_noise_(e: torch.Tensor, rnd: torch.Tensor, noise_degree: float):
     """In place e += sign(e) * normalize_rows(rnd) * noise_degree (Main.py:320-321)."""
+    _f32_matrix(e, "e")
+    _f32_matrix(rnd, "rnd")
+    if rnd.shape != e.shape:
+        raise ValueError(f"rnd: expected the shape of e {tuple(e.shape)}, got {tuple(rnd.shape)}")
     _lib.call("dmm_sign_noise_", _ctx(e), _p(e), _row_major(e, "e"), _p(rnd), _row_major(rnd, "rnd"), e.shape[0],
               e.shape[1], float(noise_degree), _stream())
     return e
@@ -475,7 +497,12 @@ def rownorm_fwd(x: torch.Tensor, eps: float = 1e-12):
 
 
 def rownorm_bwd(y: torch.Tensor, inv: torch.Tensor, g: torch.Tensor):
-    gx = torch.empty_like(y)
+    _f32_matrix(y, "y")
+    _f32_rows(g, y.shape[1], "g")
+    if g.shape[0] != y.shape[0]:
+        raise ValueError(f"g: expected the shape of y {tuple(y.shape)}, got {tuple(g.shape)}")
+    _f32_vector(inv, y.shape[0], "inv")
+    gx = torch.empty((y.shape[0], y.shape[1]), dtype=torch.float32, device=y.device)
     _lib.call("dmm_rownorm_bwd", _ctx(y), _p(y), _row_major(y, "y"), _p(inv), _p(g), _row_major(g, "g"), y.shape[0], y.shape[1],
               _p(gx), gx.shape[1], _stream())
     return gx
@@ -486,15 +513,35 @@ def _ptr_array(tensors):
 
 
 def _dense(t: torch.Tensor, name: str) -> torch.Tensor:
-    if not t.is_contiguous() or t.dtype != torch.float32:
-        raise _lib.DiffMMError(f"{name}: dense contiguous fp32 tensor expected")
+    if not isinstance(t, torch.Tensor) or not t.is_contiguous() or t.dtype != torch.float32:
+        raise ValueError(f"{name}: dense contiguous fp32 tensor expected")
     return t
+
+
+_MIX_MAX_M = 4          # PROP_MAX_M of csrc/prop.cu
+
+
+def _mix_operands(y, zs, w, g=None):
+    """The modality mix reads y, every z_m (and g) as one flat dense fp32 array of y's size and w as M floats."""
+    y = _dense(y, "y")
+    zs = list(zs)
+    if not 1 <= len(zs) <= _MIX_MAX_M:
+        raise ValueError(f"zs: 1 .. {_MIX_MAX_M} modalities, got {len(zs)}")
+    for m, z in enumerate(zs):
+        _dense(z, f"z[{m}]")
+        if z.shape != y.shape:
+            raise ValueError(f"z[{m}]: expected the shape of y {tuple(y.shape)}, got {tuple(z.shape)}")
+    if g is not None:
+        _dense(g, "g")
+        if g.shape != y.shape:
+            raise ValueError(f"g: expected the shape of y {tuple(y.shape)}, got {tuple(g.shape)}")
+    _f32_vector(w, len(zs), "w")
+    return y, zs
 
 
 def modal_mix_fwd(y: torch.Tensor, zs, w: torch.Tensor, lam: float):
     """sum_m w[m] (y + lam zs[m]) (Model.py:116-119,125-127); w: device fp32 [M]."""
-    y = _dense(y, "y")
-    zs = [_dense(z, "z") for z in zs]
+    y, zs = _mix_operands(y, zs, w)
     out = torch.empty_like(y)
     arr = _ptr_array(zs)
     _lib.call("dmm_modal_mix_fwd", _ctx(y), _p(y), arr, _p(w), len(zs), float(lam), y.numel(), _p(out), _stream())
@@ -503,7 +550,7 @@ def modal_mix_fwd(y: torch.Tensor, zs, w: torch.Tensor, lam: float):
 
 def modal_mix_bwd(g: torch.Tensor, y: torch.Tensor, zs, w: torch.Tensor, lam: float, need_gz=True):
     """Returns (gy, [gz_m], gw [M]) of modal_mix_fwd; gw from per-CTA partial sums added in a fixed order."""
-    g = _dense(g, "g")
+    y, zs = _mix_operands(y, zs, w, g)
     M = len(zs)
     gy = torch.empty_like(y)
     gzs = [torch.empty_like(y) if need_gz else None for _ in range(M)]
@@ -516,7 +563,11 @@ def modal_mix_bwd(g: torch.Tensor, y: torch.Tensor, zs, w: torch.Tensor, lam: fl
 
 # ----------------------------------------------------------------------------------------- losses
 def bpr_fwd_bwd(u_emb, i_emb, users, pos, neg, grad_scale=1.0, want_grad=True):
+    _f32_matrix(u_emb, "u_emb")
     B, D = users.numel(), u_emb.shape[1]
+    _f32_rows(i_emb, D, "i_emb")
+    for t, name in ((users, "users"), (pos, "pos"), (neg, "neg")):
+        _i64_index(t, B, name)
     dev = u_emb.device
     row_loss = torch.empty(B, dtype=torch.float32, device=dev)
     loss = torch.empty((), dtype=torch.float32, device=dev)
@@ -527,8 +578,15 @@ def bpr_fwd_bwd(u_emb, i_emb, users, pos, neg, grad_scale=1.0, want_grad=True):
     return loss, g
 
 
+def _infonce_operands(v1, v2, idx):
+    _f32_matrix(v1, "v1")
+    _f32_rows(v2, v1.shape[1], "v2")
+    _i64_index(idx, None, "idx")
+    return idx.numel(), v1.shape[1]
+
+
 def infonce_fwd(v1, v2, idx, temperature):
-    B, D = idx.numel(), v1.shape[1]
+    B, D = _infonce_operands(v1, v2, idx)
     dev = v1.device
     ws = torch.empty(int(_lib.load().dmm_infonce_workspace_floats(B, D, 0)), dtype=torch.float32, device=dev)
     row_loss = torch.empty(B, dtype=torch.float32, device=dev)
@@ -542,9 +600,11 @@ def infonce_fwd(v1, v2, idx, temperature):
 
 
 def infonce_bwd(v1, v2, idx, temperature, saved, grad_scale=1.0):
-    B, D = idx.numel(), v1.shape[1]
+    B, D = _infonce_operands(v1, v2, idx)
     dev = v1.device
     lse, inv1, inv2 = saved
+    for t, name in ((lse, "lse"), (inv1, "inv1"), (inv2, "inv2")):
+        _f32_vector(t, B, name)
     ws = torch.empty(int(_lib.load().dmm_infonce_workspace_floats(B, D, 1)), dtype=torch.float32, device=dev)
     g1 = torch.empty((B, D), dtype=torch.float32, device=dev)
     g2 = torch.empty((B, D), dtype=torch.float32, device=dev)
@@ -554,6 +614,10 @@ def infonce_bwd(v1, v2, idx, temperature, saved, grad_scale=1.0):
 
 
 def scatter_add_rows(src, idx, dst):
+    """dst[idx[b]] += src[b] (atomic adds: indices may repeat)."""
+    _f32_matrix(src, "src")
+    _i64_index(idx, src.shape[0], "idx")
+    _f32_rows(dst, src.shape[1], "dst")
     _lib.call("dmm_scatter_add_rows", _ctx(src), _p(src), _row_major(src, "src"), _p(idx), idx.numel(), src.shape[1],
               _p(dst), _row_major(dst, "dst"), _stream())
     return dst
@@ -700,19 +764,28 @@ def atb_small(x, y):
 
 
 # ----------------------------------------------------------------------------------------- fused BPR + InfoNCE
-def _loss_structs(tables, problems, bpr):
-    """problems: [(i1, i2, idx, row_offset, temperature, weight)] over `tables`; bpr: (i_table, item_offset, users, pos, neg)."""
+_NCE_MAX_PROBLEMS = 12  # NCE_MAX_PROBLEMS of csrc/loss.cu
+
+
+def _loss_structs(tables, problems, bpr, B):
+    """problems: [(i1, i2, idx, row_offset, temperature, weight)] over `tables`; bpr: (i_table, item_offset, users, pos, neg).
+    The kernels read 64 columns of every view and B int64 ids from every index tensor."""
     P = len(problems)
+    if not 1 <= P <= _NCE_MAX_PROBLEMS:
+        raise ValueError(f"problems: 1 .. {_NCE_MAX_PROBLEMS} InfoNCE problems, got {P}")
     arr = (_lib.NceProblem * P)()
     for k, (i1, i2, idx, off, temp, weight) in enumerate(problems):
         a, b = tables[i1], tables[i2]
-        arr[k].v1, arr[k].ld1 = a.data_ptr(), _row_major(a, "view")
-        arr[k].v2, arr[k].ld2 = b.data_ptr(), _row_major(b, "view")
+        arr[k].v1, arr[k].ld1 = a.data_ptr(), _f32_rows(a, 64, f"tables[{i1}]")
+        arr[k].v2, arr[k].ld2 = b.data_ptr(), _f32_rows(b, 64, f"tables[{i2}]")
+        _i64_index(idx, B, f"problems[{k}] idx")
         arr[k].idx, arr[k].row_offset = idx.data_ptr(), int(off)
         arr[k].temperature, arr[k].weight = float(temp), float(weight)
     it, item_off, users, pos, neg = bpr
+    for t, name in ((users, "users"), (pos, "pos"), (neg, "neg")):
+        _i64_index(t, B, name)
     bp = _lib.BprProblem()
-    bp.emb, bp.ld_emb, bp.item_offset = tables[it].data_ptr(), _row_major(tables[it], "emb"), int(item_off)
+    bp.emb, bp.ld_emb, bp.item_offset = tables[it].data_ptr(), _f32_rows(tables[it], 64, f"tables[{it}]"), int(item_off)
     bp.users, bp.pos, bp.neg = users.data_ptr(), pos.data_ptr(), neg.data_ptr()
     return arr, bp
 
@@ -722,7 +795,7 @@ def bpr_infonce_fwd(tables, problems, bpr, B):
     total; saved = (lse [P, B], inv [P, 2, B]))."""
     P = len(problems)
     dev = tables[0].device
-    arr, bp = _loss_structs(tables, problems, bpr)
+    arr, bp = _loss_structs(tables, problems, bpr, B)
     ws = torch.empty(int(_lib.load().dmm_bpr_infonce_workspace_floats(B, P, 0)), dtype=torch.float32, device=dev)
     losses = torch.empty(P + 2, dtype=torch.float32, device=dev)
     lse = torch.empty((P, B), dtype=torch.float32, device=dev)
@@ -735,8 +808,22 @@ def bpr_infonce_bwd(tables, problems, bpr, B, saved, g_cl, g_bpr, grad_tables):
     """Scatter-adds d(g_bpr BPR + g_cl total) into grad_tables (one zeroed fp32 [N, 64] tensor or None per table)."""
     P = len(problems)
     dev = tables[0].device
-    arr, bp = _loss_structs(tables, problems, bpr)
+    arr, bp = _loss_structs(tables, problems, bpr, B)
     lse, inv = saved
+    for t, n, name in ((lse, P * B, "lse"), (inv, P * 2 * B, "inv"), (g_cl, 1, "g_cl"), (g_bpr, 1, "g_bpr")):
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != n:
+            raise ValueError(f"{name}: expected a contiguous float32 tensor of {n} elements, got "
+                             f"{getattr(t, 'dtype', type(t).__name__)} {tuple(getattr(t, 'shape', ()))}")
+
+    def grad_ld(it):
+        g = grad_tables[it]
+        if g is None:
+            return 0
+        ld = _f32_rows(g, 64, f"grad_tables[{it}]")
+        if g.shape[0] != tables[it].shape[0]:
+            raise ValueError(f"grad_tables[{it}]: expected {tables[it].shape[0]} rows (those of tables[{it}]), got {g.shape[0]}")
+        return ld
+
     ws = torch.empty(int(_lib.load().dmm_bpr_infonce_workspace_floats(B, P, 1)), dtype=torch.float32, device=dev)
     ptrs = (C.c_void_p * (2 * P + 1))()
     lds = (C.c_int64 * (2 * P + 1))()
@@ -745,9 +832,9 @@ def bpr_infonce_bwd(tables, problems, bpr, B, saved, g_cl, g_bpr, grad_tables):
         for s, it in enumerate((i1, i2)):
             g = grad_tables[it]
             ptrs[2 * k + s] = g.data_ptr() if g is not None else None
-            lds[2 * k + s] = _row_major(g, "grad") if g is not None else 0
+            lds[2 * k + s] = grad_ld(it)
     gb = grad_tables[bpr[0]]
     ptrs[2 * P] = gb.data_ptr() if gb is not None else None
-    lds[2 * P] = _row_major(gb, "grad") if gb is not None else 0
+    lds[2 * P] = grad_ld(bpr[0])
     _lib.call("dmm_bpr_infonce_bwd", _ctx(tables[0]), arr, P, C.byref(bp), int(B), _p(lse), _p(inv), _p(g_cl), _p(g_bpr), _p(ws),
               ptrs, lds, _stream())
