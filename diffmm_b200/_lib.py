@@ -56,8 +56,7 @@ PROTOTYPES = {
                                      c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp]),
     "dmm_csr_gather_act_split": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64,
                                            c_vp, C.c_int, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp]),
-    "dmm_csr_qsample_values_rng": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_f32, c_f32, c_vp, C.c_int,
-                                             c_vp]),
+    "dmm_csr_qsample_values_rng": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_f32, c_f32, c_vp, c_vp]),
     "dmm_csr_qsample_values": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_f32, c_f32, c_vp, c_vp]),
     "dmm_rows_long_first": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "dmm_gemv_f32": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),

@@ -15,8 +15,6 @@
 // ("bf16x3"), which restores fp32-level accuracy without leaving the bf16 tensor pipe.
 #include "common.cuh"
 
-#include <stdlib.h>
-
 namespace {
 
 constexpr int BLOCK_M = 128;
@@ -1056,10 +1054,8 @@ int launch(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda
   if (tepi) {
     // Shared-memory layout of the TMA epilogue.  With an fp32 residual every epilogue warp owns a ring of chunk buffers
     // (prefetch depth nbuf - 1) and the operand ring takes what is left; otherwise one staging buffer per warp.
-    static const int env_nbuf = []() { const char* e = getenv("DMM_GEMM_NBUF"); return e ? atoi(e) : 0; }();
     const bool has_res = p.ep.residual != nullptr;
     p.nbuf = has_res ? 2 : 1;   // measured: a 4-stage operand ring + 2 chunk buffers beats 3 stages + 3 buffers
-    if (has_res && env_nbuf >= 2 && env_nbuf <= TEPI_MAX_BUF) p.nbuf = env_nbuf;
     const int f32_bytes = EPI_WARPS * p.nbuf * 4096;
     const int b16_bytes = p.ep.out_hi ? EPI_WARPS * 2048 : 0;
     const int bias_bytes = EPI_WARPS * 256;
@@ -1270,8 +1266,6 @@ int run_gemm(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t l
 
   // Tile shape by a small cost model: waves over the SMs (or SM pairs) x work per SM and wave / measured relative
   // efficiency of the shape (256-wide pair tiles 1.0, single-CTA 256 / 128 / 64 columns 0.93 / 0.80 / 0.55).
-  // DMM_GEMM_PAIR=0 keeps the single-CTA kernels (A/B switch for measurements).
-  static const bool pair_ok = []() { const char* e = getenv("DMM_GEMM_PAIR"); return !(e && e[0] == '0'); }();
   const int64_t m128 = dmm_ceil_div(M, BLOCK_M), m256 = dmm_ceil_div(M, 2 * BLOCK_M);
   auto waves = [](int64_t tiles, int64_t slots) { return (double)dmm_ceil_div(tiles, slots); };
   const int sms = ctx->num_sms;
@@ -1285,25 +1279,16 @@ int run_gemm(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t l
   if (N > 64) consider(128, false, waves(m128 * dmm_ceil_div(N, 128), sms) * 128.0 / 0.80);
   if (N > 128) {
     consider(256, false, waves(m128 * dmm_ceil_div(N, 256), sms) * 256.0 / 0.93);
-    if (pair_ok && sms >= 2) consider(256, true, waves(m256 * dmm_ceil_div(N, 256), sms / 2) * 256.0 / 1.0);
-  }
-  // DMM_GEMM_BN=64|128|256 (with DMM_GEMM_PAIR) overrides the cost model (tile-shape experiments)
-  static const int force_bn = []() { const char* e = getenv("DMM_GEMM_BN"); return e ? atoi(e) : 0; }();
-  if (force_bn == 64 || force_bn == 128 || force_bn == 256) {
-    static const bool force_pair = []() { const char* e = getenv("DMM_GEMM_PAIR"); return e && e[0] == '1'; }();
-    bn = force_bn;
-    pair = force_bn == 256 && force_pair;
+    if (sms >= 2) consider(256, true, waves(m256 * dmm_ceil_div(N, 256), sms / 2) * 256.0 / 1.0);
   }
   if (p.ksplit > 1) {
     bn = 256;
     pair = true;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  // TMA epilogue (residual prefetch ring + bulk tensor stores) for the single-pass bf16 configurations;
-  // DMM_GEMM_TEPI=0 keeps the register-staged epilogue (A/B switch for measurements)
-  static const bool tepi_ok = []() { const char* e = getenv("DMM_GEMM_TEPI"); return !(e && e[0] == '0'); }();
-  const bool tepi = (tepi_ok || p.ksplit > 1) && !a_lo && !b_lo && !ep->res_hi && !ep->res_lo && !ep->out_lo &&
-                    (ep->out_f32 || ep->out_hi);
+  // TMA epilogue (residual prefetch ring + bulk tensor stores) for the single-pass bf16 configurations; the
+  // register-staged epilogue serves the rest (split-bf16 operands, bf16 residual or lo output)
+  const bool tepi = !a_lo && !b_lo && !ep->res_hi && !ep->res_lo && !ep->out_lo && (ep->out_f32 || ep->out_hi);
   DMM_CHECK_ARG(p.ksplit == 1 || (tepi && ep->out_f32 && !ep->out_hi && !ep->residual && !ep->bias && !ep->cmax && ep->act == 0),
                 "dmm_gemm_bf16_tn: split-K writes plain fp32 partial products");
   switch (bn) {

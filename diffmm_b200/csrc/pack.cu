@@ -634,9 +634,9 @@ __global__ void __launch_bounds__(256) csr_qsample_values_kernel(const int64_t* 
 // the kernel instead of being written to and re-read from HBM by a separate generator launch (19445 x 7050 normals are
 // 548 MB each way per modality: ncu showed generator + reader at 37 % of a conf/baby.toml rebuild step).  Counter-based
 // Philox4x32-10 keyed by a 64-bit seed taken from torch's device generator, counter = (row, column / 4): element c of row r
-// is a pure function of (seed, r, c), so the row norm pass and the per-entry lookups see the same normals without
-// storing them; Box-Muller on the four 32-bit outputs.  The draw is i.i.d. N(0, 1) like the reference's; the stream is
-// not torch's (no two GPU runs of the reference share a stream with each other either: its loader shuffles the users).
+// is a pure function of (seed, r, c), so any entry can be drawn on its own without storing the row; Box-Muller on the
+// four 32-bit outputs.  The draw is i.i.d. N(0, 1) like the reference's; the stream is not torch's (no two GPU runs of
+// the reference share a stream with each other either: its loader shuffles the users).
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 #pragma unroll
   for (int i = 0; i < 10; ++i) {
@@ -659,54 +659,11 @@ __device__ __forceinline__ float4 normal4(uint4 u) {
   return make_float4(r0 * c0, r0 * s0, r1 * c1, r1 * s1);
 }
 
-__global__ void __launch_bounds__(256) csr_qsample_values_rng_kernel(const int64_t* __restrict__ indptr,
-                                                                     const int32_t* __restrict__ indices,
-                                                                     const int64_t* __restrict__ row_ids, int64_t row0,
-                                                                     int64_t n_cols, const int64_t* __restrict__ seed,
-                                                                     float coef_a, float coef_b, float* __restrict__ vals) {
-  __shared__ float red[8];
-  const int64_t r = blockIdx.x;
-  const int tid = threadIdx.x;
-  const int64_t u = row_ids ? row_ids[r] : row0 + r;
-  const int64_t b = indptr[u], e = indptr[u + 1];
-  if (b >= e) return;                                   // block-uniform: nothing to emit for an empty row
-  const uint64_t sd = (uint64_t)seed[0];
-  const uint2 key = make_uint2((uint32_t)sd, (uint32_t)(sd >> 32));
-  const uint32_t row_lo = (uint32_t)u, row_hi = (uint32_t)((uint64_t)u >> 32);
-  const int64_t n4 = (n_cols + 3) >> 2;
-  float ss = 0.f;
-  for (int64_t q = tid; q < n4; q += 256) {
-    const float4 n = normal4(philox4x32_10(make_uint4((uint32_t)q, row_lo, row_hi, 0u), key));
-    const int64_t c = q << 2;
-    ss = fmaf(n.x, n.x, ss);
-    if (c + 1 < n_cols) ss = fmaf(n.y, n.y, ss);
-    if (c + 2 < n_cols) ss = fmaf(n.z, n.z, ss);
-    if (c + 3 < n_cols) ss = fmaf(n.w, n.w, ss);
-  }
-  ss = dmm_warp_sum(ss);
-  if ((tid & 31) == 0) red[tid >> 5] = ss;
-  __syncthreads();
-  float tot = 0.f;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) tot += red[i];
-  const float inv = 1.f / fmaxf(sqrtf(tot), 1e-12f);
-  for (int64_t k = b + tid; k < e; k += 256) {
-    const int32_t c = indices[k];
-    float nv = 0.f;
-    if (c >= 0 && c < n_cols) {
-      const float4 n = normal4(philox4x32_10(make_uint4((uint32_t)(c >> 2), row_lo, row_hi, 0u), key));
-      const int w = c & 3;
-      nv = w == 0 ? n.x : (w == 1 ? n.y : (w == 2 ? n.z : n.w));
-    }
-    vals[k] = __fadd_rn(coef_a, __fmul_rn(coef_b, __fmul_rn(nv, inv)));
-  }
-}
-
 // ------------------------------------------------------------------ q_sample on binary CSR rows, sufficient statistics only
 // The entry values need only two things from the N(0, 1) row n: its entries on the row's support S (k = |S| normals) and
 // its squared norm  ||n||^2 = sum_{c in S} n_c^2 + R,  R = sum_{c not in S} n_c^2 ~ chi^2(I - k), independent of n_S.
 // So instead of I normals per row (137 M per modality at baby, ~0.18 ms of Philox + Box-Muller) the kernel draws the k
-// support normals (the SAME Philox elements (seed, row, c) the full-row kernel would use) and ONE chi-square variate:
+// support normals (the Philox elements (seed, row, c): the same normals a full row would have) and ONE chi-square variate:
 // exactly the reference's joint distribution of the outputs (Model.py:337-341), O(k) work per row.
 // chi^2(nu) = 2 Gamma(nu / 2) by Marsaglia-Tsang (exact rejection sampler, acceptance > 99.9 % at nu ~ 7000); nu <= 64:
 // the sum of nu explicit normals.  One warp per row.
@@ -1055,16 +1012,12 @@ extern "C" int dmm_csr_qsample_values(dmm_ctx* ctx, const int64_t* indptr, const
 
 extern "C" int dmm_csr_qsample_values_rng(dmm_ctx* ctx, const int64_t* indptr, const int32_t* indices, const int64_t* row_ids,
                                           int64_t row0, int64_t n_rows, int64_t n_cols, const int64_t* seed, float coef_a,
-                                          float coef_b, float* vals, int full_rows, void* stream) {
+                                          float coef_b, float* vals, void* stream) {
   DMM_CHECK_ARG(ctx && indptr && indices && seed && vals, "dmm_csr_qsample_values_rng: null argument");
   DMM_CHECK_ARG(n_rows >= 0 && n_rows < (1LL << 31) && n_cols > 0 && n_cols < (1LL << 31), "dmm_csr_qsample_values_rng: bad shape");
   if (n_rows == 0) return DMM_OK;
-  if (full_rows)
-    csr_qsample_values_rng_kernel<<<(unsigned)n_rows, 256, 0, (cudaStream_t)stream>>>(indptr, indices, row_ids, row0, n_cols, seed,
-                                                                                     coef_a, coef_b, vals);
-  else
-    csr_qsample_values_chi2_kernel<<<(unsigned)dmm_ceil_div(n_rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(
-        indptr, indices, row_ids, row0, n_rows, n_cols, seed, coef_a, coef_b, vals);
+  csr_qsample_values_chi2_kernel<<<(unsigned)dmm_ceil_div(n_rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+      indptr, indices, row_ids, row0, n_rows, n_cols, seed, coef_a, coef_b, vals);
   DMM_LAUNCH_CHECK();
   return DMM_OK;
 }

@@ -942,12 +942,11 @@ static int topk_dispatch(dmm_ctx* ctx, const float* scores, int64_t ld, int64_t 
                          int64_t n_edges, cudaStream_t st) {
   constexpr int PER_THREAD = 4 * TOPK_V4;
   static const bool force_generic = getenv("DMM_TOPK_GENERIC") != nullptr;   // test hook: exercise the generic kernels
-  static const bool seg_ok = []() { const char* e = getenv("DMM_TOPK_SEG"); return !(e && e[0] == '0'); }();   // A/B switch
 
   // wide rows: segment pass + merge for the rows that qualify, whole-row kernels for the rest (see SegCfg)
   SegCfg sg = make_seg(n_cols);
   const bool rows_aligned = (reinterpret_cast<uintptr_t>(scores) & 15u) == 0 && ld % 4 == 0;
-  const bool segmented = seg_ok && !force_generic && sg.S > 0 && rows_aligned && workspace != nullptr && n_edges >= 0 &&
+  const bool segmented = !force_generic && sg.S > 0 && rows_aligned && workspace != nullptr && n_edges >= 0 &&
                          workspace_bytes >= dmm_topk_workspace_bytes(n_cols, n_edges) && n_rows * (int64_t)sg.S < (1LL << 31);
   if (segmented) {
     sg.mode = 1;
@@ -1017,7 +1016,7 @@ inline size_t prune_head_bytes(int64_t n_rows) { return 256 + prune_align((size_
 
 extern "C" int64_t dmm_topk_pruned_workspace_bytes(int64_t n_rows, int64_t n_cols, int64_t n_edges) {
   // [deferred-row count | deferred-row list | chunk lists of the deferred rows (one slot per emitted entry) | workspace of
-  //  the segmented kernels (only used when pruning is switched off)]
+  //  the segmented kernels (only used by the whole-row fallback for chunk counts outside the pruned kernels' range)]
   return (int64_t)prune_head_bytes(n_rows) + (int64_t)prune_align((size_t)(n_edges > 0 ? n_edges : 1) * sizeof(int32_t)) +
          dmm_topk_workspace_bytes(n_cols, n_edges);
 }
@@ -1041,8 +1040,7 @@ extern "C" int dmm_topk_edges_pruned(dmm_ctx* ctx, const float* scores, int64_t 
   int32_t* const chunk_list = (int32_t*)((uint8_t*)workspace + prune_head_bytes(n_rows));
   uint8_t* const seg_ws = (uint8_t*)workspace + prune_head_bytes(n_rows) + list_bytes;
   const int64_t seg_ws_bytes = workspace_bytes - (int64_t)prune_head_bytes(n_rows) - (int64_t)list_bytes;
-  static const bool prune_ok = []() { const char* e = getenv("DMM_TOPK_PRUNE"); return !(e && e[0] == '0'); }();   // A/B switch
-  if (!prune_ok || n_chunks > 512 * 4 * TOPK_V4 || n_chunks < 8)
+  if (n_chunks > 512 * 4 * TOPK_V4 || n_chunks < 8)
     return topk_dispatch(ctx, scores, ld, n_rows, n_cols, out_ptr, row_base, out_users, out_items, status, order, nullptr,
                          seg_ws, seg_ws_bytes, n_edges, st);
   int32_t* left_count = (int32_t*)workspace;

@@ -61,50 +61,13 @@ class EdgeGatherPlan:
         self.world = world
 
 
-# Backends on which the unequal-segment all_gather is used.  Off by default even for NCCL: torch issues it as one
-# ncclBroadcast per rank inside a group call, and at 8 ranks those eight small broadcasts measured slower (+0.1 ms per
-# modality) than ONE padded ncclAllGather followed by one index_select; DIFFMM_UNEVEN_ALLGATHER=1 switches it on.
-import os as _os
-_UNEVEN_OK = {"nccl": _os.environ.get("DIFFMM_UNEVEN_ALLGATHER", "0") == "1"}
-
-
-def _backend(group=None) -> str:
-    try:
-        return str(td.get_backend(group))
-    except Exception:
-        return ""
-
-
-def allgather_edges(items_local: torch.Tensor, indptr: torch.Tensor, n_users: int, group=None,
-                    plan: Optional[EdgeGatherPlan] = None) -> torch.Tensor:
-    """Every rank filled items[indptr[r0]:indptr[r1]) for its user block; returns the complete edge list on every rank.
-
-    NCCL: ONE all-gather with unequal segment sizes straight into the final buffer, in place (torch issues it as a
-    group of broadcasts inside one NCCL group call) -- no padding, no zero fill, no unpack copies.  Other backends
-    (gloo in the CPU tests): padded equal-size segments and one index_select to unpack."""
-    world, rk = world_size(group), rank(group)
-    if world == 1:
-        return items_local
-    if plan is None or plan.world != world:
-        plan = EdgeGatherPlan(indptr, n_users, world)
-    offs, seg = plan.offs, plan.seg
-    be = _backend(group)
-    if _UNEVEN_OK.get(be, False) and all(e > s for s, e in offs):
-        try:
-            views = [items_local[s:e] for s, e in offs]
-            td.all_gather(views, views[rk], group=group)
-            return items_local
-        except (RuntimeError, ValueError):       # pragma: no cover - backend without unequal all_gather
-            _UNEVEN_OK[be] = False
-    return allgather_edges_multi({"_": items_local}, indptr, n_users, group, plan)["_"]
-
-
 def allgather_edges_multi(items: dict, indptr: torch.Tensor, n_users: int, group=None,
                           plan: Optional[EdgeGatherPlan] = None) -> dict:
-    """The edge lists of ALL modalities in ONE collective: every rank packs its segment of each list into one padded send
-    buffer [M, seg] (padding is never read back), one all_gather_into_tensor, and one index_select per modality compacts
-    the [world, M, seg] result into the CSR-ordered list (the index is precomputed per plan).  3 + M launches per
-    rebuild instead of M x (zero fill + copy + collective + world slice copies)."""
+    """Every rank filled items[m][indptr[r0]:indptr[r1]) of each modality m for its user block; returns the complete
+    edge lists on every rank.  The edge lists of ALL modalities go in ONE collective: every rank packs its segment of
+    each list into one padded send buffer [M, seg] (padding is never read back), one all_gather_into_tensor, and one
+    index_select per modality compacts the [world, M, seg] result into the CSR-ordered list (the index is precomputed
+    per plan).  3 + M launches per rebuild instead of M x (zero fill + copy + collective + world slice copies)."""
     world, rk = world_size(group), rank(group)
     if world == 1:
         return dict(items)

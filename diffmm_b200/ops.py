@@ -6,7 +6,6 @@ calls exactly one C-ABI entry point on the current stream.  No arithmetic happen
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 from typing import Optional
 
@@ -169,9 +168,6 @@ def time_bias(emb_w, emb_b, weight, col0, bias, t0, n_t=1, out=None):
     return out
 
 
-_GATHER_SPLIT = os.environ.get("DIFFMM_GATHER_SPLIT", "1") != "0"
-
-
 def csr_gather_act(indptr, indices, n_rows, n_cols, wt_hi, wt_lo, bias, act, n_out, h_hi, h_lo, *, row_ids=None, row0=0,
                    z_f32=None, order=None, vals=None):
     """h = act(bias + sum of the rows of W^T selected by each binary CSR row) -> bf16 hi (+ lo); z_f32 (optional)
@@ -181,7 +177,7 @@ def csr_gather_act(indptr, indices, n_rows, n_cols, wt_hi, wt_lo, bias, act, n_o
     assert order is None or (order.dtype == torch.int32 and order.numel() == n_rows)
     assert vals is None or (vals.dtype == torch.float32 and vals.numel() == indices.numel())
     counters = getattr(order, "_dmm_counters", None) if order is not None else None
-    if counters is not None and n_out <= 1024 and _GATHER_SPLIT:
+    if counters is not None and n_out <= 1024:
         # rows divided by length inside one launch (order / counters from rows_long_first): bit-identical results
         max_long = indices.numel() // (order._dmm_threshold + 1)
         _lib.call("dmm_csr_gather_act_split", _ctx(indptr), _p(indptr), _p(indices), _p(vals), _p(row_ids), _p(order),
@@ -204,14 +200,13 @@ def csr_qsample_values(indptr, indices, n_rows, n_cols, noise, coef_a, coef_b, v
     return vals
 
 
-def csr_qsample_values_rng(indptr, indices, n_rows, n_cols, seed, coef_a, coef_b, vals, *, row_ids=None, row0=0,
-                           full_rows=False):
-    """csr_qsample_values with the N(0, 1) rows generated inside the kernel (Philox keyed by the device int64 `seed`).
-    full_rows=False draws only the support normals and one chi-square variate for the rest of the squared norm (the
-    same joint distribution of the outputs, O(k) per row)."""
+def csr_qsample_values_rng(indptr, indices, n_rows, n_cols, seed, coef_a, coef_b, vals, *, row_ids=None, row0=0):
+    """csr_qsample_values with the N(0, 1) rows generated inside the kernel (Philox keyed by the device int64 `seed`):
+    it draws only the support normals and one chi-square variate for the rest of the squared norm (the same joint
+    distribution of the outputs as full rows of normals, O(k) per row)."""
     assert seed.dtype == torch.int64 and seed.is_cuda and vals.dtype == torch.float32 and vals.numel() == indices.numel()
     _lib.call("dmm_csr_qsample_values_rng", _ctx(indptr), _p(indptr), _p(indices), _p(row_ids), int(row0), int(n_rows),
-              int(n_cols), _p(seed), float(coef_a), float(coef_b), _p(vals), int(bool(full_rows)), _stream())
+              int(n_cols), _p(seed), float(coef_a), float(coef_b), _p(vals), _stream())
     return vals
 
 

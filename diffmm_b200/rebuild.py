@@ -55,7 +55,6 @@ class ChainWorkspace:
         self.x = torch.empty((rows, self.ld_x), dtype=torch.float32, device=device)
         self.z = None             # fp32 hidden pre-activation state [rows, pad4(hidden)] of the hidden-space chain
         self.bias_eff = None      # [S, hidden] fp32, sized on first use
-        self.partial = None       # fp32 partial sums of a K-chunked GEMM1 (scale-out widths only)
         self._cmax = None         # fp32 [rows, pad4(ceil(I / 32))] chunk maxima of the scores (top-k pruning side array)
 
     def operand(self):
@@ -266,8 +265,8 @@ NOISE_BLOCK_BYTES = 64 << 20     # randn sub-block of the sparse q_sample: writt
 def _qsample_values(diff, csr, row_ids, row0, M, I, sampling_step, noise, dev):
     """Entry values of x_t = q_sample(x0, sampling_step - 1) for the binary CSR rows [row0, row0 + M) (fp32, indexed like
     csr[1]; entries of other rows are left untouched).  Device RNG (default): dmm_csr_qsample_values_rng generates the
-    rows in the kernel.  DIFFMM_CPU_RNG=1 / DIFFMM_QSAMPLE_RNG=torch: the randn draw is torch's (Model.py:337), made in row
-    sub-blocks of NOISE_BLOCK_BYTES that stay L2 resident between the generator's write and the kernel's read."""
+    rows in the kernel.  DIFFMM_CPU_RNG=1: the randn draw is torch's CPU generator (Model.py:337), made in row sub-blocks
+    of NOISE_BLOCK_BYTES that stay L2 resident between the copy and the kernel's read."""
     indptr, indices = csr
     vals = torch.empty(indices.numel(), dtype=torch.float32, device=dev)
     t = sampling_step - 1
@@ -276,26 +275,19 @@ def _qsample_values(diff, csr, row_ids, row0, M, I, sampling_step, noise, dev):
     if noise is not None:
         ops.csr_qsample_values(indptr, indices, M, I, noise, ca, cb, vals, row_ids=row_ids, row0=row0)
         return vals
-    mode = os.environ.get("DIFFMM_QSAMPLE_RNG", "chi2")
-    if mode not in ("chi2", "philox", "torch"):
-        raise ValueError(f"DIFFMM_QSAMPLE_RNG must be chi2, philox or torch, got {mode!r}")
-    if not rng.cpu_rng() and mode != "torch":
+    if not rng.cpu_rng():
         # default: the noise is generated inside the kernel (Philox keyed by one draw of torch's device generator:
-        # reproducible under torch.manual_seed, no host sync) and never written to HBM.  'chi2' draws the support normals
-        # and one chi-square variate for the rest of the row's squared norm (same joint distribution of the outputs, O(k)
-        # per row); 'philox' generates all I normals of every row
+        # reproducible under torch.manual_seed, no host sync) and never written to HBM.  It draws the support normals
+        # and one chi-square variate for the rest of the row's squared norm (same joint distribution of the outputs as
+        # all I normals of every row, O(k) per row)
         seed = torch.randint(0, 2 ** 62, (1,), dtype=torch.int64, device=dev)
-        ops.csr_qsample_values_rng(indptr, indices, M, I, seed, ca, cb, vals, row_ids=row_ids, row0=row0,
-                                   full_rows=mode == "philox")
+        ops.csr_qsample_values_rng(indptr, indices, M, I, seed, ca, cb, vals, row_ids=row_ids, row0=row0)
         return vals
     sub = max(1, min(M, NOISE_BLOCK_BYTES // (4 * I)))
     buf = torch.empty((sub, ops.pad_to(I, 4)), dtype=torch.float32, device=dev)
     for s0 in range(0, M, sub):
         n = min(sub, M - s0)
-        if rng.cpu_rng():
-            buf[:n, :I].copy_(torch.randn((n, I), dtype=torch.float32))
-        else:
-            buf[:n].normal_()             # device generator like randn_like; rows padded to 16 bytes (pad columns unused)
+        buf[:n, :I].copy_(torch.randn((n, I), dtype=torch.float32))
         ops.csr_qsample_values(indptr, indices, n, I, buf[:n, :I], ca, cb, vals,
                                row_ids=row_ids[s0:s0 + n] if row_ids is not None else None, row0=row0 + s0)
     return vals
@@ -373,7 +365,7 @@ def _denoise_chain_full(diff, den, ws, M, *, x_dense, csr, row_ids, row0, sampli
             ops.csr_gather_act(csr[0], csr[1], M, I, w1t_hi, w1t_lo, bias1, 1, H, h_hi, h_lo,
                                row_ids=row_ids, row0=row0, order=order)
         else:
-            _gemm1(ws, a_hi, a_lo, w1_hi, w1_lo, M, H, I, bias1, h_hi, h_lo)
+            ops.gemm_bf16_tn(a_hi, a_lo, w1_hi, w1_lo, M, H, I, bias=bias1, act=1, out_hi=h_hi, out_lo=h_lo)
         if inner_ops:
             h_hi, h_lo, g_hi, g_lo = _inner_layers(inner_ops, M, h_hi, h_lo, g_hi, g_lo)
         c1 = float(np.float32(diff._h_coef1[i]))          # fp64 table -> .float() (Model.py:352)
@@ -394,40 +386,6 @@ def _denoise_chain_full(diff, den, ws, M, *, x_dense, csr, row_ids, row0, sampli
             if first_sparse and c2 != 0.0:
                 ops.csr_axpy_bf16(csr[0], csr[1], M, I, c2, ax_hi, ax_lo, row_ids=row_ids, row0=row0)
     return xv
-
-
-K_CHUNK = 8192          # columns of W1 per launch once W1 outgrows the L2 (128 k-blocks of 64)
-L2_WEIGHT_BYTES = 48 << 20
-
-
-def _gemm1(ws, a_hi, a_lo, w1_hi, w1_lo, M, H, K, bias, h_hi, h_lo):
-    """h = tanh(x_t W1[:, :K]^T + bias).  At scale-out widths (K = 500k items) W1 is ~1 GB and the persistent CTAs
-    walk 7813 k-blocks; with narrow single-CTA tiles they drifted apart until nothing was shared through the L2
-    (measured: 35 GB of DRAM reads for 5 GB of operands, 461 TFLOP/s).  The tile cost model now picks the CTA-pair
-    kernel there (829 TFLOP/s in one launch).  DIFFMM_K_CHUNK=1 instead issues the contraction in K chunks of 8192
-    columns, each launch re-aligning the CTAs, with the partial sums in an fp32 buffer
-    (dmm_gemm_epilogue.res_pre_act) and bias + tanh in the last chunk: measured equal, kept as an option."""
-    if H * K * 2 <= L2_WEIGHT_BYTES or K <= 2 * K_CHUNK or os.environ.get("DIFFMM_K_CHUNK", "0") != "1":
-        ops.gemm_bf16_tn(a_hi, a_lo, w1_hi, w1_lo, M, H, K, bias=bias, act=1, out_hi=h_hi, out_lo=h_lo)
-        return
-    ld = ops.pad_to(H, 4)
-    if ws.partial is None or ws.partial.shape[0] < M or ws.partial.shape[1] != ld:
-        ws.partial = torch.empty((ws.rows, ld), dtype=torch.float32, device=a_hi.device)
-    part = ws.partial[:M, :H]
-    k0 = 0
-    while k0 < K:
-        kc = min(K_CHUNK, K - k0)
-        last = k0 + kc >= K
-        sl = slice(k0, k0 + kc)
-        al = a_lo[:, sl] if a_lo is not None else None
-        wl = w1_lo[:, sl] if w1_lo is not None else None
-        res = part if k0 > 0 else None
-        if last:
-            ops.gemm_bf16_tn(a_hi[:, sl], al, w1_hi[:, sl], wl, M, H, kc, bias=bias, act=1, beta=1.0, residual=res,
-                             res_pre_act=True, out_hi=h_hi, out_lo=h_lo)
-        else:
-            ops.gemm_bf16_tn(a_hi[:, sl], al, w1_hi[:, sl], wl, M, H, kc, beta=1.0, residual=res, out_f32=part)
-        k0 += kc
 
 
 def default_block_rows(n_users: int, n_items: int, hidden, split: bool, budget_bytes: int = 12 << 30) -> int:
@@ -460,16 +418,11 @@ def longest_rows_first(indptr: torch.Tensor, row0: int, n_rows: int) -> torch.Te
 _SIDE_STREAMS: Dict[Tuple[int, int], list] = {}
 
 
-def _side_streams(dev: torch.device, n: int, staggered: bool = False):
-    """n side streams of the device.  staggered: falling priorities (stream 0 highest), so the pipeline on stream 0 gets
-    the SMs first and finishes first while the later ones fill its gaps -- its tail (collective, adjacency build) then
-    overlaps the pipelines still running."""
-    key = (dev.index if dev.index is not None else torch.cuda.current_device(), n, staggered)
+def _side_streams(dev: torch.device, n: int):
+    """n side streams of the device (created once, reused by every rebuild)."""
+    key = (dev.index if dev.index is not None else torch.cuda.current_device(), n)
     if key not in _SIDE_STREAMS:
-        if staggered:
-            _SIDE_STREAMS[key] = [torch.cuda.Stream(device=dev, priority=-(n - 1 - i)) for i in range(n)]
-        else:
-            _SIDE_STREAMS[key] = [torch.cuda.Stream(device=dev) for _ in range(n)]
+        _SIDE_STREAMS[key] = [torch.cuda.Stream(device=dev) for _ in range(n)]
     return _SIDE_STREAMS[key]
 
 
@@ -477,8 +430,8 @@ def rebuild_edges(diff, denoise_models: Dict[str, torch.nn.Module], indptr: torc
                   n_users: int, n_items: int, sampling_step: int = 0, precision: Optional[str] = None,
                   row_range: Optional[Tuple[int, int]] = None, block_rows: Optional[int] = None,
                   out_items: Optional[Dict[str, torch.Tensor]] = None, per_modality=None,
-                  per_modality_out: Optional[dict] = None, status: Optional[torch.Tensor] = None,
-                  staggered: bool = False) -> Dict[str, torch.Tensor]:
+                  per_modality_out: Optional[dict] = None,
+                  status: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
     """Top-k item ids per modality for users in ``row_range`` (default all), written at the train-CSR
     offsets (k_u = deg(u), Main.py:215-216,226).  Returns {modality: int32 [E]} (only this range filled).
 
@@ -494,21 +447,16 @@ def rebuild_edges(diff, denoise_models: Dict[str, torch.nn.Module], indptr: torc
     split = precision == "bf16x3"
     if block_rows is None:
         block_rows = default_block_rows(r1 - r0, n_items, max(max(hidden_widths(d)) for d in denoise_models.values()), split)
-        env = os.environ.get("DIFFMM_BLOCK_ROWS")
-        if env:
-            block_rows = max(128, min(block_rows, int(env)))
     E = int(indices.numel())
     dev = indptr.device
-    prune = os.environ.get("DIFFMM_TOPK_PRUNE", "1") != "0"
     if out_items is None:
         out_items = {m: torch.empty(max(E, 1), dtype=torch.int32, device=dev)[:E] for m in denoise_models}
     mods = list(denoise_models.items())
     orders = {b0: longest_rows_first(indptr, b0, min(b0 + block_rows, r1) - b0) for b0 in range(r0, r1, block_rows)}
     n_streams = min(int(os.environ.get("DIFFMM_STREAMS", "2")), len(mods))
     streams = []
-    staggered = staggered or os.environ.get("DIFFMM_STAGGER_ALL") == "1"      # experiment switch: priorities without a tail
     if n_streams > 1 and dev.type == "cuda" and not torch.cuda.is_current_stream_capturing():
-        streams = _side_streams(dev, n_streams, staggered)
+        streams = _side_streams(dev, n_streams)
         main = torch.cuda.current_stream(dev)
         fork = torch.cuda.Event()
         fork.record(main)
@@ -526,13 +474,10 @@ def rebuild_edges(diff, denoise_models: Dict[str, torch.nn.Module], indptr: torc
                         ws = ChainWorkspace(b1 - b0, n_items, widths, den.time_emb_dim, split, dev)
                     scores = denoise_chain(diff, den, csr=(indptr, indices), row0=b0, n_rows=b1 - b0,
                                            sampling_step=sampling_step, precision=precision, ws=ws, order=orders.get(b0),
-                                           want_cmax=prune)
-                    if prune:      # the contraction left the chunk maxima: the top-k reads only the chunks that matter
-                        ops.topk_edges_pruned(scores, n_items, ws.chunk_max()[:b1 - b0], indptr[b0:], b0, None, out_items[m],
-                                              status=status, order=orders.get(b0))
-                    else:
-                        ops.topk_edges(scores, n_items, indptr[b0:], b0, None, out_items[m], status=status,
-                                       order=orders.get(b0))
+                                           want_cmax=True)
+                    # the contraction left the chunk maxima: the top-k reads only the chunks that matter
+                    ops.topk_edges_pruned(scores, n_items, ws.chunk_max()[:b1 - b0], indptr[b0:], b0, None, out_items[m],
+                                          status=status, order=orders.get(b0))
                 if per_modality is not None:
                     per_modality_out[m] = per_modality(out_items[m])
     for st in streams:
@@ -567,33 +512,13 @@ def rebuild_sharded(diff, denoise_models, indptr, indices, n_users, n_items, sam
                     group=None, plan=None, block_rows=None, status=None, full_items: Optional[dict] = None,
                     local_hook=None):
     """User-sharded rebuild of one rank: chain + top-k on ``row_range``, the edge lists of all ranks, the whole-graph
-    adjacencies.  Default: equal-priority modality pipelines, join, ONE all-gather for all modalities, then the builds on
-    the side streams.  DIFFMM_STAGGER=1 (experiment, measured SLOWER: 1.458 vs 1.412 ms per step at 2 GPUs): the pipelines
-    run on side streams of falling priority and each one continues into its own all-gather and adjacency build, so that
-    the first modality's exchange would overlap the chains still running (collectives in modality order on every rank).
-    local_hook(items_m) (optional) runs inside every modality's pipeline once its local edge list is complete (e.g. a copy
-    of the rank's slice to pinned host memory that overlaps the exchange)."""
-    from . import dist as ddist
-    if os.environ.get("DIFFMM_STAGGER", "0") != "1" or len(denoise_models) < 2:
-        items = rebuild_edges(diff, denoise_models, indptr, indices, n_users, n_items, sampling_step, precision,
-                              row_range=row_range, block_rows=block_rows, status=status, per_modality=local_hook,
-                              per_modality_out={} if local_hook is not None else None)
-        return gather_and_build(items, indptr, n_users, n_items, group, plan, full_items=full_items, status=status)
-    if plan is None or plan.world != ddist.world_size(group):
-        plan = ddist.EdgeGatherPlan(indptr, n_users, ddist.world_size(group))
-
-    def tail(local_items):
-        if local_hook is not None:
-            local_hook(local_items)
-        full = ddist.allgather_edges(local_items, indptr, n_users, group, plan)
-        return ops.build_norm_adj(indptr, full, n_users, n_items, status=status), full
-
-    res: dict = {}
-    rebuild_edges(diff, denoise_models, indptr, indices, n_users, n_items, sampling_step, precision, row_range=row_range,
-                  block_rows=block_rows, status=status, per_modality=tail, per_modality_out=res, staggered=True)
-    if full_items is not None:
-        full_items.update({m: r[1] for m, r in res.items()})
-    return {m: res[m][0] for m in denoise_models}
+    adjacencies: equal-priority modality pipelines, join, ONE all-gather for all modalities, then the builds on the side
+    streams.  local_hook(items_m) (optional) runs inside every modality's pipeline once its local edge list is complete
+    (e.g. a copy of the rank's slice to pinned host memory that overlaps the exchange)."""
+    items = rebuild_edges(diff, denoise_models, indptr, indices, n_users, n_items, sampling_step, precision,
+                          row_range=row_range, block_rows=block_rows, status=status, per_modality=local_hook,
+                          per_modality_out={} if local_hook is not None else None)
+    return gather_and_build(items, indptr, n_users, n_items, group, plan, full_items=full_items, status=status)
 
 
 def gather_and_build(items: Dict[str, torch.Tensor], indptr: torch.Tensor, n_users: int, n_items: int, group=None,

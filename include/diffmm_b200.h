@@ -109,14 +109,13 @@ int dmm_csr_qsample_values(dmm_ctx* ctx, const int64_t* indptr, const int32_t* i
  * DEVICE scalar drawn from the framework's generator; counter = (row id, column / 4); Box-Muller): no randn block is
  * written to or read from HBM.  Element (r, c) is a pure function of (seed, r, c): deterministic per seed, independent of
  * blocking and launch geometry.  i.i.d. N(0, 1) like Model.py:337; not torch's stream.
- * full_rows != 0: all n_cols normals of every row are generated (norm pass + per-entry lookups).
- * full_rows == 0: only the row's support normals (the same elements (seed, r, c)) plus ONE chi-square(n_cols - k) variate
+ * Only the row's support normals (elements (seed, r, c)) are generated, plus ONE chi-square(n_cols - k) variate
  * for the squared norm of the rest (Marsaglia-Tsang): the outputs depend on the row only through n_S and ||n||^2, and
  * (n_S, ||n||^2 - ||n_S||^2) ~ N(0, I_k) x chi^2(n_cols - k) independent, so the joint distribution of the outputs is
  * exactly the reference's at O(k) instead of O(n_cols) work per row.                                           */
 int dmm_csr_qsample_values_rng(dmm_ctx* ctx, const int64_t* indptr, const int32_t* indices, const int64_t* row_ids,
                                int64_t row0, int64_t n_rows, int64_t n_cols, const int64_t* seed, float coef_a,
-                               float coef_b, float* vals, int full_rows, void* stream);
+                               float coef_b, float* vals, void* stream);
 
 /* dmm_csr_gather_act with the rows divided by length inside one launch.  `order` and `n_long` come from
  * dmm_rows_long_first (order: the rows of more than `threshold` entries first; n_long = its counters[0], a DEVICE scalar:

@@ -512,14 +512,13 @@ GA_CASES = ["binary_hi", "weighted_hi", "binary_split", "weighted_split"]
 @pytest.mark.parametrize("kernel", ["per_slice", "row_split"])
 @pytest.mark.parametrize("case", GA_CASES)
 @pytest.mark.parametrize("n_out", GA_N)
-def test_csr_gather_act(ops, monkeypatch, n_out, case, kernel):
+def test_csr_gather_act_kernels(ops, n_out, case, kernel):
     """z = sum over a row's entries of vals * (hi + lo) of W^T, h = act(z + bias) split, on the per-slice kernel (order
     None or a plain permutation) and the row-split kernel (a rows_long_first order, n_out <= 1024): weighted rows,
     split weights, row_ids with a repeated and a permuted user, empty rows (z = 0, h = act(bias)), skipped ids; the table
     rows past n_cols hold huge values, so a gathered out-of-range id would show."""
     if kernel == "row_split" and n_out > 1024:
         pytest.skip("the row-split kernel takes at most 1024 output columns")
-    monkeypatch.setattr(ops, "_GATHER_SPLIT", True)
     ci = GA_CASES.index(case)
     weighted, with_lo = "weighted" in case, "split" in case
     rng = np.random.default_rng(n_out * 10 + ci)

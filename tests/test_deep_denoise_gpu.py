@@ -179,7 +179,9 @@ def test_deep_chain_precision_at_the_baby_shape():
 # ---------------------------------------------------------------------------------------------- 3. rebuild
 @pytest.mark.parametrize("precision", PRECISIONS)
 @pytest.mark.parametrize("denoise_dim", DIMS)
-def test_deep_rebuild_edges_pruned_unpruned_and_chain_topk_agree(denoise_dim, precision, monkeypatch):
+def test_deep_rebuild_edges_and_chain_topk_agree(denoise_dim, precision):
+    """rebuild_edges (pruned top-k on the chunk maxima of the last contraction) against per-block denoise_chain and the
+    whole-row top-k: the same edges, bit for bit."""
     from diffmm_b200 import ops, rebuild
     U, I = 700, 1000
     _, gd, den = _model(denoise_dim, I, precision, seed=1)
@@ -187,21 +189,17 @@ def test_deep_rebuild_edges_pruned_unpruned_and_chain_topk_agree(denoise_dim, pr
     k, ptr, idx, _ = _csr_rows(U, I, 6)
     d_ptr, d_idx = T(ptr), T(idx)
     dens = {"image": den, "text": den2}
-    out = {}
-    for prune in ("1", "0"):
-        monkeypatch.setenv("DIFFMM_TOPK_PRUNE", prune)
-        items = rebuild.rebuild_edges(gd, dens, d_ptr, d_idx, U, I, sampling_step=0, block_rows=256)
-        out[prune] = {m: v.clone() for m, v in items.items()}
+    items = rebuild.rebuild_edges(gd, dens, d_ptr, d_idx, U, I, sampling_step=0, block_rows=256)
+    out = {m: v.clone() for m, v in items.items()}
     for m, d in dens.items():
-        assert torch.equal(out["1"][m], out["0"][m]), m
-        want = torch.empty_like(out["1"][m])
+        want = torch.empty_like(out[m])
         with torch.no_grad():
             for b0 in range(0, U, 256):
                 n = min(256, U - b0)
                 sc = rebuild.denoise_chain(gd, d, csr=(d_ptr, d_idx), row0=b0, n_rows=n, sampling_step=0,
                                            order=rebuild.longest_rows_first(d_ptr, b0, n))
                 ops.topk_edges(sc, I, d_ptr[b0:], b0, None, want)
-        assert torch.equal(out["1"][m], want), m
+        assert torch.equal(out[m], want), m
 
 
 # ---------------------------------------------------------------------------------------------- 4. fused training step

@@ -46,7 +46,7 @@ def _worker(rank, world, port, U, I, ret):
         items = torch.full((int(indptr[-1]),), -1, dtype=torch.int32)
         local = O.topk_edges(scores[r0:r1], deg[r0:r1])      # stand-in for denoise chain + dmm_topk_edges
         items[indptr[r0]:indptr[r1]] = torch.from_numpy(np.concatenate(local).astype(np.int32))
-        full = ddist.allgather_edges(items, torch.from_numpy(indptr), U)
+        full = ddist.allgather_edges_multi({"m": items}, torch.from_numpy(indptr), U)["m"]
         want = np.concatenate(O.topk_edges(scores, deg)).astype(np.int32)
         ok_edges = bool((full.numpy() == want).all())
 
@@ -67,7 +67,7 @@ def _worker(rank, world, port, U, I, ret):
 
 
 @pytest.mark.parametrize("world", [2])
-def test_sharded_rebuild_and_propagation_gloo(world):
+def test_sharded_edge_gather_and_propagation_gloo(world):
     mgr = mp.Manager()
     ret = mgr.dict()
     mp.spawn(_worker, args=(world, _free_port(), 101, 37, ret), nprocs=world, join=True)

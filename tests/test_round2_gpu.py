@@ -450,7 +450,7 @@ def test_spmm_bf16_autograd_path_matches_fp32_within_tolerance(ops, monkeypatch)
     assert torch.equal(ag.spmm(generic, x, "bf16"), ops.spmm(generic, x))
 
 
-def test_fused_rng_qsample_values_are_standard_normal_and_counter_based(ops):
+def test_chi2_rng_qsample_values_are_standard_normal_and_counter_based(ops):
     """dmm_csr_qsample_values_rng: (vals - a) / b = n_c / ||n|| for i.i.d. N(0, 1) rows generated in the kernel.  Checked:
     moments of sqrt(I) (vals - a) / b (mean 0, variance 1, kurtosis 3), row norms through the identity
     sum_c (n_c / ||n||)^2 over a FULL row = 1, determinism per seed, independence of blocking (element (r, c) is a pure
@@ -464,39 +464,31 @@ def test_fused_rng_qsample_values_are_standard_normal_and_counter_based(ops):
     d_ptr, d_idx = T(ptr), T(idx)
     a, b = 0.9, 0.4
     seed = torch.tensor([1234567], dtype=torch.int64, device=DEV)
-    vals = torch.empty(idx.size, dtype=torch.float32, device=DEV)
-    ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed, a, b, vals, full_rows=True)
-    v = vals.cpu().numpy().astype(np.float64)
-    z = (v - a) / b                                      # n_c / ||n||
-    assert abs((z[:I] ** 2).sum() - 1.0) < 1e-4          # row 0 holds every column
+    ref = torch.empty(idx.size, dtype=torch.float32, device=DEV)
+    ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed, a, b, ref)
+    z = (ref.cpu().numpy().astype(np.float64) - a) / b   # n_c / ||n||
+    assert abs((z[:I] ** 2).sum() - 1.0) < 1e-4          # row 0 holds every column: the rest of the norm is empty
     s = z[I:] * np.sqrt(I)
     assert abs(s.mean()) < 0.03 and abs(s.var() - 1.0) < 0.05 and abs((s ** 4).mean() / s.var() ** 2 - 3.0) < 0.25
     # deterministic, and independent of how the rows are blocked / addressed
-    for full in (True, False):
-        ref = torch.empty_like(vals)
-        ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed, a, b, ref, full_rows=full)
-        vals2 = torch.empty_like(vals)
-        ops.csr_qsample_values_rng(d_ptr, d_idx, 300, I, seed, a, b, vals2, full_rows=full)
-        ops.csr_qsample_values_rng(d_ptr, d_idx, U - 300, I, seed, a, b, vals2, row0=300, full_rows=full)
-        assert torch.equal(ref, vals2)
-        vals3 = torch.full_like(vals, float("nan"))
-        ids = torch.arange(U - 1, -1, -1, device=DEV)
-        ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed, a, b, vals3, row_ids=ids, full_rows=full)
-        assert torch.equal(ref, vals3)
-        vals4 = torch.empty_like(vals)
-        ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed + 1, a, b, vals4, full_rows=full)
-        assert float((vals4 - ref).abs().max()) > 1e-3
-        zz = (ref.cpu().numpy().astype(np.float64) - a) / b
-        assert abs((zz[:I] ** 2).sum() - 1.0) < 1e-4      # full row: the rest of the norm is empty (chi-square with 0 dof)
-        ss = zz[I:] * np.sqrt(I)
-        assert abs(ss.mean()) < 0.03 and abs(ss.var() - 1.0) < 0.05
+    vals2 = torch.empty_like(ref)
+    ops.csr_qsample_values_rng(d_ptr, d_idx, 300, I, seed, a, b, vals2)
+    ops.csr_qsample_values_rng(d_ptr, d_idx, U - 300, I, seed, a, b, vals2, row0=300)
+    assert torch.equal(ref, vals2)
+    vals3 = torch.full_like(ref, float("nan"))
+    ids = torch.arange(U - 1, -1, -1, device=DEV)
+    ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed, a, b, vals3, row_ids=ids)
+    assert torch.equal(ref, vals3)
+    vals4 = torch.empty_like(ref)
+    ops.csr_qsample_values_rng(d_ptr, d_idx, U, I, seed + 1, a, b, vals4)
+    assert float((vals4 - ref).abs().max()) > 1e-3
 
 
 @pytest.mark.parametrize("n_cols", [40, 70, 7050])
-def test_qsample_values_follow_the_exact_beta_law(ops, n_cols):
+def test_chi2_qsample_values_follow_the_exact_beta_law(ops, n_cols):
     """One interaction per user: z^2 = n_c^2 / ||n||^2 ~ Beta(1/2, (I - 1)/2) exactly.  Checks mean and variance over
-    40 000 rows for both generators: all I normals per row, and support normals + one chi-square(I - 1) variate
-    (explicit normals for I - 1 <= 64, Marsaglia-Tsang above)."""
+    40 000 rows for the generator of support normals + one chi-square(I - 1) variate (explicit normals for I - 1 <= 64,
+    Marsaglia-Tsang above)."""
     U = 40000
     rng = np.random.default_rng(n_cols)
     ptr = np.arange(U + 1, dtype=np.int64)
@@ -505,16 +497,15 @@ def test_qsample_values_follow_the_exact_beta_law(ops, n_cols):
     al, be = 0.5, 0.5 * (n_cols - 1)
     mean = al / (al + be)
     var = al * be / ((al + be) ** 2 * (al + be + 1))
-    for full in (True, False):
-        vals = torch.empty(U, dtype=torch.float32, device=DEV)
-        ops.csr_qsample_values_rng(T(ptr), T(idx), U, n_cols, seed, 0.0, 1.0, vals, full_rows=full)
-        z2 = vals.cpu().numpy().astype(np.float64) ** 2
-        assert abs(z2.mean() - mean) < 5.0 * np.sqrt(var / U), (full, z2.mean(), mean)
-        assert abs(z2.var() - var) < 0.08 * var, (full, z2.var(), var)
+    vals = torch.empty(U, dtype=torch.float32, device=DEV)
+    ops.csr_qsample_values_rng(T(ptr), T(idx), U, n_cols, seed, 0.0, 1.0, vals)
+    z2 = vals.cpu().numpy().astype(np.float64) ** 2
+    assert abs(z2.mean() - mean) < 5.0 * np.sqrt(var / U), (z2.mean(), mean)
+    assert abs(z2.var() - var) < 0.08 * var, (z2.var(), var)
 
 
 @pytest.mark.parametrize("n_cols", [50, 7050])
-def test_qsample_values_short_row_path_equals_general_path(ops, n_cols):
+def test_chi2_qsample_short_row_path_equals_general_path(ops, n_cols):
     """Rows of fewer than 32 entries take the one-round path of the sufficient-statistics generator (one entry per lane, the
     chi-square draw in lockstep on the free lane).  The values are a pure function of (seed, row, column, support size):
     the same rows padded to >= 32 entries with out-of-range columns (ignored by contract) go through the general path and
@@ -534,8 +525,8 @@ def test_qsample_values_short_row_path_equals_general_path(ops, n_cols):
     seed = torch.tensor([1234567], dtype=torch.int64, device=DEV)
     va = torch.zeros(len(idx_a), dtype=torch.float32, device=DEV)
     vb = torch.zeros(len(idx_b), dtype=torch.float32, device=DEV)
-    ops.csr_qsample_values_rng(T(ptr_a), T(idx_a), U, n_cols, seed, 0.25, 0.75, va, full_rows=False)
-    ops.csr_qsample_values_rng(T(ptr_b), T(idx_b), U, n_cols, seed, 0.25, 0.75, vb, full_rows=False)
+    ops.csr_qsample_values_rng(T(ptr_a), T(idx_a), U, n_cols, seed, 0.25, 0.75, va)
+    ops.csr_qsample_values_rng(T(ptr_b), T(idx_b), U, n_cols, seed, 0.25, 0.75, vb)
     keep = torch.from_numpy(idx_b < n_cols).to(DEV)
     assert torch.equal(va, vb[keep])
     assert float((va - 0.25).abs().max()) > 0.0

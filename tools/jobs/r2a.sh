@@ -8,7 +8,6 @@ echo "pytest rc=$?" >> gpurun_out/r2a_pytest.log
 timeout 600 python bench.py --steps 10 --warmup 3 > gpurun_out/r2a_bench_baby.json 2> gpurun_out/r2a_bench_baby.err
 echo "bench rc=$?"
 timeout 300 python bench.py --steps 10 --warmup 3 --sampling-step 0 --no-epoch --no-cpu-baseline --no-aux > gpurun_out/r2a_bench_baby_ss0.json 2> gpurun_out/r2a_bench_baby_ss0.err
-DIFFMM_TOPK_PRUNE=0 timeout 300 python bench.py --steps 10 --warmup 3 --sampling-step 0 --no-epoch --no-cpu-baseline --no-aux > gpurun_out/r2a_bench_baby_ss0_noprune.json 2> gpurun_out/r2a_bench_baby_ss0_noprune.err
 timeout 300 python bench.py --steps 10 --warmup 3 --workload sports --no-epoch --no-cpu-baseline --no-aux > gpurun_out/r2a_bench_sports.json 2> gpurun_out/r2a_bench_sports.err
 timeout 400 python bench.py --steps 4 --warmup 3 --workload scaleout --no-epoch --no-cpu-baseline --no-aux > gpurun_out/r2a_bench_scaleout.json 2> gpurun_out/r2a_bench_scaleout.err
 tail -5 gpurun_out/r2a_pytest.log

@@ -12,5 +12,5 @@ print('variants', json.dumps(d.get('variants'))[:600])
 print('roofline', round(d['roofline']['frac'],3), {k:(round(v['avg_ms'],4),round(v['tflops'])) for k,v in d['roofline']['by_shape_MxNxK'].items()})
 print('breakdown',{k:v['ms_per_step'] for k,v in d['breakdown_ms_per_step'].items()})
 P
-DMM_SPMM_V2=0 python tools/bench_spmm.py baby | tail -2; python tools/bench_spmm.py baby | tail -2
-DMM_SPMM_V2=0 python tools/bench_spmm.py sports | tail -2; python tools/bench_spmm.py sports | tail -2
+python tools/bench_spmm.py baby | tail -2
+python tools/bench_spmm.py sports | tail -2

@@ -13,4 +13,3 @@ print('aux', {k:(round(v.get('frac',0),3), round(v.get('avg_launch_ms',0),4)) fo
 print('roofline', round(d['roofline']['frac'],3), {k:(round(v['avg_ms'],4),round(v['tflops'])) for k,v in d['roofline']['by_shape_MxNxK'].items()})
 print('breakdown',{k:v['ms_per_step'] for k,v in d['breakdown_ms_per_step'].items()})
 P
-DIFFMM_QSAMPLE_RNG=philox timeout 200 python bench.py --steps 10 --warmup 3 --quick | python -c "import json,sys; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print('philox full rows: ms', d['ms_per_step'])"
