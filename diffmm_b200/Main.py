@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import argparse
 import ast
+import numbers
 import os
 import random
 import time
@@ -733,6 +734,71 @@ class Coach:
         with torch.no_grad():
             u = user_embs[recommend.to_device(rid.astype(np.int64), self.device)]
             return recommend.rank_candidates(u, item_embs, candidates, n, precision="bf16x3")
+
+    _VIEWS = ("final", "image", "text", "audio")
+
+    def _check_view(self, view):
+        if view not in self._VIEWS:
+            raise ValueError(f"view must be one of {self._VIEWS}, got {view!r}")
+        if view == "audio" and not self.has_audio:
+            raise ValueError("view 'audio' needs a dataset with audio features")
+
+    def _view_embs(self, view, final_items=None):
+        """Item vectors of one view: "final" = gcn_MM's final item embeddings (final_items when the caller already has
+        them: the propagation is not run twice); "image" / "text" / "audio" = the trained modality projections
+        (getImageFeats / getTextFeats / getAudioFeats) that gcn_MM normalises and propagates."""
+        self._check_view(view)
+        if view == "final":
+            return self._final_embs()[1] if final_items is None else final_items
+        with torch.no_grad():
+            return {"image": self.model.getImageFeats, "text": self.model.getTextFeats,
+                    "audio": self.model.getAudioFeats}[view]().detach()
+
+    def _item_view(self, view, final_items=None):
+        """Unit item vectors of one view (F.normalize semantics, ops.rownorm_fwd): their dot products are cosines."""
+        x = self._view_embs(view, final_items)
+        with torch.no_grad(), torch.cuda.device(x.device):
+            return ops.rownorm_fwd(x)[0]
+
+    def similar_items(self, items, n, view="final"):
+        """The n items most similar to each of ``items`` (host ints or a CUDA tensor) by cosine in one view's space
+        (final embeddings, or one modality's projection): (items int64, cosines fp32) [len(items), n] on the device,
+        cosine descending then item id ascending, never the query itself (recommend.similar_items, bf16x3).  Draws no
+        random numbers and changes no parameter."""
+        return recommend.similar_items(self._view_embs(view), items, n, precision="bf16x3")
+
+    def recommend_diverse(self, users, n, lam=0.5, view="final", pool=None):
+        """MMR-diversified lists: the ``pool`` best items of each user (``recommend``'s bf16x3 scores, train items
+        excluded) re-ranked greedily by lam * score - (1 - lam) * (largest cosine, in ``view``'s space, to the items
+        already picked) (recommend.mmr_rerank).  Returns (items int64, scores fp32) [len(users), n] on the device, each
+        item with its score; lam = 1 gives exactly ``recommend(users, n)``.  pool defaults to min(4 n, I, 32768 // D,
+        1024) (D = the view's width) and must satisfy n <= pool <= min(I, 32768 // D, 1024).  Draws no random numbers and
+        changes no parameter."""
+        U, I = self.config.data.user_num, self.config.data.item_num
+        lam = recommend.check_lam(lam)
+        rid = np.asarray(users.numpy() if isinstance(users, Tensor) else users)
+        if rid.ndim != 1 or (rid.size and (rid.dtype.kind not in "iu" or rid.min() < 0 or rid.max() >= U)):
+            raise ValueError(f"users must be a 1-D sequence of user ids in 0..{U - 1}")
+        self._check_view(view)
+        D = self.config.base.latdim                   # the width of every view
+        cap = min(I, recommend.MMR_MAX_FLOATS // D, recommend.MMR_MAX_C)
+        if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= n <= cap:
+            raise ValueError(f"n must be an int in 1..{cap}, got {n!r}")
+        n = int(n)
+        if pool is None:
+            pool = min(4 * n, cap)
+        if isinstance(pool, bool) or not isinstance(pool, numbers.Integral) or not n <= pool <= cap:
+            raise ValueError(f"pool must be an int in {n}..{cap}, got {pool!r}")
+        rid = rid.astype(np.int64)
+        h = self.handler
+        user_embs, item_embs = self._final_embs()
+        unit = self._item_view(view, item_embs)
+        with torch.no_grad(), torch.cuda.device(self.device):
+            rid_dev = recommend.to_device(rid, self.device)
+            cand, rel = recommend._topn(user_embs[rid_dev], item_embs, int(pool),
+                                        (h.train_indptr, h.train_indices, rid_dev), float("-inf"), "bf16x3")
+            items, scores = recommend._mmr_rerank(unit, cand, rel, n, lam)
+            return items.long(), scores
 
     def evaluate_sampled(self, n_neg=100, cutoffs=(1, 5, 10), seed=0):
         """HR@K and NDCG@K of the sampled-negative protocol over testEpoch's test users: every (user, held-out item)

@@ -126,6 +126,8 @@ PROTOTYPES = {
     "dmm_score_pairs": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64, C.c_int, c_vp, c_vp]),
     "dmm_rank_candidates": (C.c_int, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, C.c_int,
                                       c_vp, c_i64, c_vp, c_i64, c_vp]),
+    "dmm_mmr_rerank": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_f32,
+                                 c_vp, c_i64, c_vp, c_i64, c_vp]),
     "dmm_bpr_infonce_workspace_floats":(c_i64, [c_i64, C.c_int, C.c_int]),
     "dmm_bpr_infonce_fwd": (C.c_int, [c_vp, C.POINTER(NceProblem), C.c_int, C.POINTER(BprProblem), c_i64, c_vp, c_vp, c_vp, c_vp,
                                       c_vp]),

@@ -21,6 +21,10 @@
 // Both compute the score with pair_score: the same split-bf16 terms as the tensor-pipe contraction (bf16x3 or bf16),
 // added by fp32 FMAs in a fixed lane layout.  A pair gets the same bits from either kernel, but not dmm_topn_rank's
 // (contraction) bits: the summation order differs.
+//
+// Diversified lists from given candidates:
+//   dmm_mmr_rerank              row r's candidates deduplicated, their vectors staged in shared memory once, and N greedy
+//                               MMR steps (relevance against the largest similarity to the items already picked)
 #include "common.cuh"
 
 namespace {
@@ -302,6 +306,142 @@ __global__ void __launch_bounds__(rank_cand_threads(P)) rank_candidates_kernel(
   }
 }
 
+// ---- MMR re-ranking of caller-supplied candidates ---------------------------------------------------------------------
+constexpr int MMR_MAX_FLOATS = 32768;   // C * D: the row's vectors as fp32 in 128 KB of shared memory (before padding)
+
+// One thread per candidate up to 512: at C = 512, D = 64 one CTA fills an SM's shared memory, and 16 warps instead of 8
+// took a step from 15.6 to 13.3 ms at baby (DESIGN §7).
+__host__ __device__ constexpr int mmr_threads(int P) { return P < 32 ? 32 : (P > 512 ? 512 : P); }
+
+// Floats per staged row: D rounded up to whole quads, plus one quad when the quad count is even, so the row stride in
+// 16-byte units is odd and the eight lanes of each phase of a float4 load (eight different rows) hit eight bank groups.
+__host__ __device__ constexpr int mmr_row_floats(int D) { return ((D + 3) / 4) % 2 ? (D + 3) / 4 * 4 : (D + 3) / 4 * 4 + 4; }
+
+// Largest dynamic shared memory of any allowed (C, D): C * mmr_row_floats(D) <= C * D + 7 C <= 32768 + 7 * 1024 floats.
+constexpr int MMR_SMEM_MAX = (MMR_MAX_FLOATS + 7 * 1024) * 4;
+
+// sim of the staged rows a, b (Q quads each, zero past D): four partial sums s_q over d = q mod 4 from +0.0, each term
+// fl(a_d * b_d) added in ascending d, then (s0 + s1) + (s2 + s3).  The zero padding adds +0 products to sums that are
+// never -0.0, so it leaves every bit unchanged.
+__device__ __forceinline__ float mmr_sim(const float* __restrict__ a, const float* __restrict__ b, int Q) {
+  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+  for (int q = 0; q < Q; ++q) {
+    const float4 x = reinterpret_cast<const float4*>(a)[q];
+    const float4 y = reinterpret_cast<const float4*>(b)[q];
+    s0 = __fadd_rn(s0, __fmul_rn(x.x, y.x));
+    s1 = __fadd_rn(s1, __fmul_rn(x.y, y.y));
+    s2 = __fadd_rn(s2, __fmul_rn(x.z, y.z));
+    s3 = __fadd_rn(s3, __fmul_rn(x.w, y.w));
+  }
+  return __fadd_rn(__fadd_rn(s0, s1), __fadd_rn(s2, s3));
+}
+
+// One CTA per row, P = the power of two >= C, NT = mmr_threads(P) threads, E = P / NT candidates per thread.
+//  1. Dedup: the words (item << 32 | slot) of the valid slots are sorted; the first word of each item run is that item's
+//     first occurrence, and its position i in the sorted order is ascending in the item id.
+//  2. Order: the first occurrences are re-sorted as (~order_key(rel) << 32 | i << 10 | slot), the library's rank order
+//     (relevance descending, then item ascending), so candidate index j (< nv, the distinct valid count) is that rank.
+//  3. Stage: the nv rows of vec go to shared memory in that order (mmr_row_floats(D) floats each, zero-padded).
+//  4. Greedy: thread t owns the candidates j = t + e NT; it keeps lam rel_j, m_j and the picked flag in registers.  Each
+//     step takes the block maximum of (order_key(obj_j) << 32 | ~j) over the unpicked candidates, i.e. obj descending,
+//     then j ascending (relevance descending, item ascending), and then raises m_j to sim(j, pick).
+template <int P>
+__global__ void __launch_bounds__(mmr_threads(P)) mmr_rerank_kernel(
+    const float* __restrict__ vec, int64_t ld_v, int64_t n_items, int D, const int32_t* __restrict__ cand, int64_t ld_c,
+    const float* __restrict__ rel, int64_t ld_r, int C, int N, float lam, int32_t* __restrict__ out_items,
+    int64_t ld_oi, float* __restrict__ out_rel, int64_t ld_or) {
+  constexpr int NT = mmr_threads(P);
+  constexpr int E = P / NT;
+  constexpr int NW = NT / 32;
+  extern __shared__ float4 s_vec4[];
+  float* s_vec = reinterpret_cast<float*>(s_vec4);
+  __shared__ uint64_t w[P];
+  __shared__ uint64_t s_red[2][NW];
+  const int64_t r = blockIdx.x;
+  const int t = threadIdx.x;
+  const int32_t* crow = cand + r * ld_c;
+  const float* rrow = rel + r * ld_r;
+
+  for (int i = t; i < P; i += NT) {
+    const int32_t it = i < C ? crow[i] : -1;
+    w[i] = (it >= 0 && it < n_items) ? ((uint64_t)(uint32_t)it << 32 | (uint32_t)i) : ~0ull;
+  }
+  bitonic_sort_smem<P, NT>(w);
+  uint64_t nw[E];
+  int nv = 0;
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int i = t + e * NT;
+    const uint64_t x = w[i];
+    const bool f = x != ~0ull && (i == 0 || (w[i - 1] >> 32) != (x >> 32));
+    const uint32_t slot = (uint32_t)x;
+    nw[e] = f ? ((uint64_t)~order_key(__ldg(rrow + slot)) << 32 | (uint32_t)i << 10 | slot) : ~0ull;
+    nv += __syncthreads_count(f);   // also orders every read of w before the writes below
+  }
+#pragma unroll
+  for (int e = 0; e < E; ++e) w[t + e * NT] = nw[e];
+  bitonic_sort_smem<P, NT>(w);
+
+  // stage the nv rows, one warp per row, zero past D up to the whole quads
+  const int Q = (D + 3) / 4;
+  const int ldS = mmr_row_floats(D);
+  for (int k = t >> 5; k < nv; k += NW) {
+    const int32_t it = __ldg(crow + (uint32_t)w[k] % 1024u);
+    const float* src = vec + (int64_t)it * ld_v;
+    for (int d = t & 31; d < 4 * Q; d += 32) s_vec[k * ldS + d] = d < D ? __ldg(src + d) : 0.f;
+  }
+  float lr[E], m[E];
+  int jj[E];   // candidate index, or -1 once picked / when absent
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int j = t + e * NT;
+    jj[e] = j < nv ? j : -1;
+    lr[e] = j < nv ? __fmul_rn(lam, __ldg(rrow + (uint32_t)w[j] % 1024u)) : 0.f;
+    m[e] = __uint_as_float(0xFF800000u);
+  }
+  const float mu = __fsub_rn(1.f, lam);
+  const int steps = N < nv ? N : nv;
+  __syncthreads();   // the staged rows are visible
+  for (int s = 0; s < steps; ++s) {
+    uint64_t best = 0;
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+      if (jj[e] < 0) continue;
+      const float obj = s == 0 ? lr[e] : __fsub_rn(lr[e], __fmul_rn(mu, m[e]));
+      const uint64_t key = (uint64_t)order_key(obj) << 32 | (uint32_t)~jj[e];
+      best = key > best ? key : best;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const uint64_t y = __shfl_xor_sync(0xffffffffu, best, o);
+      best = y > best ? y : best;
+    }
+    if ((t & 31) == 0) s_red[s & 1][t >> 5] = best;
+    __syncthreads();   // s_red[s & 1] is rewritten two steps later, after the next step's barrier
+    best = s_red[s & 1][0];
+#pragma unroll
+    for (int q = 1; q < NW; ++q) best = s_red[s & 1][q] > best ? s_red[s & 1][q] : best;
+    const int p = (int)~(uint32_t)best;
+    if (t == 0) {
+      const uint32_t slot = (uint32_t)w[p] % 1024u;
+      out_items[r * ld_oi + s] = __ldg(crow + slot);
+      out_rel[r * ld_or + s] = __ldg(rrow + slot);
+    }
+    if (s + 1 == steps) break;
+    const float* sp = s_vec + p * ldS;
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+      if (jj[e] == p) jj[e] = -1;
+      if (jj[e] < 0) continue;
+      m[e] = fmaxf(m[e], mmr_sim(s_vec + jj[e] * ldS, sp, Q));
+    }
+  }
+  for (int i = steps + t; i < N; i += NT) {
+    out_items[r * ld_oi + i] = -1;
+    out_rel[r * ld_or + i] = __uint_as_float(0xFF800000u);
+  }
+}
+
 constexpr int CUT_NT = 128;
 constexpr int CUT_MAX = 1024;
 constexpr int CUT_PER = CUT_MAX / CUT_NT;   // cutoffs per thread
@@ -552,6 +692,52 @@ extern "C" int dmm_rank_candidates(dmm_ctx* ctx, const float* user, int64_t ld_u
 #undef DMM_RANKC
   DMM_LAUNCH_CHECK();
   return DMM_OK;
+}
+
+template <int P>
+static int launch_mmr_rerank(const dmm_ctx* ctx, unsigned grid, size_t smem, cudaStream_t st, const float* vec,
+                             int64_t ld_v, int64_t n_items, int D, const int32_t* cand, int64_t ld_c, const float* rel,
+                             int64_t ld_r, int C, int N, float lam, int32_t* out_items, int64_t ld_oi, float* out_rel,
+                             int64_t ld_or) {
+  static DmmPerDeviceOnce smem_once;
+  if (smem_once.need(ctx)) {
+    DMM_CUDA(cudaFuncSetAttribute(mmr_rerank_kernel<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, MMR_SMEM_MAX));
+    smem_once.mark(ctx);
+  }
+  mmr_rerank_kernel<P><<<grid, mmr_threads(P), smem, st>>>(vec, ld_v, n_items, D, cand, ld_c, rel, ld_r, C, N, lam,
+                                                           out_items, ld_oi, out_rel, ld_or);
+  DMM_LAUNCH_CHECK();
+  return DMM_OK;
+}
+
+extern "C" int dmm_mmr_rerank(dmm_ctx* ctx, const float* vec, int64_t ld_v, int64_t n_items, int64_t D, const int32_t* cand,
+                              int64_t ld_c, const float* rel, int64_t ld_r, int64_t n_rows, int64_t C, int64_t N, float lam,
+                              int32_t* out_items, int64_t ld_oi, float* out_rel, int64_t ld_or, void* stream) {
+  DMM_CHECK_ARG(ctx, "dmm_mmr_rerank: null argument");
+  DMM_CHECK_ARG(C >= 1 && C <= 1024, "dmm_mmr_rerank: C must be 1..1024 (got %lld)", (long long)C);
+  DMM_CHECK_ARG(D >= 1 && D <= 256, "dmm_mmr_rerank: D must be 1..256 (got %lld)", (long long)D);
+  DMM_CHECK_ARG(C * D <= MMR_MAX_FLOATS, "dmm_mmr_rerank: C * D must be <= %d (got %lld * %lld)", MMR_MAX_FLOATS,
+                (long long)C, (long long)D);
+  DMM_CHECK_ARG(N >= 1 && N <= C, "dmm_mmr_rerank: N must be 1..C (got %lld, C = %lld)", (long long)N, (long long)C);
+  DMM_CHECK_ARG(lam >= 0.f && lam <= 1.f, "dmm_mmr_rerank: lam must be in [0, 1]");
+  DMM_CHECK_ARG(n_rows >= 0 && n_rows < (1LL << 31) && n_items >= 0 && n_items < (1LL << 31) && ld_v >= D &&
+                    ld_c >= C && ld_r >= C && ld_oi >= N && ld_or >= N,
+                "dmm_mmr_rerank: bad shape");
+  if (n_rows == 0) return DMM_OK;
+  DMM_CHECK_ARG(cand && rel && out_items && out_rel && (vec || n_items == 0), "dmm_mmr_rerank: null argument");
+  const size_t smem = (size_t)C * mmr_row_floats((int)D) * sizeof(float);
+  const unsigned g = (unsigned)n_rows;
+  const int c = (int)C;
+#define DMM_MMR(P)                                                                                                  \
+  launch_mmr_rerank<P>(ctx, g, smem, (cudaStream_t)stream, vec, ld_v, n_items, (int)D, cand, ld_c, rel, ld_r, c, \
+                       (int)N, lam, out_items, ld_oi, out_rel, ld_or)
+  if (c <= 32) return DMM_MMR(32);
+  if (c <= 64) return DMM_MMR(64);
+  if (c <= 128) return DMM_MMR(128);
+  if (c <= 256) return DMM_MMR(256);
+  if (c <= 512) return DMM_MMR(512);
+  return DMM_MMR(1024);
+#undef DMM_MMR
 }
 
 extern "C" int dmm_eval_metrics_cutoffs(dmm_ctx* ctx, const int32_t* ranked, int64_t ld_ranked, int64_t n_rows, int64_t N,

@@ -678,6 +678,39 @@ def rank_candidates(user, item, cand, N, x3, items, out_scores):
               _p(items), _row_major(items, "items"), _p(out_scores), _row_major(out_scores, "out_scores"), _stream())
 
 
+def mmr_rerank(vec, cand, rel, N, lam, items, out_rel):
+    """Row r's candidates cand[r] (int32 [rows, C], -1 = empty) with relevance rel[r] (fp32 [rows, C]) re-ranked by MMR
+    over the fp32 rows of vec [n_items, D] (dmm_mmr_rerank): the first N picks into items int32 [rows, >= N] and their
+    relevance into out_rel fp32 [rows, >= N], (-1, -inf) past the distinct valid candidates.  Every operand is a 2-D
+    tensor with unit inner stride (leading dimensions may be wider than the data); lam is passed as fp32."""
+    ld_v = _f32_matrix(vec, "vec")
+    if not isinstance(cand, torch.Tensor) or cand.dtype != torch.int32:
+        raise ValueError(f"cand: expected an int32 tensor, got {getattr(cand, 'dtype', type(cand).__name__)}")
+    ld_c = _row_major(cand, "cand")
+    n_rows, n_cols = cand.shape
+    ld_r = _f32_matrix(rel, "rel")
+    if tuple(rel.shape) != (n_rows, n_cols):
+        raise ValueError(f"rel: expected the shape of cand {(n_rows, n_cols)}, got {tuple(rel.shape)}")
+    if not isinstance(items, torch.Tensor) or items.dtype != torch.int32:
+        raise ValueError(f"items: expected an int32 tensor, got {getattr(items, 'dtype', type(items).__name__)}")
+    ld_oi = _row_major(items, "items")
+    ld_or = _f32_matrix(out_rel, "out_rel")
+    for name, t in (("items", items), ("out_rel", out_rel)):
+        if t.shape[0] != n_rows or t.shape[1] < N:
+            raise ValueError(f"{name}: expected {n_rows} rows of >= {N} columns, got {tuple(t.shape)}")
+    D = vec.shape[1]
+    if not (1 <= n_cols <= 1024 and 1 <= D <= 256 and n_cols * D <= 32768 and 1 <= N <= n_cols):
+        raise ValueError(f"need 1 <= C <= 1024, 1 <= D <= 256, C * D <= 32768 and 1 <= N <= C (C = {n_cols}, D = {D}, "
+                         f"N = {N})")
+    if not 0.0 <= float(lam) <= 1.0:
+        raise ValueError(f"lam must be in [0, 1], got {lam!r}")
+    for name, t in (("cand", cand), ("rel", rel), ("items", items), ("out_rel", out_rel)):
+        if t.device != vec.device:
+            raise ValueError(f"{name} is on {t.device}, vec on {vec.device}")
+    _lib.call("dmm_mmr_rerank", _ctx(vec), _p(vec), ld_v, vec.shape[0], D, _p(cand), ld_c, _p(rel), ld_r, n_rows, n_cols,
+              int(N), float(lam), _p(items), ld_oi, _p(out_rel), ld_or, _stream())
+
+
 def eval_metrics_cutoffs(ranked, N, cutoffs, row_ids, test_ptr, test_items, inv_log2, max_dcg, out):
     """out[r, j] = (recall, ndcg, precision) at cutoffs[j] (host ints, strictly increasing, <= N) of user row_ids[r]'s
     ranked list ranked[r, :N] in float64 (Main.py:422-448 per prefix)."""

@@ -14,6 +14,10 @@ without the full contraction (dmm_score_pairs / dmm_rank_candidates): the same s
 fixed order, so a pair gets the same bits from both, though not score_topn's bits (the contraction sums in another
 order).  ``sampled_candidates`` builds the rows of the sampled-negative evaluation protocol (one held-out item against
 n_neg sampled negatives) on the host.
+
+``similar_items`` lists the items closest to given items by cosine: score_topn over the normalised rows with each
+query masked out of its own row.  ``mmr_rerank`` diversifies given candidate lists by Maximal Marginal Relevance
+(dmm_mmr_rerank: one CTA per row, the row's candidate vectors staged once in shared memory, n greedy steps).
 """
 from __future__ import annotations
 
@@ -33,6 +37,10 @@ MAX_CANDIDATES = 4096  # longest candidate row of rank_candidates (dmm_rank_cand
 # spread at 11.  The value equals the PRUNE_RATIO of csrc/topk.cu below which the pruned kernel defers a row (k <= 64)
 # to its slower second pass; keep the two together.
 PRUNE_RATIO = 4
+# dmm_mmr_rerank stages one row's candidate vectors as fp32 in 128 KB of shared memory: C <= 1024, D <= 256, C * D <= 32768
+MMR_MAX_C = 1024
+MMR_MAX_D = 256
+MMR_MAX_FLOATS = 32768
 
 
 def to_device(a: np.ndarray, device) -> torch.Tensor:
@@ -293,6 +301,121 @@ def _rank_candidates(user_embs, item_embs, cand, n, precision):
     if B:
         ops.rank_candidates(user_embs, item_embs, cand, n, precision == "bf16x3", items, scores)
     return items, scores
+
+
+def check_lam(lam) -> float:
+    """The MMR trade-off: a real number in [0, 1] (NaN refused)."""
+    if isinstance(lam, bool) or not isinstance(lam, numbers.Real) or not 0.0 <= float(lam) <= 1.0:
+        raise ValueError(f"lam must be a number in [0, 1], got {lam!r}")
+    return float(lam)
+
+
+def _check_vecs(item_vecs):
+    if not isinstance(item_vecs, torch.Tensor) or item_vecs.dtype != torch.float32 or item_vecs.dim() != 2:
+        raise ValueError(f"item_vecs must be a 2-D float32 tensor, got "
+                         f"{getattr(item_vecs, 'dtype', type(item_vecs).__name__)} {tuple(getattr(item_vecs, 'shape', ()))}")
+    if item_vecs.shape[0] < 1:
+        raise ValueError("item_vecs has no rows")
+
+
+def _rel(a, shape):
+    """Relevance as a host float32 numpy array or a float32 CUDA tensor (left where it is), of the candidates' shape."""
+    if isinstance(a, torch.Tensor):
+        if a.dtype != torch.float32 or tuple(a.shape) != shape:
+            raise ValueError(f"relevance must be float32 of shape {shape}, got {a.dtype} {tuple(a.shape)}")
+        return a if a.is_cuda else a.numpy()
+    arr = np.asarray(a)
+    if arr.dtype != np.float32 or arr.shape != shape:
+        raise ValueError(f"relevance must be float32 of shape {shape}, got {arr.dtype} {arr.shape}")
+    return arr
+
+
+def mmr_rerank(item_vecs: torch.Tensor, candidates, relevance, n: int, lam: float) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Maximal Marginal Relevance lists: row b's candidates re-ranked greedily, each step taking the candidate with the
+    largest lam * relevance - (1 - lam) * (its largest similarity to the items already picked) (dmm_mmr_rerank).
+
+    item_vecs fp32 [I, D] (CUDA; used as given: pass unit rows for cosine similarity), 1 <= D <= MMR_MAX_D.
+    candidates int [B, C] (-1 = empty slot) and relevance float32 [B, C]: host data or CUDA tensors on item_vecs'
+    device; 1 <= C <= MMR_MAX_C, C * D <= MMR_MAX_FLOATS, every candidate in -1..I-1 and every relevance at a
+    candidate slot finite, checked before any launch (one device synchronisation for CUDA input).  An item listed
+    twice in a row counts once, with its first relevance.  Ties go to the larger relevance, then the smaller item id, so
+    lam = 1 returns the relevance ranking.  1 <= n <= C.  Returns (items int64 [B, n], relevance fp32 [B, n]) on the
+    device, each pick with its given relevance; slots past the row's distinct candidates hold (-1, -inf)."""
+    _check_vecs(item_vecs)
+    I, D = item_vecs.shape
+    if not 1 <= D <= MMR_MAX_D:
+        raise ValueError(f"item_vecs must have 1..{MMR_MAX_D} columns, got {D}")
+    cand = _ids(candidates, "candidates", 2)
+    B, C = cand.shape
+    if not 1 <= C <= MMR_MAX_C or C * D > MMR_MAX_FLOATS:
+        raise ValueError(f"candidates must have 1..{min(MMR_MAX_C, MMR_MAX_FLOATS // D)} columns at D = {D} "
+                         f"(C <= {MMR_MAX_C}, C * D <= {MMR_MAX_FLOATS}), got {C}")
+    rel = _rel(relevance, (B, C))
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= n <= C:
+        raise ValueError(f"n must be an int in 1..{C} (the candidates per row), got {n!r}")
+    n, lam = int(n), check_lam(lam)
+    on_dev = isinstance(cand, torch.Tensor) or isinstance(rel, torch.Tensor)
+    if not on_dev:
+        bad = np.count_nonzero(~np.isfinite(rel) & (cand >= 0))
+        _check_ranges([(cand, -1, I - 1, "candidates"), (np.array([bad]), 0, 0, "non-finite relevance count")])
+    if not item_vecs.is_cuda:
+        raise ValueError(f"item_vecs must be a CUDA tensor, got {item_vecs.device}")
+    dev = item_vecs.device
+    for name, a in (("candidates", cand), ("relevance", rel)):
+        if isinstance(a, torch.Tensor) and a.device != dev:
+            raise ValueError(f"{name} is on {a.device}, item_vecs on {dev}")
+    with torch.cuda.device(dev):
+        r = rel if isinstance(rel, torch.Tensor) else to_device(rel, dev)
+        if on_dev:
+            # on the ids as given: the int32 cast below would wrap an id outside the int32 range into the valid range
+            valid = cand >= 0 if isinstance(cand, torch.Tensor) else to_device(cand >= 0, dev)
+            bad = (~torch.isfinite(r) & valid).sum()
+            _check_ranges([(cand, -1, I - 1, "candidates"), (bad, 0, 0, "non-finite relevance count")])
+        items, out = _mmr_rerank(item_vecs, _to(cand, dev, torch.int32), r.contiguous(), n, lam)
+        return items.long(), out
+
+
+def _mmr_rerank(item_vecs, cand, rel, n, lam):
+    """mmr_rerank without the argument checks: cand int32 / rel fp32 on the device, int32 items."""
+    B = cand.shape[0]
+    items = torch.empty((B, n), dtype=torch.int32, device=item_vecs.device)
+    out = torch.empty((B, n), dtype=torch.float32, device=item_vecs.device)
+    ops.mmr_rerank(item_vecs, cand, rel, n, lam, items, out)
+    return items, out
+
+
+def similar_items(item_vecs: torch.Tensor, items, n: int, precision: str = "bf16x3") -> Tuple[torch.Tensor, torch.Tensor]:
+    """The n items with the largest cosine to each query item, never the query itself: (items int64 [Q, n], cosines fp32
+    [Q, n]) on the device, cosine descending then item id ascending.
+
+    item_vecs fp32 [I, D] (CUDA); items: 1-D integer query ids (host data or a CUDA tensor on item_vecs' device), checked
+    before any launch; 1 <= n <= min(MAX_N, I - 1).  The rows are normalised as F.normalize does (ops.rownorm_fwd), and
+    the lists are score_topn(unit[items], unit, n, exclude=each query itself) with ``precision``, bit for bit."""
+    _check_precision(precision)
+    _check_vecs(item_vecs)
+    I = item_vecs.shape[0]
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= n <= min(MAX_N, I - 1):
+        raise ValueError(f"n must be an int in 1..{min(MAX_N, I - 1)} (at most {MAX_N} and the {I - 1} other items), "
+                         f"got {n!r}")
+    q = _ids(items, "items", 1)
+    check = [(q, 0, I - 1, "items")]
+    on_dev = isinstance(q, torch.Tensor)
+    if not on_dev:
+        _check_ranges(check)
+    if not item_vecs.is_cuda:
+        raise ValueError(f"item_vecs must be a CUDA tensor, got {item_vecs.device}")
+    dev = item_vecs.device
+    if on_dev and q.device != dev:
+        raise ValueError(f"items is on {q.device}, item_vecs on {dev}")
+    with torch.cuda.device(dev):
+        if on_dev:
+            _check_ranges(check)
+        qi = _to(q, dev, torch.int32)
+        Q = qi.shape[0]
+        unit, _ = ops.rownorm_fwd(item_vecs)
+        rows = torch.arange(Q + 1, dtype=torch.int64, device=dev)
+        out, cos = _topn(unit[qi.long()], unit, int(n), (rows, qi, rows[:Q]), float("-inf"), precision)
+        return out.long(), cos
 
 
 def check_n_neg(n_neg) -> int:

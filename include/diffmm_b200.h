@@ -506,6 +506,33 @@ int dmm_rank_candidates(dmm_ctx* ctx, const float* user, int64_t ld_u, const flo
                         int64_t D, const int32_t* cand, int64_t ld_c, int64_t n_rows, int64_t C, int64_t N, int x3,
                         int32_t* out_items, int64_t ld_oi, float* out_scores, int64_t ld_os, void* stream);
 
+/* ---- Maximal Marginal Relevance re-ranking of given candidates (Carbonell & Goldstein 1998) -----------------------
+ * dmm_mmr_rerank: row r (< n_rows) re-ranks its candidates cand[r * ld_c + 0 .. C) with relevance rel[r * ld_r + 0 .. C)
+ * greedily.  -1 or any id outside [0, n_items) is an empty slot, and so is a later occurrence of an item already in the
+ * row (the first occurrence's relevance counts).  sim(j, k) is the dot product of the fp32 rows vec[j * ld_v + 0 .. D)
+ * and vec[k * ld_v + 0 .. D) (unit rows give the cosine).  With S the picks so far, each step picks the unpicked valid
+ * candidate with the largest obj_j:
+ *     obj_j = lam * rel_j                          while S is empty,
+ *     obj_j = lam * rel_j - mu * m_j               afterwards, mu = fl(1 - lam), m_j = max over k in S of sim(j, k);
+ * ties on obj go to the larger relevance, then to the smaller item id (obj and relevance compared in the top-k kernels'
+ * total order: -0.0 ties with +0.0, +NaN above +inf, -NaN below -inf).  lam = 1 therefore reproduces the relevance
+ * order (relevance descending, then item ascending) and lam = 0 starts with the most relevant item.  The first N picks
+ * go to out_items[r * ld_oi + i] with their given relevance in out_rel[r * ld_or + i] (bit for bit); slots past the
+ * row's distinct valid candidates hold (-1, -inf).
+ * Arithmetic, every operation a separately rounded fp32 operation (no FMA contraction), fl() = round to nearest even:
+ *     sim(j, k): s_q = +0.0 for q = 0..3; for d = 0 .. D-1 ascending: s_{d mod 4} = fl(s_{d mod 4} + fl(v_j[d] * v_k[d]));
+ *                sim = fl(fl(s_0 + s_1) + fl(s_2 + s_3));
+ *     m_j:       -inf before the first pick, then m_j = fmax(m_j, sim(j, pick)) after each pick (IEEE maxNum: a NaN
+ *                sim is ignored);
+ *     obj_j:     fl(lam * rel_j) while S is empty, then fl(fl(lam * rel_j) - fl(mu * m_j)).
+ * 1 <= C <= 1024, 1 <= D <= 256, C * D <= 32768 (the row's vectors in 128 KB of shared memory), 1 <= N <= C,
+ * 0 <= lam <= 1; ld_v >= D, ld_c >= C, ld_r >= C, ld_oi >= N, ld_or >= N.  Zero rows is a no-op (the device pointers
+ * may then be NULL).  Each row reads its distinct valid candidates' vectors once and does about N * C * D
+ * multiply-adds from shared memory.                                                                                   */
+int dmm_mmr_rerank(dmm_ctx* ctx, const float* vec, int64_t ld_v, int64_t n_items, int64_t D, const int32_t* cand,
+                   int64_t ld_c, const float* rel, int64_t ld_r, int64_t n_rows, int64_t C, int64_t N, float lam,
+                   int32_t* out_items, int64_t ld_oi, float* out_rel, int64_t ld_or, void* stream);
+
 /* ---- host helper (no device work) --------------------------------------------------------------
  * Replays the reference's rejection-sampling loop (TrainData.negSampling, DataHandler.py:159-169)
  * over `n_draws` values pre-drawn by the caller from the same numpy generator: interaction i
