@@ -29,6 +29,18 @@ class GemmEpilogue(C.Structure):
     ]
 
 
+class GemmLaunchPlan(C.Structure):
+    """Mirror of struct dmm_gemm_launch_plan (dmm_gemm_plan)."""
+    _fields_ = [("bn", c_i32), ("ctas", c_i32), ("grid", c_i32), ("split", c_i32), ("sub_bn", c_i32), ("ksplit", c_i32),
+                ("epilogue", c_i32), ("stages", c_i32), ("nbuf", c_i32)]
+
+
+# enum dmm_gemm_plan_flag / dmm_gemm_epilogue_kind
+GEMM_A_LO, GEMM_B_LO, GEMM_RESIDUAL, GEMM_RES_HI, GEMM_RES_LO = 1, 2, 4, 8, 16
+GEMM_OUT_F32, GEMM_OUT_HI, GEMM_OUT_LO, GEMM_SPLITK = 32, 64, 128, 256
+GEMM_EPI_TMA, GEMM_EPI_REG, GEMM_EPI_REG_X3 = 0, 1, 2
+
+
 class NceProblem(C.Structure):
     """Mirror of struct dmm_nce_problem."""
     _fields_ = [("v1", c_vp), ("ld1", c_i64), ("v2", c_vp), ("ld2", c_i64), ("idx", c_vp), ("row_offset", c_i64),
@@ -69,6 +81,7 @@ PROTOTYPES = {
     "dmm_gemm_splitk_workspace_bytes": (c_i64, [c_vp, c_i64, c_i64, c_i64]),
     "dmm_gemm_bf16_tn_splitk": (C.c_int, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64,
                                           c_vp, c_i64, c_vp]),
+    "dmm_gemm_plan": (C.c_int, [C.c_int, c_i64, c_i64, c_i64, C.c_uint32, C.POINTER(GemmLaunchPlan)]),
     "dmm_gemm_f32_tn": (C.c_int, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, C.POINTER(GemmEpilogue), c_vp]),
     "dmm_topk_workspace_bytes": (c_i64, [c_i64, c_i64]),
     "dmm_topk_edges": (C.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64,

@@ -14,7 +14,7 @@ void dmm_set_error(const char* fmt, ...) {
   va_end(ap);
 }
 
-extern "C" int dmm_version(void) { return 101; }  // 0.1.1
+extern "C" int dmm_version(void) { return 102; }  // 0.1.2
 
 extern "C" const char* dmm_last_error(void) { return g_err; }
 

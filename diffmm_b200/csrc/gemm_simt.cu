@@ -76,6 +76,7 @@ __global__ void __launch_bounds__(256) gemm_f32_tn_kernel(const float* __restric
 extern "C" int dmm_gemm_f32_tn(dmm_ctx* ctx, const float* a, int64_t lda, const float* b, int64_t ldb, int64_t M,
                                int64_t N, int64_t K, const dmm_gemm_epilogue* ep, void* stream) {
   DMM_CHECK_ARG(ctx && a && b && ep, "dmm_gemm_f32_tn: null argument");
+  DMM_CHECK_ARG(!ep->cmax, "dmm_gemm_f32_tn: cmax is not supported");
   DMM_CHECK_ARG(M > 0 && N > 0 && K > 0 && lda >= K && ldb >= K, "dmm_gemm_f32_tn: bad shape");
   DMM_CHECK_ARG(dmm_ceil_div(M, TM) < 65536, "dmm_gemm_f32_tn: M too large for the verification kernel");
   dim3 grid((unsigned)dmm_ceil_div(N, TN), (unsigned)dmm_ceil_div(M, TM));

@@ -1019,28 +1019,112 @@ int make_epi_map(dmm_ctx* ctx, CUtensorMap* map, const void* base, bool f32, int
   return DMM_OK;
 }
 
+// Shared-memory bytes of the TMA epilogue next to the operand ring: per epilogue warp nbuf fp32 chunk buffers (4 KB,
+// SWIZZLE_128B boxes), a bf16 chunk buffer (2 KB, SWIZZLE_64B boxes) when there is a bf16 output, and 256 B of bias
+// slots; then the barrier block.
+int tepi_bytes(int nbuf, bool out_hi) { return EPI_WARPS * nbuf * 4096 + (out_hi ? EPI_WARPS * 2048 : 0) + EPI_WARPS * 256 + BAR_BYTES; }
+
+// split-K work items per tile (1: the shape does not split)
+int splitk_factor(int sms, int64_t M, int64_t N, int64_t K) {
+  const int64_t tiles = dmm_ceil_div(M, 2 * BLOCK_M) * dmm_ceil_div(N, 256);
+  const int64_t slots = sms / 2;
+  const int64_t kblocks = dmm_ceil_div(K, BLOCK_K);
+  int64_t ks = slots / (tiles > 0 ? tiles : 1);
+  if (ks > 8) ks = 8;
+  if (ks > kblocks / 8) ks = kblocks / 8;          // at least 8 k blocks (512 columns of K) per work item
+  if (ks < 2 || N <= 128) return 1;
+  const int64_t per = dmm_ceil_div(kblocks, ks);
+  return (int)dmm_ceil_div(kblocks, per);          // no empty split
+}
+
+// The launch plan (dmm_gemm_plan): every decision of a launch that is not fixed by the arguments.  Host arithmetic
+// only; the contraction launches exactly what this returns.
+int plan_gemm(int sms, int64_t M, int64_t N, int64_t K, uint32_t flags, dmm_gemm_launch_plan* pl) {
+  pl->ksplit = 1;
+  if (flags & DMM_GEMM_SPLITK) {
+    pl->ksplit = splitk_factor(sms, M, N, K);
+    if (pl->ksplit > 1) flags = DMM_GEMM_OUT_F32;   // the work items write plain fp32 partial products to slabs
+  }
+  // Tile shape by a small cost model: waves over the SMs (or SM pairs) x work per SM and wave / measured relative
+  // efficiency of the shape (256-wide pair tiles 1.0, single-CTA 256 / 128 / 64 columns 0.93 / 0.80 / 0.55).
+  const int64_t m128 = dmm_ceil_div(M, BLOCK_M), m256 = dmm_ceil_div(M, 2 * BLOCK_M);
+  auto waves = [](int64_t tiles, int64_t slots) { return (double)dmm_ceil_div(tiles, slots); };
+  double best = 1e300;
+  int bn = 64;
+  bool pair = false;
+  auto consider = [&](int cand_bn, bool cand_pair, double cost) {
+    if (cost < best) { best = cost; bn = cand_bn; pair = cand_pair; }
+  };
+  consider(64, false, waves(m128 * dmm_ceil_div(N, 64), sms) * 64.0 / 0.55);
+  if (N > 64) consider(128, false, waves(m128 * dmm_ceil_div(N, 128), sms) * 128.0 / 0.80);
+  if (N > 128) {
+    consider(256, false, waves(m128 * dmm_ceil_div(N, 256), sms) * 256.0 / 0.93);
+    if (sms >= 2) consider(256, true, waves(m256 * dmm_ceil_div(N, 256), sms / 2) * 256.0 / 1.0);
+  }
+  if (pl->ksplit > 1) {
+    bn = 256;
+    pair = true;
+  }
+  pl->bn = bn;
+  pl->ctas = pair ? 2 : 1;
+  // work items are tiles of (BLOCK_M * CTAS) rows; one persistent CTA (or CTA pair) per SM (or TPC)
+  const int64_t tiles = dmm_ceil_div(M, (int64_t)BLOCK_M * pl->ctas) * dmm_ceil_div(N, bn) * pl->ksplit;
+  const int64_t slots = sms / pl->ctas;
+  const int64_t grid = tiles < slots ? tiles : slots;
+  pl->grid = (int)(grid * pl->ctas);
+  // tail wave: when the last wave would fill at most half of the grid, cut its tiles into column slices
+  const int64_t rem = tiles % grid;
+  pl->split = 1;
+  if (rem > 0 && tiles > grid && pl->ksplit == 1) {
+    while (pl->split * 2 <= bn / 64 && rem * pl->split * 2 <= grid) pl->split *= 2;
+  }
+  pl->sub_bn = bn / pl->split;
+  // TMA epilogue (residual prefetch ring + bulk tensor stores) for the single-pass bf16 configurations; the
+  // register-staged epilogue serves the rest (split-bf16 operands, bf16 residual or lo output), in its split-bf16
+  // (fp32-faithful) instantiation whenever ANY lo part takes part: it keeps the accurate tanh in the post stage
+  const bool tepi = !(flags & (DMM_GEMM_A_LO | DMM_GEMM_B_LO | DMM_GEMM_RES_HI | DMM_GEMM_RES_LO | DMM_GEMM_OUT_LO)) &&
+                    (flags & (DMM_GEMM_OUT_F32 | DMM_GEMM_OUT_HI));
+  const bool x3 = flags & (DMM_GEMM_A_LO | DMM_GEMM_B_LO | DMM_GEMM_RES_LO | DMM_GEMM_OUT_LO);
+  pl->epilogue = tepi ? DMM_GEMM_EPI_TMA : (x3 ? DMM_GEMM_EPI_REG_X3 : DMM_GEMM_EPI_REG);
+  const int stage_bytes = BLOCK_M * BLOCK_K * 2 + (bn / pl->ctas) * BLOCK_K * 2;   // Cfg<bn, pair>::STAGE_BYTES
+  const int max_stages = bn == 64 ? Cfg<64>::STAGES : bn == 128 ? Cfg<128>::STAGES
+                         : pair ? Cfg<256, true>::STAGES : Cfg<256, false>::STAGES;
+  pl->nbuf = 1;
+  pl->stages = max_stages;
+  if (tepi) {
+    // with an fp32 residual every epilogue warp owns a ring of chunk buffers (prefetch depth nbuf - 1) and the
+    // operand ring takes what is left
+    pl->nbuf = (flags & DMM_GEMM_RESIDUAL) ? 2 : 1;   // measured: a 4-stage operand ring + 2 chunk buffers beats 3 stages + 3 buffers
+    const int stages = (SMEM_LIMIT - 1024 - tepi_bytes(pl->nbuf, flags & DMM_GEMM_OUT_HI)) / stage_bytes;
+    if (stages < 2) {
+      dmm_set_error("dmm_gemm_bf16_tn: no room for the operand ring next to the TMA epilogue (BN=%d)", bn);
+      return DMM_ERR_INVALID;
+    }
+    if (stages < pl->stages) pl->stages = stages;
+  }
+  return DMM_OK;
+}
+
 template <int BN, bool PAIR>
 int launch(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda, const uint16_t* b_hi,
-           const uint16_t* b_lo, int64_t ldb, GemmParams& p, bool tepi, cudaStream_t stream) {
+           const uint16_t* b_lo, int64_t ldb, GemmParams& p, const dmm_gemm_launch_plan& pl, cudaStream_t stream) {
   using C = Cfg<BN, PAIR>;
+  static_assert(C::STAGE_BYTES == BLOCK_M * BLOCK_K * 2 + (BN / C::CTAS) * BLOCK_K * 2, "plan_gemm's ring arithmetic");
   CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo, mbs_hi, mbs_lo, m_res, m_o32, m_o16;
   int rc;
+  const bool tepi = pl.epilogue == DMM_GEMM_EPI_TMA;
   p.num_n_blocks = (int)dmm_ceil_div(p.N, BN);
-  // work items are tiles of (BLOCK_M * CTAS) rows; one persistent CTA (or CTA pair) per SM (or TPC)
   const int m_items = (int)dmm_ceil_div(p.M, (int64_t)BLOCK_M * C::CTAS);
   p.num_m_blocks = m_items;
   const int tiles = m_items * p.num_n_blocks * p.ksplit;      // split-K: every tile is ksplit work items
-  const int slots = ctx->num_sms / C::CTAS;
-  const int grid = tiles < slots ? tiles : slots;
-  // tail wave: when the last wave would fill at most half of the grid, cut its tiles into column slices
+  const int grid = pl.grid / C::CTAS;
   const int rem = tiles % grid;
-  p.split = 1;
-  if (rem > 0 && tiles > grid && p.ksplit == 1) {
-    while (p.split * 2 <= BN / 64 && rem * p.split * 2 <= grid) p.split *= 2;
-  }
-  p.sub_bn = BN / p.split;
+  p.split = pl.split;
+  p.sub_bn = pl.sub_bn;
   p.full_items = p.split > 1 ? tiles - rem : tiles;
   p.total_items = p.full_items + (p.split > 1 ? rem * p.split : 0);
+  p.stages = pl.stages;
+  p.nbuf = pl.nbuf;
   if ((rc = make_map(ctx, &ma_hi, a_hi, p.M, p.K, lda, BLOCK_M))) return rc;
   if ((rc = make_map(ctx, &ma_lo, a_lo ? a_lo : a_hi, p.M, p.K, lda, BLOCK_M))) return rc;
   if ((rc = make_map(ctx, &mb_hi, b_hi, p.N, p.K, ldb, BN / C::CTAS))) return rc;
@@ -1052,25 +1136,11 @@ int launch(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda
   m_o16 = ma_hi;   // placeholders: never dereferenced unless the matching epilogue pointer is set
   int smem_bytes;
   if (tepi) {
-    // Shared-memory layout of the TMA epilogue.  With an fp32 residual every epilogue warp owns a ring of chunk buffers
-    // (prefetch depth nbuf - 1) and the operand ring takes what is left; otherwise one staging buffer per warp.
-    const bool has_res = p.ep.residual != nullptr;
-    p.nbuf = has_res ? 2 : 1;   // measured: a 4-stage operand ring + 2 chunk buffers beats 3 stages + 3 buffers
-    const int f32_bytes = EPI_WARPS * p.nbuf * 4096;
-    const int b16_bytes = p.ep.out_hi ? EPI_WARPS * 2048 : 0;
-    const int bias_bytes = EPI_WARPS * 256;
-    const int epi_bytes = f32_bytes + b16_bytes + bias_bytes + BAR_BYTES;
-    int stages = (SMEM_LIMIT - 1024 - epi_bytes) / C::STAGE_BYTES;
-    if (stages > C::STAGES) stages = C::STAGES;
-    if (stages < 2) {
-      dmm_set_error("dmm_gemm_bf16_tn: no room for the operand ring next to the TMA epilogue (BN=%d)", BN);
-      return DMM_ERR_INVALID;
-    }
-    p.stages = stages;
-    p.off_epi = stages * C::STAGE_BYTES;
-    p.off_b16 = p.off_epi + f32_bytes;
-    p.off_bias = p.off_b16 + b16_bytes;
-    p.off_bar = p.off_bias + bias_bytes;
+    // shared-memory layout of the TMA epilogue (tepi_bytes)
+    p.off_epi = p.stages * C::STAGE_BYTES;
+    p.off_b16 = p.off_epi + EPI_WARPS * p.nbuf * 4096;
+    p.off_bias = p.off_b16 + (p.ep.out_hi ? EPI_WARPS * 2048 : 0);
+    p.off_bar = p.off_bias + EPI_WARPS * 256;
     smem_bytes = p.off_bar + BAR_BYTES + 1024;
     if (p.ep.residual && (rc = make_epi_map(ctx, &m_res, p.ep.residual, true, p.M, p.N, p.ep.ld_res))) return rc;
     // split-K: the partial products are slabs of ks_rows rows, one per split
@@ -1078,8 +1148,6 @@ int launch(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda
     if (p.ep.out_f32 && (rc = make_epi_map(ctx, &m_o32, p.ep.out_f32, true, o32_rows, p.N, p.ep.ld_out))) return rc;
     if (p.ep.out_hi && (rc = make_epi_map(ctx, &m_o16, p.ep.out_hi, false, p.M, p.N, p.ep.ld_out16))) return rc;
   } else {
-    p.nbuf = 1;
-    p.stages = C::STAGES;
     p.off_bar = C::STAGES * C::STAGE_BYTES;
     p.off_epi = p.off_bar + BAR_BYTES;
     p.off_b16 = p.off_bias = 0;
@@ -1092,10 +1160,8 @@ int launch(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda
     DMM_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_kernel<BN, false, PAIR, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_once.mark(ctx);
   }
-  // split-bf16 (fp32-faithful) instantiation whenever ANY lo part takes part: it keeps the accurate tanh in the post stage
-  const bool x3 = a_lo != nullptr || b_lo != nullptr || p.ep.res_lo != nullptr || p.ep.out_lo != nullptr;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(grid * C::CTAS));
+  cfg.gridDim = dim3((unsigned)pl.grid);
   cfg.blockDim = dim3(NUM_THREADS);
   cfg.dynamicSmemBytes = (size_t)smem_bytes;
   cfg.stream = stream;
@@ -1109,7 +1175,7 @@ int launch(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda
   if (tepi) {
     DMM_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_tn_kernel<BN, false, PAIR, true>, ma_hi, ma_lo, mb_hi, mb_lo, mbs_hi, mbs_lo,
                                 m_res, m_o32, m_o16, p));
-  } else if (x3) {
+  } else if (pl.epilogue == DMM_GEMM_EPI_REG_X3) {
     DMM_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_tn_kernel<BN, true, PAIR, false>, ma_hi, ma_lo, mb_hi, mb_lo, mbs_hi, mbs_lo,
                                 m_res, m_o32, m_o16, p));
   } else {
@@ -1149,35 +1215,23 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restr
 }
 
 int run_gemm(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda, const uint16_t* b_hi, const uint16_t* b_lo,
-             int64_t ldb, int64_t M, int64_t N, int64_t K, const dmm_gemm_epilogue* ep, int ksplit, int ks_rows, void* stream);
+             int64_t ldb, int64_t M, int64_t N, int64_t K, const dmm_gemm_epilogue* ep, bool splitk, int ks_rows, void* stream);
 
 }  // namespace
 
 extern "C" int dmm_gemm_bf16_tn(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda,
                                 const uint16_t* b_hi, const uint16_t* b_lo, int64_t ldb, int64_t M, int64_t N,
                                 int64_t K, const dmm_gemm_epilogue* ep, void* stream) {
-  return run_gemm(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, M, N, K, ep, 1, 0, stream);
+  return run_gemm(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, M, N, K, ep, false, 0, stream);
 }
 
 // Split-K for contractions with few output tiles and a long K (P = W1x W2 of the hidden-space chain: 1024 x 1024 x I is 16
 // pair tiles on 74 pair slots): each tile's k blocks are divided over up to 8 work items whose fp32 partial products go to
 // slabs of the workspace; a second small launch adds the slabs in a fixed order (deterministic) and writes the fp32 result
 // and / or its bf16 operand copies.  Falls back to the plain contraction when the tiles already fill the machine.
-static int splitk_factor(const dmm_ctx* ctx, int64_t M, int64_t N, int64_t K) {
-  const int64_t tiles = dmm_ceil_div(M, 2 * BLOCK_M) * dmm_ceil_div(N, 256);
-  const int64_t slots = ctx->num_sms / 2;
-  const int64_t kblocks = dmm_ceil_div(K, BLOCK_K);
-  int64_t ks = slots / (tiles > 0 ? tiles : 1);
-  if (ks > 8) ks = 8;
-  if (ks > kblocks / 8) ks = kblocks / 8;          // at least 8 k blocks (512 columns of K) per work item
-  if (ks < 2 || N <= 128) return 1;
-  const int64_t per = dmm_ceil_div(kblocks, ks);
-  return (int)dmm_ceil_div(kblocks, per);          // no empty split
-}
-
 extern "C" int64_t dmm_gemm_splitk_workspace_bytes(dmm_ctx* ctx, int64_t M, int64_t N, int64_t K) {
   if (!ctx) return 0;
-  const int ks = splitk_factor(ctx, M, N, K);
+  const int ks = splitk_factor(ctx->num_sms, M, N, K);
   if (ks <= 1) return 0;
   const int64_t rows = dmm_ceil_div(M, 2 * BLOCK_M) * 2 * BLOCK_M, ld = (N + 3) & ~(int64_t)3;
   return (int64_t)ks * rows * ld * (int64_t)sizeof(float);
@@ -1192,14 +1246,18 @@ extern "C" int dmm_gemm_bf16_tn_splitk(dmm_ctx* ctx, const uint16_t* a_hi, int64
   DMM_CHECK_ARG(!out_f32 || ld_out >= N, "dmm_gemm_bf16_tn_splitk: ld_out must be >= N");
   DMM_CHECK_ARG(!out_hi || ld_out16 >= N, "dmm_gemm_bf16_tn_splitk: ld_out16 must be >= N");
   DMM_CHECK_ARG(!out_lo || out_hi, "dmm_gemm_bf16_tn_splitk: out_lo requires out_hi");
-  const int ks = splitk_factor(ctx, M, N, K);
+  uint32_t flags = DMM_GEMM_SPLITK | (out_f32 ? DMM_GEMM_OUT_F32 : 0) | (out_hi ? DMM_GEMM_OUT_HI : 0) | (out_lo ? DMM_GEMM_OUT_LO : 0);
+  dmm_gemm_launch_plan pl;
+  int rc = plan_gemm(ctx->num_sms, M, N, K, flags, &pl);
+  if (rc) return rc;
+  const int ks = pl.ksplit;
   if (ks <= 1) {
     // plain contraction; the bf16 lo part needs the fp32 result, which the split path has anyway
     DMM_CHECK_ARG(!out_lo || out_f32, "dmm_gemm_bf16_tn_splitk: out_lo without out_f32 needs a split (shape does not split)");
     dmm_gemm_epilogue ep = {};
     ep.alpha = 1.f;
     ep.out_f32 = out_f32, ep.ld_out = ld_out, ep.out_hi = out_hi, ep.out_lo = out_lo, ep.ld_out16 = ld_out16;
-    return run_gemm(ctx, a_hi, nullptr, lda, b_hi, nullptr, ldb, M, N, K, &ep, 1, 0, stream);
+    return run_gemm(ctx, a_hi, nullptr, lda, b_hi, nullptr, ldb, M, N, K, &ep, false, 0, stream);
   }
   DMM_CHECK_ARG(workspace && workspace_bytes >= dmm_gemm_splitk_workspace_bytes(ctx, M, N, K) &&
                     (reinterpret_cast<uintptr_t>(workspace) & 15u) == 0,
@@ -1209,7 +1267,7 @@ extern "C" int dmm_gemm_bf16_tn_splitk(dmm_ctx* ctx, const uint16_t* a_hi, int64
   ep.alpha = 1.f;
   ep.out_f32 = (float*)workspace;
   ep.ld_out = ld;
-  int rc = run_gemm(ctx, a_hi, nullptr, lda, b_hi, nullptr, ldb, M, N, K, &ep, ks, (int)rows, stream);
+  rc = run_gemm(ctx, a_hi, nullptr, lda, b_hi, nullptr, ldb, M, N, K, &ep, true, (int)rows, stream);
   if (rc) return rc;
   const int64_t work = M * ((N + 3) >> 2);
   splitk_reduce_kernel<<<(unsigned)dmm_ceil_div(work, 256), 256, 0, (cudaStream_t)stream>>>(
@@ -1220,7 +1278,7 @@ extern "C" int dmm_gemm_bf16_tn_splitk(dmm_ctx* ctx, const uint16_t* a_hi, int64
 
 namespace {
 int run_gemm(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda, const uint16_t* b_hi, const uint16_t* b_lo,
-             int64_t ldb, int64_t M, int64_t N, int64_t K, const dmm_gemm_epilogue* ep, int ksplit, int ks_rows, void* stream) {
+             int64_t ldb, int64_t M, int64_t N, int64_t K, const dmm_gemm_epilogue* ep, bool splitk, int ks_rows, void* stream) {
   DMM_CHECK_ARG(ctx && a_hi && b_hi && ep, "dmm_gemm_bf16_tn: null argument");
   DMM_CHECK_ARG(ctx->encode_tiled, "dmm_gemm_bf16_tn: cuTensorMapEncodeTiled unavailable");
   DMM_CHECK_ARG(M > 0 && N > 0 && K > 0, "dmm_gemm_bf16_tn: empty problem M=%lld N=%lld K=%lld", (long long)M,
@@ -1247,13 +1305,23 @@ int run_gemm(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t l
   DMM_CHECK_ARG(al16(ep->post_bias), "dmm_gemm_bf16_tn: post_bias must be 16-byte aligned");
   DMM_CHECK_ARG(!ep->cmax || ep->ld_cmax >= dmm_ceil_div(N, 32), "dmm_gemm_bf16_tn: ld_cmax must be >= ceil(N / 32)");
 
+  const uint32_t flags = (a_lo ? DMM_GEMM_A_LO : 0) | (b_lo ? DMM_GEMM_B_LO : 0) | (ep->residual ? DMM_GEMM_RESIDUAL : 0) |
+                         (ep->res_hi ? DMM_GEMM_RES_HI : 0) | (ep->res_lo ? DMM_GEMM_RES_LO : 0) |
+                         (ep->out_f32 ? DMM_GEMM_OUT_F32 : 0) | (ep->out_hi ? DMM_GEMM_OUT_HI : 0) |
+                         (ep->out_lo ? DMM_GEMM_OUT_LO : 0) | (splitk ? DMM_GEMM_SPLITK : 0);
+  dmm_gemm_launch_plan pl;
+  int rc = plan_gemm(ctx->num_sms, M, N, K, flags, &pl);
+  if (rc) return rc;
+  DMM_CHECK_ARG(pl.ksplit == 1 || (ep->out_f32 && !ep->out_hi && !ep->residual && !ep->bias && !ep->cmax && ep->act == 0),
+                "dmm_gemm_bf16_tn: split-K writes plain fp32 partial products");
+
   GemmParams p;
   p.M = (int)M;
   p.N = (int)N;
   p.K = (int)K;
   p.num_m_blocks = (int)dmm_ceil_div(M, BLOCK_M);
   p.num_k_blocks = (int)dmm_ceil_div(K, BLOCK_K);
-  p.ksplit = ksplit > 1 ? ksplit : 1;
+  p.ksplit = pl.ksplit;
   p.kb_per = (int)dmm_ceil_div(p.num_k_blocks, p.ksplit);
   p.ks_rows = ks_rows;
   p.n_pass = 0;
@@ -1264,39 +1332,20 @@ int run_gemm(dmm_ctx* ctx, const uint16_t* a_hi, const uint16_t* a_lo, int64_t l
   for (int i = p.n_pass; i < 3; ++i) p.pass_a[i] = p.pass_b[i] = 0;
   p.ep = *ep;
 
-  // Tile shape by a small cost model: waves over the SMs (or SM pairs) x work per SM and wave / measured relative
-  // efficiency of the shape (256-wide pair tiles 1.0, single-CTA 256 / 128 / 64 columns 0.93 / 0.80 / 0.55).
-  const int64_t m128 = dmm_ceil_div(M, BLOCK_M), m256 = dmm_ceil_div(M, 2 * BLOCK_M);
-  auto waves = [](int64_t tiles, int64_t slots) { return (double)dmm_ceil_div(tiles, slots); };
-  const int sms = ctx->num_sms;
-  double best = 1e300;
-  int bn = 64;
-  bool pair = false;
-  auto consider = [&](int cand_bn, bool cand_pair, double cost) {
-    if (cost < best) { best = cost; bn = cand_bn; pair = cand_pair; }
-  };
-  consider(64, false, waves(m128 * dmm_ceil_div(N, 64), sms) * 64.0 / 0.55);
-  if (N > 64) consider(128, false, waves(m128 * dmm_ceil_div(N, 128), sms) * 128.0 / 0.80);
-  if (N > 128) {
-    consider(256, false, waves(m128 * dmm_ceil_div(N, 256), sms) * 256.0 / 0.93);
-    if (sms >= 2) consider(256, true, waves(m256 * dmm_ceil_div(N, 256), sms / 2) * 256.0 / 1.0);
-  }
-  if (p.ksplit > 1) {
-    bn = 256;
-    pair = true;
-  }
   cudaStream_t st = (cudaStream_t)stream;
-  // TMA epilogue (residual prefetch ring + bulk tensor stores) for the single-pass bf16 configurations; the
-  // register-staged epilogue serves the rest (split-bf16 operands, bf16 residual or lo output)
-  const bool tepi = !a_lo && !b_lo && !ep->res_hi && !ep->res_lo && !ep->out_lo && (ep->out_f32 || ep->out_hi);
-  DMM_CHECK_ARG(p.ksplit == 1 || (tepi && ep->out_f32 && !ep->out_hi && !ep->residual && !ep->bias && !ep->cmax && ep->act == 0),
-                "dmm_gemm_bf16_tn: split-K writes plain fp32 partial products");
-  switch (bn) {
-    case 64: return launch<64, false>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, tepi, st);
-    case 128: return launch<128, false>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, tepi, st);
+  switch (pl.bn) {
+    case 64: return launch<64, false>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, pl, st);
+    case 128: return launch<128, false>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, pl, st);
     default:
-      return pair ? launch<256, true>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, tepi, st)
-                  : launch<256, false>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, tepi, st);
+      return pl.ctas == 2 ? launch<256, true>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, pl, st)
+                          : launch<256, false>(ctx, a_hi, a_lo, lda, b_hi, b_lo, ldb, p, pl, st);
   }
 }
 }  // namespace
+
+extern "C" int dmm_gemm_plan(int num_sms, int64_t M, int64_t N, int64_t K, uint32_t flags, dmm_gemm_launch_plan* plan) {
+  DMM_CHECK_ARG(plan && num_sms > 0, "dmm_gemm_plan: null plan or num_sms < 1");
+  DMM_CHECK_ARG(M > 0 && N > 0 && K > 0 && M < (1LL << 31) && N < (1LL << 31) && K < (1LL << 31), "dmm_gemm_plan: bad shape");
+  DMM_CHECK_ARG((flags & ~0x1FFu) == 0, "dmm_gemm_plan: unknown flag bits 0x%x", flags);
+  return plan_gemm(num_sms, M, N, K, flags, plan);
+}

@@ -206,7 +206,35 @@ int dmm_gemm_bf16_tn_splitk(dmm_ctx* ctx, const uint16_t* a_hi, int64_t lda, con
                             int64_t M, int64_t N, int64_t K, float* out_f32, int64_t ld_out, uint16_t* out_hi,
                             uint16_t* out_lo, int64_t ld_out16, void* workspace, int64_t workspace_bytes, void* stream);
 
-/* Same contract on the fp32 CUDA-core pipe from fp32 operands (verification mode; no tensor cores). */
+/* Launch plan of dmm_gemm_bf16_tn (or, with DMM_GEMM_SPLITK, of dmm_gemm_bf16_tn_splitk) on a device of `num_sms` SMs:
+ * the plan those calls launch, computed from the shape and from which pointers are non-NULL (`flags`, an OR of
+ * dmm_gemm_plan_flag).  Makes no CUDA call.  Returns DMM_ERR_INVALID for a bad shape and for a plan that leaves no room
+ * for the operand ring, the error the contraction itself would return.                                           */
+enum dmm_gemm_plan_flag {
+  DMM_GEMM_A_LO = 1, DMM_GEMM_B_LO = 2, DMM_GEMM_RESIDUAL = 4, DMM_GEMM_RES_HI = 8, DMM_GEMM_RES_LO = 16,
+  DMM_GEMM_OUT_F32 = 32, DMM_GEMM_OUT_HI = 64, DMM_GEMM_OUT_LO = 128,
+  DMM_GEMM_SPLITK = 256   /* the split-K entry; its outputs are given as OUT_F32 / OUT_HI / OUT_LO */
+};
+enum dmm_gemm_epilogue_kind {
+  DMM_GEMM_EPI_TMA = 0,     /* single-pass bf16, TMA residual ring and bulk tensor stores     */
+  DMM_GEMM_EPI_REG = 1,     /* single-pass bf16, register-staged (bf16 residual, no lo part)  */
+  DMM_GEMM_EPI_REG_X3 = 2   /* split-bf16: any lo operand, residual or output                 */
+};
+typedef struct dmm_gemm_launch_plan {
+  int32_t bn;        /* tile columns: 64, 128 or 256                                                       */
+  int32_t ctas;      /* CTAs per tile: 1, or 2 for a cta_group::2 pair tile of 256 rows                    */
+  int32_t grid;      /* CTAs launched (persistent)                                                         */
+  int32_t split;     /* the tiles of a partly filled last wave are cut into `split` slices of sub_bn columns */
+  int32_t sub_bn;
+  int32_t ksplit;    /* work items per tile along K (split-K entry), else 1                                 */
+  int32_t epilogue;  /* dmm_gemm_epilogue_kind                                                             */
+  int32_t stages;    /* depth of the shared-memory operand ring                                            */
+  int32_t nbuf;      /* fp32 chunk buffers per epilogue warp (TMA epilogue), else 1                        */
+} dmm_gemm_launch_plan;
+int dmm_gemm_plan(int num_sms, int64_t M, int64_t N, int64_t K, uint32_t flags, dmm_gemm_launch_plan* plan);
+
+/* Same contract on the fp32 CUDA-core pipe from fp32 operands (verification mode; no tensor cores); cmax is not
+ * supported (an argument error). */
 int dmm_gemm_f32_tn(dmm_ctx* ctx, const float* a, int64_t lda, const float* b, int64_t ldb,
                     int64_t M, int64_t N, int64_t K, const dmm_gemm_epilogue* ep, void* stream);
 
