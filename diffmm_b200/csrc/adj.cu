@@ -82,19 +82,25 @@ __global__ void __launch_bounds__(256) fill_adj_kernel(const int64_t* __restrict
   const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t N = n_users + n_items;
   if (j < n_edges) {
+    // an item id outside [0, n_items) (flagged in status bit 1) indexes neither dinv nor an item-side slot: its user-side
+    // entry becomes (the row's own node, NaN) and its item-side entry is not written, so nothing outside the arrays is
+    // touched and no stored column is >= N
     {
       const int64_t u = edge_user[j];
       const int32_t it = items[j];
+      const bool ok = it >= 0 && it < n_items;
       const int64_t o = j + u + 1;  // one self loop per user row up to and including u
-      adj_idx[o] = (int32_t)(n_users + it);
-      adj_val[o] = (float)((dinv[u] * 1.0) * dinv[n_users + it]);
+      adj_idx[o] = ok ? (int32_t)(n_users + it) : (int32_t)u;
+      adj_val[o] = ok ? (float)((dinv[u] * 1.0) * dinv[n_users + it]) : __int_as_float(0x7FC00000);
     }
     {
       const int64_t it = items_sorted[j];
       const int32_t u = users_by_item[j];
-      const int64_t o = n_edges + n_users + j + it;  // user block, then one self loop per preceding item row
-      adj_idx[o] = u;
-      adj_val[o] = (float)((dinv[n_users + it] * 1.0) * dinv[u]);
+      if (it >= 0 && it < n_items) {
+        const int64_t o = n_edges + n_users + j + it;  // user block, then one self loop per preceding item row
+        adj_idx[o] = u;
+        adj_val[o] = (float)((dinv[n_users + it] * 1.0) * dinv[u]);
+      }
     }
   }
   if (j < N) {
@@ -147,8 +153,11 @@ inline size_t carve(Workspace& w, void* base, int64_t U, int64_t I, int64_t E) {
 extern "C" int64_t dmm_build_adj_workspace_bytes(int64_t n_users, int64_t n_items, int64_t n_edges) {
   Workspace w;
   const size_t fixed = carve(w, nullptr, n_users, n_items, n_edges);
-  // CUB radix-sort temporary storage is O(#tiles) histograms; bound it generously
-  return (int64_t)(fixed + (size_t)(32u << 20) + (size_t)(n_edges > 0 ? n_edges : 0));
+  // CUB's SortPairs with separate input and output arrays allocates, besides its histograms and look-back tiles (< 32 MiB
+  // + 1 byte per item for int32 keys), one more key and one more value array of E x 4 bytes each whenever the sort takes
+  // more than one digit pass (dispatch_radix_sort.cuh, both the onesweep and the upsweep/downsweep paths)
+  const size_t e = (size_t)(n_edges > 0 ? n_edges : 0);
+  return (int64_t)(fixed + (size_t)(32u << 20) + e + 2 * align256(e * sizeof(int32_t)));
 }
 
 extern "C" int dmm_build_norm_adj_csr(dmm_ctx* ctx, const int64_t* row_ptr, const int32_t* items, int64_t n_users,

@@ -261,7 +261,10 @@ int dmm_topk_edges(dmm_ctx* ctx, const float* scores, int64_t ld, int64_t n_rows
  * a quarter of the row, NaN scores, crowded ties) are collected on the device and finished in the same call by a small
  * persistent grid: two-level exact radix select (top-k of the chunk maxima, then top-k of those chunks' scores) or, for
  * rows with NaN / k chunks above half of the row, the whole-row generic path.
- * `workspace` (required): dmm_topk_pruned_workspace_bytes(n_rows, n_cols, n_edges).                              */
+ * `workspace` (required): dmm_topk_pruned_workspace_bytes(n_rows, n_cols, n_edges).  After a call that runs the pruned
+ * kernel (8 <= ceil(n_cols / 32) <= 16384), the workspace holds the deferred rows: an int32 count at byte offset 0 and
+ * that many int32 row indices r (in no particular order) from byte offset 256.  Other widths take the dmm_topk_edges
+ * kernels for the whole call and leave the count unwritten.                                                      */
 int64_t dmm_topk_pruned_workspace_bytes(int64_t n_rows, int64_t n_cols, int64_t n_edges);
 int dmm_topk_edges_pruned(dmm_ctx* ctx, const float* scores, int64_t ld, int64_t n_rows, int64_t n_cols,
                           const float* cmax, int64_t ld_cmax, const int64_t* out_ptr, int64_t row_base,
@@ -274,7 +277,9 @@ int dmm_topk_edges_pruned(dmm_ctx* ctx, const float* scores, int64_t ld, int64_t
  * adj_ptr int64 [N+1], adj_idx int32 [2E+N] (sorted within rows), adj_val fp32 with the
  * reference's fp64 arithmetic (d_r^-1/2 * 1) * d_c^-1/2 rounded to fp32.
  * An item id outside [0, n_items) is an error flagged by OR-ing bit 1 into *status (device int, optional; the
- * arrays written for such a list are unspecified and must not be used).
+ * contents of adj_ptr / adj_idx / adj_val for such a list are unspecified and must not be used, but nothing outside
+ * them or the workspace is read or written, and no stored column is >= N).
+ * dmm_build_adj_workspace_bytes covers the radix sort's scratch, including its two extra E x 4-byte arrays.
  * Replaces Coach.makeTorchAdj (Main.py:113-116) -> DataHandler.makeTorchAdj / normalizeAdj
  * (DataHandler.py:53-93), which run on the host in scipy.                                    */
 int64_t dmm_build_adj_workspace_bytes(int64_t n_users, int64_t n_items, int64_t n_edges);

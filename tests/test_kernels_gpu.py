@@ -77,11 +77,18 @@ def test_topk_random_vs_oracle(ops, n_cols, ld):
 
 def test_topk_generic_kernels_forced():
     """The register path covers every shipped row width, so the generic kernels (bucket histogram + radix
-    select; rows wider than 32768 columns) are also forced onto small and mid-sized rows in a subprocess."""
+    select; rows wider than 32768 columns) are also forced onto small and mid-sized rows in a subprocess, on the
+    widths of the register kernels' and the shared-memory kernel's boundaries (tests/test_rebuild_tail_kernels_gpu.py),
+    with aligned rows and with ld % 4 == 1."""
     import subprocess
     import sys
     env = dict(os.environ, DMM_TOPK_GENERIC="1")
+    optin = torch.cuda.get_device_properties(0).shared_memory_per_block_optin
+    cap = (optin - 20480) // 4                       # widest row the shared-memory generic kernel stages
     args = ["500:500:0", "7050:7104:1", "33:36:1", "40000:40000:1"]
+    for n in (8191, 8192, 8193, 16384, 16386, 32767, 32768, 32769, cap, cap + 1):
+        ld4 = (n + 3) // 4 * 4
+        args += [f"{n}:{ld4}:1", f"{n}:{ld4 + 1}:1"]
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "dbg_topk.py"), *args], env=env, capture_output=True,
                        text=True, timeout=600)
     assert r.returncode == 0, r.stdout + r.stderr
